@@ -4,6 +4,7 @@ denoiser (BASELINE.json configs[1]/[4]: chs=[32,64,128,256], conditioning field 
 
     python bench.py --gpus N --steps K --warmup W            # this repository's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU oracle port on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR  # ... and write the last timed step's outputs to DIR
 
 A "step" is one reverse step of the chain for the whole batch of realisations on every rank: one CUNet
 forward (about 30 tcgen05 conv launches + the fused elementwise kernels) plus the fused sampler update.
@@ -32,6 +33,8 @@ METRIC = "denoiser voxel-steps/s at 128^3 (reverse ancestral sampling)"
 UNIT = "voxel-steps/s"
 PARAM_LO = [0.1, 0.6, 0.25, 0.25, 0.5, 0.5]      # CAMELS parameter ranges (SURVEY.md section 8d)
 PARAM_HI = [0.5, 1.0, 4.0, 4.0, 2.0, 2.0]
+DUMP_MAX_ELEMENTS = 1 << 22      # per dumped array (16 MiB of float32): the two arrays of --dump-outputs stay under 64 MB
+DUMP_SAMPLE_SEED = 2024
 
 
 def synthetic_batch(batch, grid, seed, device="cpu"):
@@ -84,6 +87,21 @@ class ClockSampler:
         busy = [v for v in sm if v > 0.5 * (mx[0] if mx else 1)] or sm
         return {"sm_mhz": statistics.median(busy) if busy else None, "sm_max_mhz": mx[0] if mx else None,
                 "reasons": reasons, "samples": len(sm)}
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of ``arrays`` as ``out_dir/<name>.npy`` in float32.  A tensor of at most DUMP_MAX_ELEMENTS
+    elements is written whole, in its shape; a larger one as the 1-D array of its elements at DUMP_MAX_ELEMENTS flat
+    indices drawn without replacement by numpy's default_rng(DUMP_SAMPLE_SEED) and sorted.  The indices depend on the
+    element count only, so two runs with the same arguments can be compared element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 def measured_peaks():
@@ -319,6 +337,9 @@ def run_b200(args, rank, world, local_rank):
     value = world * batch * voxels * args.steps / (ms_max * 1e-3)
     launches = sess.kernels_per_step * args.steps
     assert torch.isfinite(sess.z).all(), "sampler state went non-finite"
+    if args.dump_outputs and rank == 0:
+        # the latent after the last timed step (what the chain hands on) and the denoiser output that step used
+        dump_outputs(args.dump_outputs, {"z": sess.z, "eps": sess.eps})
 
     # ---- end to end through the public API: host conditioning in, host sample out ----
     # one public-API call = one whole chain: the reference's default length (LightVDM.draw_samples(n_sampling_steps=250),
@@ -807,7 +828,14 @@ def main():
     ap.add_argument("--no-torch-gpu-baseline", action="store_true", help="skip the stock-PyTorch-on-GPU arm")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the SFM 160^3 / VDM 224^3 training steps")
     ap.add_argument("--pipeline-steps", type=int, default=20, help="reverse steps of the scaled-down ensemble pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's latent z and denoiser output eps of the last timed step "
+                         "as DIR/z.npy and DIR/eps.npy (float32; arrays above 2^22 elements as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
