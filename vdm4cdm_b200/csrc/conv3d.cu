@@ -41,10 +41,9 @@
 // slices, twelve epilogue warps (or eight + four transform warps).
 //
 // Roofline: tensor-bound; algorithmic FLOPs = 2 * taps * Cin * Cout * B*D*H*W.
-#include <cudaTypedefs.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
+#include "tma_host.cuh"
 
 // Ablation branches (timing experiments whose results are wrong by construction) exist in bring-up builds only
 // (-DVDM_BRINGUP, `make bringup`); in the release library VDM_DBG is a compile-time false and the branches vanish.
@@ -57,7 +56,7 @@
 namespace vdm {
 
 // 16 warps in four warpgroups (setmaxnreg re-balances the register file per warpgroup):
-//   WG0  warp 0 A producer, warp 1 MMA issuer, warp 2 B producer, warp 3 idle        64 registers
+//   WG0  warp 0 A producer, warp 1 MMA issuer, warps 2, 3 B producers                 64 registers
 //   WG1-2 warps 4..11  epilogue (two per TMEM lane quarter)                          176 registers
 //   WG3  warps 12..15  input transform (GroupNorm + SiLU on the landed halo tile)     88 registers
 constexpr int kConvThreads = 512;
@@ -1175,128 +1174,280 @@ conv3d_planar_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
 #include "conv3d_march.cuh"
 
 // ---- host side ------------------------------------------------------------------------------
-static PFN_cuTensorMapEncodeTiled_v12000 get_encode_fn() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = []() -> PFN_cuTensorMapEncodeTiled_v12000 {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return nullptr;
-    return reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(ptr);
-  }();
-  return fn;
-}
-
-static int num_sms() {
-  static int n = []() {
-    int dev = 0, v = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return kNumSMs;
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) return kNumSMs;
-    return v;
-  }();
-  return n;
-}
-
+// Bring-up overrides of the planner, set by vdm_debug_set in `make bringup` builds.  In the release library they are a
+// compile-time all-zero constant and their branches vanish.
+struct ConvOverrides {
+  int debug_flags;                       // ConvKernelParams::debug_flags (ablation experiments: results are wrong)
+  int force_mt, force_kc, force_nsplit;  // > 0: replaces the planned value (force_mt / force_nsplit also rule out kd-folding)
+  int no_resident;                       // generic schedule: stream the weights even where they fit shared memory
+  int no_fold;                           // no kd-folded (nor marching) schedule
+  int no_march;                          // the tile kernel's kd-folded schedule instead of the marching one
+};
 #ifdef VDM_BRINGUP
-static int g_debug_flags = 0;
-static int g_debug_force_mt = 0, g_debug_force_kc = 0, g_debug_force_nsplit = 0, g_debug_no_resident = 0, g_debug_no_fold = 0;
-static int g_debug_no_march = 0;
+static ConvOverrides g_overrides = {};
 #else
-constexpr int g_debug_flags = 0;
-constexpr int g_debug_force_mt = 0, g_debug_force_kc = 0, g_debug_force_nsplit = 0, g_debug_no_resident = 0, g_debug_no_fold = 0;
-constexpr int g_debug_no_march = 0;
+constexpr ConvOverrides g_overrides = {};
 #endif
 
-// Launch of the d-marching schedule (conv3d_march.cuh).  `p` carries the grid, the plane windows and the epilogue; this
-// fills in the unit decomposition, the shared-memory plan and the one-slice tensor map.
-static int launch_march(const VdmConvDesc& d, ConvKernelParams& p, const void* x, const void* skip_x, const float* in_norm, int kc,
-                        int halo, int x_planes, bool has_residual, PFN_cuTensorMapEncodeTiled_v12000 encode, cudaStream_t stream) {
-  p.in_norm = in_norm;                 // fused GroupNorm + SiLU of the input: warps 12..15 transform, eight epilogue warps
-  p.c_in = d.c_in;
-  const int NF = p.n_cta, planes = kc / 8, sms = num_sms();
-  // Segment length: static round-robin over equal units, so the launch takes ceil(units / SMs) rounds of (seglen + 2) slices
-  // (+1: per-unit fixed costs); short segments balance the SMs, long ones amortise the two halo slices.
-  const long long cols = (long long)d.batch * p.tiles_h * p.tiles_w;
-  int nseg_best = 1;
-  double best = -1.0;
-  for (int nseg = 1; nseg <= ceil_div(d.depth, 4); ++nseg) {
-    const int seglen = ceil_div(d.depth, nseg);
-    if (ceil_div(d.depth, seglen) != nseg) continue;
-    const long long rounds = (cols * nseg + sms - 1) / sms;
-    const double cost = (double)rounds * (seglen + 3);
-    if (best < 0.0 || cost < best * 0.999) { best = cost; nseg_best = nseg; }
+enum class ConvSchedule {
+  kTile,           // conv3d_planar_kernel<MT, KJ, 0>: generic tap loop
+  kFoldResident,   // conv3d_planar_kernel<MT, KJ, NF>: kd folded into N, all weights resident in shared memory
+  kFoldStreamed,   // conv3d_planar_kernel<4, 2, 64>: kd folded into N, weights streamed per (chunk, kh, kw)
+  kMarch,          // conv3d_march_kernel (conv3d_march.cuh): kd-folded resident layers whose input channels are one chunk
+};
+
+struct ConvPlan {
+  ConvSchedule schedule;
+  int pad;                        // 1 when a tap reads a neighbour voxel (one-voxel halo), else 0
+  int mt, kc, n_split, n_cta;     // d-slices per tile, channels per chunk, CTAs per spatial tile and their UMMA N
+  int n_tiles, grid;
+  int nsa, nsb, taps_per_stage;   // halo stages, weight stages, filter taps per weight stage
+  int a_stage_bytes, b_stage_bytes, b_resident;
+  int res_depth, res_ring_off;    // residual units in flight per epilogue thread, byte offset of their ring
+  int xf_coef_off;                // byte offset of the fused input transform's (a, b) table
+  size_t smem_bytes;              // dynamic shared memory of the launch
+  int m_units, m_nseg, m_seglen;  // marching schedule: units = columns x d-segments of m_seglen slices
+  int debug_flags;
+};
+
+// Cell kd * 9 + kh * 3 + kw of tap t in the 3x3x3 stencil.
+static int tap_cell(const VdmConvDesc& d, int t) {
+  return (d.tap_offset[t][0] + 1) * 9 + (d.tap_offset[t][1] + 1) * 3 + d.tap_offset[t][2] + 1;
+}
+
+// Launch plan of one conv layer: schedule, tiling, pipeline depths and shared-memory layout.  Host arithmetic only (the
+// descriptor's ranges are checked by the caller); returns VDM_OK, or the code and message the layer is refused with.
+static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, bool has_xf, int skip_c_in, int sms,
+                     ConvPlan& pl) {
+  const ConvOverrides& ov = g_overrides;
+  pl = ConvPlan{};
+  pl.debug_flags = ov.debug_flags;
+  int pad = 0;
+  for (int t = 0; t < d.n_taps; ++t)
+    if (d.tap_offset[t][0] != 0 || d.tap_offset[t][1] != 0 || d.tap_offset[t][2] != 0) pad = 1;
+  if (has_xf && d.circular) {
+    set_error("vdm_conv3d: the fused input transform is not available with circular padding");
+    return VDM_E_UNSUPPORTED;
   }
-  p.m_nseg = nseg_best;
-  p.m_seglen = ceil_div(d.depth, nseg_best);
-  const long long units = cols * p.m_nseg;
-  VDM_CHECK_ARG(units < (1ll << 31), "vdm_conv3d: too many units");
-  p.m_units = (int)units;
-  const int stage_bytes = planes * (kTileH + 2) * (kTileW + 2) * 16;
-  int off = kMarchStages * stage_bytes + 27 * planes * NF * 16 + p.skip_w_bytes + (int)sizeof(MarchShared) + 2 * kMEpiWarps * NF * 4 +
-            2 * NF * 8 + kMarchCaddMax * 4;
-  off = (off + 15) & ~15;
-  p.res_depth = 0;
+  if (has_skip && (skip_c_in > 64 || d.out_fp32)) {
+    set_error("vdm_conv3d: the fused skip conv supports bf16 layers with skip_c_in <= 64 only (got %d)", skip_c_in);
+    return VDM_E_UNSUPPORTED;
+  }
+  const int xf_bytes = has_xf ? ((d.c_in * 8 + 15) & ~15) : 0;      // (a, b) table of one sample
+  const int skip_w_bytes = has_skip ? skip_c_in * d.c_out_pad * 2 : 0;
+
+  // ---- schedule ----
+  // kd-folded schedules (issue_fold_tile): the full 3x3x3 stencil on a narrow layer
+  bool fold = d.n_taps == 27 && pad == 1 && (d.c_out_pad == 16 || d.c_out_pad == 32 || d.c_out_pad == 64) && d.depth >= 3 &&
+              ov.no_fold == 0 && ov.force_mt == 0 && ov.force_nsplit == 0;
+  const bool streamed = d.c_out_pad == 64;
+  int fold_mt = 0, fold_kc = 0;
+  if (fold && streamed) {
+    // N = 3*64: weights streamed per (chunk, kh, kw); MT = 4 (2 x 4 x 64 = all 512 TMEM columns), 32-channel chunks
+    fold = d.c_in % 32 == 0 && d.depth >= 4;
+    fold_mt = 4; fold_kc = 32;
+  } else if (fold) {
+    // all weights resident + two halo stages must fit; prefer tall tiles (halo efficiency), then wide chunks
+    const int budget = 227 * 1024 - 1024 - (int)sizeof(ConvShared) - (2 * 2 * 8 * d.c_out_pad * 4 + 2 * d.c_out_pad * 8) - 256 -
+                       (has_residual ? 2 * kResSlotBytes : 0) - xf_bytes;      // room for at least two residual slots
+    const int w_bytes = 27 * d.c_in * d.c_out_pad * 2 + skip_w_bytes;
+    for (int m = 4; m >= 2 && !fold_mt; --m)
+      for (int c = 32; c >= 16 && !fold_mt; c -= 16) {
+        if (d.c_in % c != 0 || (has_skip && skip_c_in % c != 0)) continue;
+        const int a_stage = (((c / 8) * (m + 2) * (kTileH + 2) * (kTileW + 2) * 16) + 127) & ~127;
+        if (2 * a_stage + w_bytes <= budget) { fold_mt = m; fold_kc = c; }
+      }
+    // (r02j: re-streaming the weights per tile so that a 96 -> 32 layer could use MT = 4 tiles instead of MT = 2 was
+    // slower, 4.42 vs 3.05 ms at 128^3 x 8: the 6 KB (chunk, kh, kw) stages are dominated by their hand-off cost.)
+    fold = fold_mt != 0;
+  }
+  if (fold) {   // every cell of the stencil exactly once
+    unsigned seen = 0;
+    for (int t = 0; t < 27; ++t) seen |= 1u << tap_cell(d, t);
+    fold = seen == (1u << 27) - 1u;
+  }
+  pl.schedule = !fold ? ConvSchedule::kTile : streamed ? ConvSchedule::kFoldStreamed
+              : d.c_in == fold_kc && ov.no_march == 0 ? ConvSchedule::kMarch : ConvSchedule::kFoldResident;
+  const bool resident_fold = pl.schedule == ConvSchedule::kFoldResident || pl.schedule == ConvSchedule::kMarch;
+
+  // ---- tiling ----
+  const int tiles_w = ceil_div(d.width, kTileW), tiles_h = ceil_div(d.height, kTileH);
+  int n_split = 1, mt = fold_mt;
+  if (!fold) {
+    // Pick (n_split, MT) with a small cost model: a CTA tile costs max(tensor time, L2->SM time) and the
+    // grid runs in ceil(tiles / SMs) waves.  n_split shares one spatial tile between CTAs that each
+    // compute c_out_pad / n_split output channels (more CTAs for the coarse levels); MT d-slices
+    // per tile amortise the halo and the weight stream (fewer, fatter tiles).
+    double best = -1.0;
+    for (int ns = 1; ns <= 8; ns *= 2) {
+      if (d.c_out_pad % (ns * 16) != 0) break;
+      const int ncta = d.c_out_pad / ns;
+      if (ns > 1 && ncta < 32) break;
+      int mt_max = 256 / ncta;
+      if (mt_max > 4) mt_max = 4;
+      if (mt_max > d.depth) mt_max = d.depth;
+      for (int m = 1; m <= mt_max; ++m) {
+        const long long tiles = (long long)tiles_w * tiles_h * ceil_div(d.depth, m) * d.batch * ns;
+        const long long waves = (tiles + sms - 1) / sms;
+        const double active = (double)(tiles < sms ? tiles : sms);
+        // one MMA (M = 128, K = 16): max(tensor time N/2, shared-memory operand fetch (4 KB of A + 32 B per row of B) at
+        // 128 B/clk): N = 32 / 64 are fetch-bound (40 / 48 cycles), N >= 128 tensor-bound (R2r sweep: with the old
+        // max(N/2, 24) the model preferred N = 64, MT = 4 over N = 128, MT = 2 and lost ~15% on every wide layer)
+        const double fetch_cyc = 32.0 + ncta / 4.0;
+        const double mma_cyc = (double)d.n_taps * (d.c_in / 16) * m * (ncta / 2.0 > fetch_cyc ? ncta / 2.0 : fetch_cyc);
+        const double bytes = (double)(m + 2 * pad) * (kTileH + 2 * pad) * (kTileW + 2 * pad) * d.c_in * 2.0 +
+                             (double)d.n_taps * d.c_in * ncta * 2.0;
+        double bw = 5500.0 / active;  // L2 -> SM bytes per cycle per SM when `active` SMs pull at once
+        if (bw > 64.0) bw = 64.0;
+        const double cyc = (mma_cyc > bytes / bw ? mma_cyc : bytes / bw) + 2000.0;  // + per-tile fixed cost
+        const double total = (double)waves * cyc;
+        if (best < 0.0 || total < best * 0.999) {
+          best = total;
+          n_split = ns;
+          mt = m;
+        }
+      }
+    }
+  }
+  if (ov.force_nsplit > 0) n_split = ov.force_nsplit;
+  VDM_CHECK_ARG(d.c_out_pad % (n_split * 16) == 0, "vdm_conv3d: n_split=%d does not divide c_out_pad=%d", n_split,
+                d.c_out_pad);
+  const int n_cta = d.c_out_pad / n_split;
+  if (ov.force_mt > 0) mt = ov.force_mt;
+  VDM_CHECK_ARG(mt >= 1 && 2 * mt * n_cta <= 512, "vdm_conv3d: MT=%d does not fit TMEM with N=%d", mt, n_cta);
+  const long long n_tiles = (long long)tiles_w * tiles_h * ceil_div(d.depth, mt) * d.batch * n_split;
+  VDM_CHECK_ARG(n_tiles < (1ll << 31), "vdm_conv3d: too many tiles");
+  if (has_skip && !resident_fold) {
+    set_error("vdm_conv3d: the fused skip conv needs the kd-folded schedule with resident weights "
+              "(3x3x3, c_out_pad 16 or 32, weights + skip weights fit shared memory); c_in=%d c_out=%d", d.c_in, d.c_out);
+    return VDM_E_UNSUPPORTED;
+  }
+  pl.pad = pad; pl.mt = mt; pl.n_split = n_split; pl.n_cta = n_cta; pl.n_tiles = (int)n_tiles;
+  pl.taps_per_stage = (d.n_taps % 3 == 0) ? 3 : 1;   // one (kd, kh) row of filter taps per weight stage
+
+  if (pl.schedule == ConvSchedule::kMarch) {
+    // Segment length: static round-robin over equal units, so the launch takes ceil(units / SMs) rounds of (seglen + 2) slices
+    // (+1: per-unit fixed costs); short segments balance the SMs, long ones amortise the two halo slices.
+    const long long cols = (long long)d.batch * tiles_h * tiles_w;
+    int nseg_best = 1;
+    double best = -1.0;
+    for (int nseg = 1; nseg <= ceil_div(d.depth, 4); ++nseg) {
+      const int seglen = ceil_div(d.depth, nseg);
+      if (ceil_div(d.depth, seglen) != nseg) continue;
+      const long long rounds = (cols * nseg + sms - 1) / sms;
+      const double cost = (double)rounds * (seglen + 3);
+      if (best < 0.0 || cost < best * 0.999) { best = cost; nseg_best = nseg; }
+    }
+    const long long units = cols * nseg_best;
+    VDM_CHECK_ARG(units < (1ll << 31), "vdm_conv3d: too many units");
+    pl.kc = fold_kc;
+    pl.m_nseg = nseg_best;
+    pl.m_seglen = ceil_div(d.depth, nseg_best);
+    pl.m_units = (int)units;
+    const int stage_bytes = (fold_kc / 8) * (kTileH + 2) * (kTileW + 2) * 16;
+    int off = kMarchStages * stage_bytes + 27 * (fold_kc / 8) * n_cta * 16 + skip_w_bytes + (int)sizeof(MarchShared) +
+              2 * kMEpiWarps * n_cta * 4 + 2 * n_cta * 8 + kMarchCaddMax * 4;
+    off = (off + 15) & ~15;
+    if (has_residual) {
+      pl.res_ring_off = off;
+      pl.res_depth = kMarchResDepth;
+      off += kMarchResDepth * (n_cta / 8) * kMEpiThreads * 16;
+    }
+    pl.smem_bytes = (size_t)off + 1024;
+    VDM_CHECK_ARG(pl.smem_bytes <= 227 * 1024, "vdm_conv3d: marching layer does not fit shared memory");
+    pl.grid = pl.m_units < sms ? pl.m_units : sms;
+    return VDM_OK;
+  }
+
+  // ---- shared memory plan: halo stages + weights (resident, or a ring of stages) + residual ring ----
+  const int plane_bytes = (mt + 2 * pad) * (kTileH + 2 * pad) * (kTileW + 2 * pad) * 16;
+  const int stat_part_bytes = 2 * 2 * 8 * n_cta * 4 + 2 * n_cta * 8;    // partials + running sums
+  const int smem_total = 227 * 1024 - 1024 /*alignment slack*/ - (int)sizeof(ConvShared) - stat_part_bytes - 256 - xf_bytes;
+  // layers with a residual keep a cp.async ring of it in shared memory: 4 units deep where the weights are streamed
+  // anyway, at least 2 where they are resident (the fold search above left room)
+  const int smem_budget = smem_total - (has_residual ? (resident_fold ? 2 : 4) * kResSlotBytes : 0);
+  if (fold) {
+    pl.kc = fold_kc;
+    pl.a_stage_bytes = ((fold_kc / 8) * plane_bytes + 127) & ~127;
+  }
+  if (pl.schedule == ConvSchedule::kFoldStreamed) {
+    pl.b_stage_bytes = 3 * fold_kc * n_cta * 2;
+    pl.nsb = (smem_budget - 2 * pl.a_stage_bytes) / pl.b_stage_bytes;
+    if (pl.nsb > kMaxBStages) pl.nsb = kMaxBStages;
+    VDM_CHECK_ARG(pl.nsb >= 2, "vdm_conv3d: folded streamed layer does not fit shared memory");
+  } else if (pl.schedule == ConvSchedule::kFoldResident) {
+    pl.b_stage_bytes = d.n_taps * d.c_in * n_cta * 2;
+    pl.nsb = 1;
+    pl.b_resident = 1;
+    VDM_CHECK_ARG(2 * pl.a_stage_bytes + pl.b_stage_bytes + skip_w_bytes <= smem_budget,
+                  "vdm_conv3d: folded layer does not fit shared memory");
+  } else {
+    for (int c : {64, 32, 16}) {   // the widest channel chunk for which two halo and two weight stages fit
+      if ((ov.force_kc > 0 && c != ov.force_kc) || d.c_in % c != 0) continue;
+      const int a_stage = ((c / 8) * plane_bytes + 127) & ~127;
+      const int b_stage = pl.taps_per_stage * c * n_cta * 2;
+      const int room = smem_budget - 2 * a_stage;
+      if (room < 2 * b_stage) continue;
+      const long long all_b = (long long)d.n_taps * d.c_in * n_cta * 2;
+      pl.kc = c;
+      pl.a_stage_bytes = a_stage;
+      pl.b_stage_bytes = b_stage;
+      pl.b_resident = (n_split == 1 && all_b <= room && ov.no_resident == 0) ? 1 : 0;
+      pl.nsb = pl.b_resident ? (int)((all_b + b_stage - 1) / b_stage) : (room / b_stage > kMaxBStages ? kMaxBStages : room / b_stage);
+      break;
+    }
+    VDM_CHECK_ARG(pl.kc > 0, "vdm_conv3d: no channel-chunk size fits shared memory (c_in=%d, N=%d, MT=%d)", d.c_in, n_cta, mt);
+  }
+  VDM_CHECK_ARG(plane_bytes <= 0x3FFF * 16, "vdm_conv3d: halo plane too large for the descriptor stride field");
+
+  // Halo stages: two are planned above; layers whose weights leave room get up to kMaxAStages.  A TMA box takes
+  // several thousand cycles to arrive from L2 / HBM, and where a chunk's MMAs are shorter than that (conv_in: 54 MMAs per
+  // tile, the 1x1x1 convs) two stages left the tensor core waiting for loads.
+  const int fixed = pl.nsb * pl.b_stage_bytes + skip_w_bytes + (has_residual ? 4 * kResSlotBytes : 0);
+  pl.nsa = 2;
+  while (pl.nsa < kMaxAStages && (pl.nsa + 1) * pl.a_stage_bytes + fixed <= smem_total) ++pl.nsa;
+  const int used = pl.nsa * pl.a_stage_bytes + pl.nsb * pl.b_stage_bytes + skip_w_bytes;
   if (has_residual) {
-    p.res_ring_off = off;
-    p.res_depth = kMarchResDepth;
-    off += kMarchResDepth * (NF / 8) * kMEpiThreads * 16;
+    const int depth = (smem_total - used) / kResSlotBytes;
+    pl.res_depth = depth > 4 ? 4 : depth;
+    VDM_CHECK_ARG(pl.res_depth >= 1, "vdm_conv3d: no shared memory left for the residual ring");
+    pl.res_ring_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 15) & ~15;
   }
-  const size_t smem_bytes = (size_t)off + 1024;
-  VDM_CHECK_ARG(smem_bytes <= 227 * 1024, "vdm_conv3d: marching layer does not fit shared memory");
-  CUtensorMap tmx;
-  {
-    const cuuint64_t Dx = d.depth + 2 * halo, Hx = d.height + 2 * halo, Wx = d.width + 2 * halo;
-    cuuint64_t gdim[4] = {Wx * 8, Hx, Dx, (cuuint64_t)d.batch * x_planes};
-    cuuint64_t gstr[3] = {Wx * 16, Hx * Wx * 16, Dx * Hx * Wx * 16};
-    cuuint32_t box[4] = {(cuuint32_t)(kTileW + 2) * 8, (cuuint32_t)(kTileH + 2), 1u, (cuuint32_t)planes};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tmx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), gdim, gstr, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d: cuTensorMapEncodeTiled(x, marching) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
-  }
-  CUtensorMap tmx2 = tmx;
-  if (p.skip_chunks > 0) {     // fused 1x1x1 skip conv: one d-slice of the tile's own face per stage (no halo)
-    const cuuint64_t V = (cuuint64_t)d.depth * d.height * d.width;
-    cuuint64_t gdim[4] = {(cuuint64_t)d.width * 8, (cuuint64_t)d.height, (cuuint64_t)d.depth, (cuuint64_t)d.batch * p.x2_planes};
-    cuuint64_t gstr[3] = {(cuuint64_t)d.width * 16, (cuuint64_t)d.height * d.width * 16, V * 16};
-    cuuint32_t box[4] = {(cuuint32_t)kTileW * 8, (cuuint32_t)kTileH, 1u, (cuuint32_t)planes};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tmx2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(skip_x), gdim, gstr, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d: cuTensorMapEncodeTiled(skip_x, marching) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
-  }
-  const int grid = p.m_units < sms ? p.m_units : sms;
-  int rc = VDM_E_UNSUPPORTED;
-#define VDM_LAUNCH_MARCH(KJv, NFv, SKv, XFv)                                                                   \
-  if (kc == 16 * KJv && NF == NFv && (p.skip_chunks > 0) == SKv && (in_norm != nullptr) == XFv) {              \
-    static bool configured = false;                                                                            \
-    if (!configured) {                                                                                         \
-      VDM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_march_kernel<KJv, NFv, SKv, XFv>,                             \
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));          \
-      configured = true;                                                                                       \
-    }                                                                                                          \
-    conv3d_march_kernel<KJv, NFv, SKv, XFv><<<grid, kConvThreads, smem_bytes, stream>>>(tmx, tmx2, p);         \
-    rc = VDM_OK;                                                                                               \
-  }
-#define VDM_LAUNCH_MARCH4(SKv, XFv)                                                                            \
-  VDM_LAUNCH_MARCH(1, 16, SKv, XFv) VDM_LAUNCH_MARCH(1, 32, SKv, XFv) VDM_LAUNCH_MARCH(2, 16, SKv, XFv) VDM_LAUNCH_MARCH(2, 32, SKv, XFv)
-  VDM_LAUNCH_MARCH4(false, false) VDM_LAUNCH_MARCH4(true, false) VDM_LAUNCH_MARCH4(false, true) VDM_LAUNCH_MARCH4(true, true)
-#undef VDM_LAUNCH_MARCH4
-#undef VDM_LAUNCH_MARCH
-  if (rc != VDM_OK) {
-    set_error("vdm_conv3d: no marching kernel instance for KC=%d N=%d", kc, NF);
-    return rc;
-  }
-  VDM_CHECK_LAUNCH();
+  pl.xf_coef_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 16 + pl.res_depth * kResSlotBytes + 15) & ~15;
+  pl.smem_bytes = (size_t)pl.xf_coef_off + xf_bytes + 1024;
+  pl.grid = pl.n_tiles < sms ? pl.n_tiles : sms;
   return VDM_OK;
+}
+
+// The kernel instance of a plan.  Every instance compiled into the library is listed here.
+static int launch_conv(const ConvPlan& pl, const CUtensorMap& tmx, const CUtensorMap& tmx2, const ConvKernelParams& p,
+                       cudaStream_t stream) {
+  if (pl.schedule == ConvSchedule::kMarch) {
+    const bool sk = p.skip_chunks > 0, xf = p.in_norm != nullptr;
+#define VDM_MARCH(KJv, NFv, SKv, XFv)                                                                          \
+    if (pl.kc == 16 * KJv && pl.n_cta == NFv && sk == SKv && xf == XFv)                                        \
+      return launch_kernel<conv3d_march_kernel<KJv, NFv, SKv, XFv>>(pl.grid, kConvThreads, pl.smem_bytes, stream, tmx, tmx2, p);
+#define VDM_MARCH4(SKv, XFv) VDM_MARCH(1, 16, SKv, XFv) VDM_MARCH(1, 32, SKv, XFv) VDM_MARCH(2, 16, SKv, XFv) VDM_MARCH(2, 32, SKv, XFv)
+    VDM_MARCH4(false, false) VDM_MARCH4(true, false) VDM_MARCH4(false, true) VDM_MARCH4(true, true)
+#undef VDM_MARCH4
+#undef VDM_MARCH
+    set_error("vdm_conv3d: no marching kernel instance for KC=%d N=%d", pl.kc, pl.n_cta);
+    return VDM_E_UNSUPPORTED;
+  }
+  const int nf = pl.schedule == ConvSchedule::kTile ? 0 : pl.n_cta;
+#define VDM_TILE(MTv, KJv, NFv)                                                                                \
+  if (pl.mt == MTv && pl.kc == 16 * KJv && nf == NFv)                                                          \
+    return launch_kernel<conv3d_planar_kernel<MTv, KJv, NFv>>(pl.grid, kConvThreads, pl.smem_bytes, stream, tmx, tmx2, p);
+  VDM_TILE(1, 1, 0) VDM_TILE(1, 2, 0) VDM_TILE(1, 4, 0)
+  VDM_TILE(2, 1, 0) VDM_TILE(2, 2, 0) VDM_TILE(2, 4, 0)
+  VDM_TILE(3, 1, 0) VDM_TILE(3, 2, 0) VDM_TILE(3, 4, 0)
+  VDM_TILE(4, 1, 0) VDM_TILE(4, 2, 0) VDM_TILE(4, 4, 0)
+  VDM_TILE(4, 1, 16) VDM_TILE(4, 1, 32) VDM_TILE(4, 2, 16) VDM_TILE(4, 2, 32) VDM_TILE(4, 2, 64)
+  VDM_TILE(3, 1, 16) VDM_TILE(3, 1, 32) VDM_TILE(3, 2, 16) VDM_TILE(3, 2, 32)
+  VDM_TILE(2, 1, 16) VDM_TILE(2, 1, 32) VDM_TILE(2, 2, 16) VDM_TILE(2, 2, 32)
+#undef VDM_TILE
+  set_error("vdm_conv3d: no kernel instance for MT=%d KC=%d", pl.mt, pl.kc);
+  return VDM_E_UNSUPPORTED;
 }
 
 }  // namespace vdm
@@ -1307,13 +1458,13 @@ using namespace vdm;
 extern "C" int vdm_debug_set(int key, int value) {
   switch (key) {
     case 0: return VDM_OK;   /* retired knob (LBO/SBO swap) */
-    case 1: g_debug_force_mt = value; return VDM_OK;
-    case 2: g_debug_force_kc = value; return VDM_OK;
-    case 3: g_debug_force_nsplit = value; return VDM_OK;
-    case 4: g_debug_no_resident = value; return VDM_OK;
-    case 5: g_debug_flags = value; return VDM_OK;
-    case 6: g_debug_no_fold = value; return VDM_OK;
-    case 7: g_debug_no_march = value; return VDM_OK;
+    case 1: g_overrides.force_mt = value; return VDM_OK;
+    case 2: g_overrides.force_kc = value; return VDM_OK;
+    case 3: g_overrides.force_nsplit = value; return VDM_OK;
+    case 4: g_overrides.no_resident = value; return VDM_OK;
+    case 5: g_overrides.debug_flags = value; return VDM_OK;
+    case 6: g_overrides.no_fold = value; return VDM_OK;
+    case 7: g_overrides.no_march = value; return VDM_OK;
     default: set_error("vdm_debug_set: unknown key %d", key); return VDM_E_BADARG;
   }
 }
@@ -1341,208 +1492,70 @@ extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w,
                     (reinterpret_cast<uintptr_t>(y) & 15) == 0,
                 "vdm_conv3d: pointers must be 16-byte aligned");
   VDM_CHECK_ARG((long long)d.batch * x_planes < (1ll << 31), "vdm_conv3d: too many planes");
-  auto encode = get_encode_fn();
-  if (!encode) {
+  for (int t = 0; t < d.n_taps; ++t)
+    for (int k = 0; k < 3; ++k)
+      VDM_CHECK_ARG(d.tap_offset[t][k] >= -1 && d.tap_offset[t][k] <= 1, "vdm_conv3d: tap offset out of range");
+  const bool has_residual = epi && epi->residual;
+  const bool has_skip = epi && epi->skip_x;
+  const bool has_xf = epi && epi->in_norm;
+  VDM_CHECK_ARG(!has_skip || (epi->skip_w && epi->skip_c_in >= 16 && epi->skip_c_in % 16 == 0),
+                "vdm_conv3d: fused skip conv needs packed weights and skip_c_in a multiple of 16, got %d", epi->skip_c_in);
+  if (!encode_fn()) {
     set_error("vdm_conv3d: cuTensorMapEncodeTiled is not available from the driver");
     return VDM_E_DRIVER;
   }
 
+  ConvPlan pl;
+  const int rc = plan_conv(d, has_residual, has_skip, has_xf, has_skip ? epi->skip_c_in : 0, num_sms(), pl);
+  if (rc != VDM_OK) return rc;
+  // (checked after planning: a layer the planner refuses reports VDM_E_UNSUPPORTED, which callers answer with a fallback)
+  const int x2_planes = !has_skip ? 0 : epi->skip_planes > 0 ? epi->skip_planes : epi->skip_c_in / 8;
+  VDM_CHECK_ARG(!has_skip || (epi->skip_plane0 >= 0 && epi->skip_plane0 + epi->skip_c_in / 8 <= x2_planes),
+                "vdm_conv3d: skip plane window out of range");
+  VDM_CHECK_ARG(!(epi && epi->stats && d.out_fp32), "vdm_conv3d: stats are only produced for bf16 outputs");
+  VDM_CHECK_ARG(!(has_residual && d.out_fp32), "vdm_conv3d: residual is only supported for bf16 outputs");
+  VDM_CHECK_ARG(!(has_residual && epi->residual_upsample) || (d.depth % 2 == 0 && d.height % 2 == 0 && d.width % 2 == 0),
+                "vdm_conv3d: an up-sampled residual needs an even grid, got (%d,%d,%d)", d.depth, d.height, d.width);
+  const bool march = pl.schedule == ConvSchedule::kMarch;
+
   ConvKernelParams p;
   memset(&p, 0, sizeof(p));
   p.B = d.batch; p.D = d.depth; p.H = d.height; p.W = d.width;
-  p.c_out = d.c_out; p.n_pad = d.c_out_pad; p.n_taps = d.n_taps;
-  int pad = 0;
-  for (int t = 0; t < d.n_taps; ++t)
-    for (int k = 0; k < 3; ++k) {
-      VDM_CHECK_ARG(d.tap_offset[t][k] >= -1 && d.tap_offset[t][k] <= 1, "vdm_conv3d: tap offset out of range");
-      if (d.tap_offset[t][k] != 0) pad = 1;
-    }
-  p.pad = pad;
-  const bool has_residual = epi && epi->residual;
-  const bool has_skip = epi && epi->skip_x;
-  const bool has_xf = epi && epi->in_norm;
-  if (has_xf && d.circular) {
-    set_error("vdm_conv3d: the fused input transform is not available with circular padding");
-    return VDM_E_UNSUPPORTED;
-  }
-  const int xf_bytes = has_xf ? ((d.c_in * 8 + 15) & ~15) : 0;      // (a, b) table of one sample
-  if (has_skip) {
-    VDM_CHECK_ARG(epi->skip_w && epi->skip_c_in >= 16 && epi->skip_c_in % 16 == 0,
-                  "vdm_conv3d: fused skip conv needs packed weights and skip_c_in a multiple of 16, got %d", epi->skip_c_in);
-    if (epi->skip_c_in > 64 || d.out_fp32) {
-      set_error("vdm_conv3d: the fused skip conv supports bf16 layers with skip_c_in <= 64 only (got %d)", epi->skip_c_in);
-      return VDM_E_UNSUPPORTED;
-    }
-  }
-  const int skip_w_bytes = has_skip ? epi->skip_c_in * d.c_out_pad * 2 : 0;
-  // kd-folded schedule (issue_fold_tile): the full 3x3x3 stencil on a narrow layer
-  bool fold = d.n_taps == 27 && pad == 1 && d.c_in % 16 == 0 && (d.c_out_pad == 16 || d.c_out_pad == 32 || d.c_out_pad == 64) &&
-              d.depth >= 3 && g_debug_no_fold == 0 && g_debug_force_mt == 0 && g_debug_force_nsplit == 0;
-  int fold_mt = 0, fold_kc = 0, fold_streamed = 0;
-  if (fold && d.c_out_pad == 64) {
-    // N = 3*64: weights streamed per (chunk, kh, kw); MT = 4 (2 x 4 x 64 = all 512 TMEM columns), 32-channel chunks
-    fold = d.c_in % 32 == 0 && d.depth >= 4 && g_debug_no_fold < 2;
-    fold_mt = 4; fold_kc = 32; fold_streamed = 1;
-  } else if (fold) {
-    // all weights resident + two halo stages must fit; prefer tall tiles (halo efficiency), then wide chunks
-    const int budget = 227 * 1024 - 1024 - (int)sizeof(ConvShared) - (2 * 2 * 8 * d.c_out_pad * 4 + 2 * d.c_out_pad * 8) - 256 -
-                       (has_residual ? 2 * kResSlotBytes : 0) - xf_bytes;      // room for at least two residual slots
-    const int w_bytes = 27 * d.c_in * d.c_out_pad * 2 + skip_w_bytes;
-    for (int m = 4; m >= 2 && !fold_mt; --m)
-      for (int c = 32; c >= 16 && !fold_mt; c -= 16) {
-        if (d.c_in % c != 0 || (has_skip && epi->skip_c_in % c != 0)) continue;
-        const int a_stage = (((c / 8) * (m + 2) * (kTileH + 2) * (kTileW + 2) * 16) + 127) & ~127;
-        if (2 * a_stage + w_bytes <= budget) { fold_mt = m; fold_kc = c; }
-      }
-    // (r02j: re-streaming the weights per tile so that a 96 -> 32 layer could use MT = 4 tiles instead of MT = 2 was
-    // slower, 4.42 vs 3.05 ms at 128^3 x 8: the 6 KB (chunk, kh, kw) stages are dominated by their hand-off cost.)
-    fold = fold_mt != 0;
-  }
-  if (fold) {
-    unsigned seen = 0;
-    for (int t = 0; t < 27; ++t) {
-      const int kd = d.tap_offset[t][0] + 1, khw = (d.tap_offset[t][1] + 1) * 3 + d.tap_offset[t][2] + 1;
-      p.tap_kd[t] = (int8_t)kd;
-      p.tap_khw[t] = (int8_t)khw;
-      seen |= 1u << (kd * 9 + khw);
-    }
-    fold = seen == (1u << 27) - 1u;
-    for (int t = 0; t < 27; ++t) p.tap_of[p.tap_kd[t]][p.tap_khw[t]] = (int8_t)t;
-  }
-  p.c_in8 = d.c_in / 8;
-  p.x_planes = x_planes; p.x_plane0 = d.x_plane0;
-  p.x_shift = halo;
-
-  // ---- tiling ----
-  p.tiles_w = ceil_div(d.width, kTileW);
-  p.tiles_h = ceil_div(d.height, kTileH);
-  // Pick (n_split, MT) with a small cost model: a CTA tile costs max(tensor time, L2->SM time) and the
-  // grid runs in ceil(tiles / SMs) waves.  n_split shares one spatial tile between CTAs that each
-  // compute c_out_pad / n_split output channels (more CTAs for the coarse levels); MT d-slices
-  // per tile amortise the halo and the weight stream (fewer, fatter tiles).
-  int n_split = 1, mt = 1;
-  {
-    double best = -1.0;
-    const int sms = num_sms();
-    for (int ns = 1; ns <= 8; ns *= 2) {
-      if (d.c_out_pad % (ns * 16) != 0) break;
-      const int ncta = d.c_out_pad / ns;
-      if (ns > 1 && ncta < 32) break;
-      int mt_max = 256 / ncta;
-      if (mt_max > 4) mt_max = 4;
-      if (mt_max > d.depth) mt_max = d.depth;
-      for (int m = 1; m <= mt_max; ++m) {
-        const long long tiles = (long long)p.tiles_w * p.tiles_h * ceil_div(d.depth, m) * d.batch * ns;
-        const long long waves = (tiles + sms - 1) / sms;
-        const double active = (double)(tiles < sms ? tiles : sms);
-        // one MMA (M = 128, K = 16): max(tensor time N/2, shared-memory operand fetch (4 KB of A + 32 B per row of B) at
-        // 128 B/clk): N = 32 / 64 are fetch-bound (40 / 48 cycles), N >= 128 tensor-bound (R2r sweep: with the old
-        // max(N/2, 24) the model preferred N = 64, MT = 4 over N = 128, MT = 2 and lost ~15% on every wide layer)
-        const double fetch_cyc = 32.0 + ncta / 4.0;
-        const double mma_cyc = (double)d.n_taps * (d.c_in / 16) * m * (ncta / 2.0 > fetch_cyc ? ncta / 2.0 : fetch_cyc);
-        const double bytes = (double)(m + 2 * pad) * (kTileH + 2 * pad) * (kTileW + 2 * pad) * d.c_in * 2.0 +
-                             (double)d.n_taps * d.c_in * ncta * 2.0;
-        double bw = 5500.0 / active;  // L2 -> SM bytes per cycle per SM when `active` SMs pull at once
-        if (bw > 64.0) bw = 64.0;
-        const double cyc = (mma_cyc > bytes / bw ? mma_cyc : bytes / bw) + 2000.0;  // + per-tile fixed cost
-        const double total = (double)waves * cyc;
-        if (best < 0.0 || total < best * 0.999) {
-          best = total;
-          n_split = ns;
-          mt = m;
-        }
-      }
-    }
-  }
-  if (fold) {
-    n_split = 1;
-    mt = fold_mt;
-  }
-  if (g_debug_force_nsplit > 0) n_split = g_debug_force_nsplit;
-  VDM_CHECK_ARG(d.c_out_pad % (n_split * 16) == 0, "vdm_conv3d: n_split=%d does not divide c_out_pad=%d", n_split,
-                d.c_out_pad);
-  p.n_split = n_split;
-  p.n_cta = d.c_out_pad / n_split;
-  if (g_debug_force_mt > 0) mt = g_debug_force_mt;
-  VDM_CHECK_ARG(mt >= 1 && 2 * mt * p.n_cta <= 512, "vdm_conv3d: MT=%d does not fit TMEM with N=%d", mt, p.n_cta);
-  p.MT = mt;
-  p.tiles_d = ceil_div(d.depth, mt);
-  const long long n_tiles = (long long)p.tiles_w * p.tiles_h * p.tiles_d * d.batch * n_split;
-  VDM_CHECK_ARG(n_tiles < (1ll << 31), "vdm_conv3d: too many tiles");
-  p.n_tiles = (int)n_tiles;
-  p.fast_div_ok = n_tiles < (1ll << 22) ? 1 : 0;
-  p.inv_n_split = 1.0f / (float)n_split; p.inv_tiles_w = 1.0f / (float)p.tiles_w;
+  p.c_out = d.c_out; p.n_pad = d.c_out_pad; p.n_taps = d.n_taps; p.pad = pl.pad;
+  p.n_split = pl.n_split; p.n_cta = pl.n_cta;
+  p.MT = pl.mt; p.KC = pl.kc; p.k_chunks = d.c_in / pl.kc;
+  p.tiles_w = ceil_div(d.width, kTileW); p.tiles_h = ceil_div(d.height, kTileH); p.tiles_d = ceil_div(d.depth, pl.mt);
+  p.n_tiles = pl.n_tiles;
+  p.fast_div_ok = pl.n_tiles < (1 << 22) ? 1 : 0;
+  p.inv_n_split = 1.0f / (float)pl.n_split; p.inv_tiles_w = 1.0f / (float)p.tiles_w;
   p.inv_tiles_h = 1.0f / (float)p.tiles_h; p.inv_tiles_d = 1.0f / (float)p.tiles_d;
-  p.Hd = mt + 2 * pad; p.Hh = kTileH + 2 * pad; p.Wh = kTileW + 2 * pad;
+  p.Hd = pl.mt + 2 * pl.pad; p.Hh = kTileH + 2 * pl.pad; p.Wh = kTileW + 2 * pl.pad;
   p.plane_bytes = p.Hd * p.Hh * p.Wh * 16;
   for (int t = 0; t < d.n_taps; ++t)
-    p.tap16[t] = (uint16_t)(((d.tap_offset[t][0] + pad) * p.Hh + (d.tap_offset[t][1] + pad)) * p.Wh + d.tap_offset[t][2] + pad);
-
-  // ---- shared memory plan: 2 halo stages + a ring of weight stages ----
-  const int stat_part_bytes = 2 * 2 * 8 * p.n_cta * 4 + 2 * p.n_cta * 8;    // partials + running sums
-  const int smem_total = 227 * 1024 - 1024 /*alignment slack*/ - (int)sizeof(ConvShared) - stat_part_bytes - 256 - xf_bytes;
-  // layers with a residual keep a cp.async ring of it in shared memory: 4 units deep where the weights are streamed
-  // anyway, at least 2 where they are resident (the fold search above left room)
-  const int smem_budget = smem_total - (has_residual ? (fold && !fold_streamed ? 2 : 4) * kResSlotBytes : 0);
-  int kc = 0, nsb = 0;
-  const int tps = (d.n_taps % 3 == 0) ? 3 : 1;   // one (kd, kh) row of filter taps per weight stage
-  const int kc_options[3] = {64, 32, 16};
-  if (fold && fold_streamed) {
-    kc = fold_kc;
-    p.a_stage_bytes = ((kc / 8) * p.plane_bytes + 127) & ~127;
-    p.b_stage_bytes = 3 * kc * p.n_cta * 2;
-    nsb = (smem_budget - 2 * p.a_stage_bytes) / p.b_stage_bytes;
-    if (nsb > kMaxBStages) nsb = kMaxBStages;
-    VDM_CHECK_ARG(nsb >= 2, "vdm_conv3d: folded streamed layer does not fit shared memory");
-    p.b_resident = 0;
-    p.fold_streamed = 1;
-  } else if (fold) {
-    kc = fold_kc;
-    p.a_stage_bytes = ((kc / 8) * p.plane_bytes + 127) & ~127;
-    p.b_stage_bytes = d.n_taps * d.c_in * p.n_cta * 2;
-    nsb = 1;
-    p.b_resident = 1;
-    VDM_CHECK_ARG(2 * p.a_stage_bytes + p.b_stage_bytes + skip_w_bytes <= smem_budget,
-                  "vdm_conv3d: folded layer does not fit shared memory");
-    if (has_skip) {
-      p.skip_chunks = epi->skip_c_in / kc;
-      p.skip_w_bytes = skip_w_bytes;
-      p.w2 = static_cast<const __nv_bfloat16*>(epi->skip_w);
-      p.x2_planes = epi->skip_planes > 0 ? epi->skip_planes : epi->skip_c_in / 8;
-      p.x2_plane0 = epi->skip_plane0;
-      VDM_CHECK_ARG(p.x2_plane0 >= 0 && p.x2_plane0 + epi->skip_c_in / 8 <= p.x2_planes, "vdm_conv3d: skip plane window out of range");
+    p.tap16[t] = (uint16_t)(((d.tap_offset[t][0] + pl.pad) * p.Hh + (d.tap_offset[t][1] + pl.pad)) * p.Wh + d.tap_offset[t][2] + pl.pad);
+  if (pl.schedule != ConvSchedule::kTile)
+    for (int t = 0; t < 27; ++t) {
+      const int c = tap_cell(d, t);
+      p.tap_kd[t] = (int8_t)(c / 9);
+      p.tap_khw[t] = (int8_t)(c % 9);
+      p.tap_of[c / 9][c % 9] = (int8_t)t;
     }
-  }
-  if (has_skip && !(fold && !fold_streamed)) {
-    set_error("vdm_conv3d: the fused skip conv needs the kd-folded schedule with resident weights "
-              "(3x3x3, c_out_pad 16 or 32, weights + skip weights fit shared memory); c_in=%d c_out=%d", d.c_in, d.c_out);
-    return VDM_E_UNSUPPORTED;
-  }
-  for (int o = 0; o < 3 && !fold; ++o) {
-    const int c = kc_options[o];
-    if (g_debug_force_kc > 0 && c != g_debug_force_kc) continue;
-    if (d.c_in % c != 0) continue;
-    const int a_stage = ((c / 8) * p.plane_bytes + 127) & ~127;
-    const int b_stage = tps * c * p.n_cta * 2;
-    const int room = smem_budget - 2 * a_stage;
-    if (room < 2 * b_stage) continue;
-    kc = c;
-    nsb = room / b_stage;
-    const long long all_b = (long long)d.n_taps * d.c_in * p.n_cta * 2;
-    p.b_resident = (n_split == 1 && all_b <= room && g_debug_no_resident == 0) ? 1 : 0;
-    if (p.b_resident) nsb = (int)((all_b + b_stage - 1) / b_stage);
-    else if (nsb > kMaxBStages) nsb = kMaxBStages;
-    p.a_stage_bytes = a_stage;
-    p.b_stage_bytes = b_stage;
-    break;
-  }
-  p.taps_per_stage = tps;
-  VDM_CHECK_ARG(kc > 0, "vdm_conv3d: no channel-chunk size fits shared memory (c_in=%d, N=%d, MT=%d)", d.c_in, p.n_cta, mt);
-  p.KC = kc; p.k_chunks = d.c_in / kc; p.nsb = nsb;
-  VDM_CHECK_ARG(p.plane_bytes <= 0x3FFF * 16, "vdm_conv3d: halo plane too large for the descriptor stride field");
+  p.fold_streamed = pl.schedule == ConvSchedule::kFoldStreamed ? 1 : 0;
+  p.nsa = pl.nsa; p.nsb = pl.nsb; p.taps_per_stage = pl.taps_per_stage;
+  p.a_stage_bytes = pl.a_stage_bytes; p.b_stage_bytes = pl.b_stage_bytes; p.b_resident = pl.b_resident;
   int cols = 32;
-  while (cols < 2 * mt * p.n_cta) cols <<= 1;
+  while (cols < 2 * pl.mt * pl.n_cta) cols <<= 1;
   p.tmem_cols = cols;
+  p.c_in = d.c_in; p.c_in8 = d.c_in / 8;
+  p.x_planes = x_planes; p.x_plane0 = d.x_plane0;
+  p.x_shift = halo;
+  if (has_skip) {
+    p.skip_chunks = epi->skip_c_in / pl.kc;
+    p.skip_w_bytes = epi->skip_c_in * d.c_out_pad * 2;
+    p.w2 = static_cast<const __nv_bfloat16*>(epi->skip_w);
+    p.x2_planes = x2_planes;
+    p.x2_plane0 = epi->skip_plane0;
+  }
   p.w = static_cast<const __nv_bfloat16*>(w);
   p.y = y; p.y_planes = y_planes; p.y_plane0 = d.y_plane0; p.out_fp32 = d.out_fp32;
   if (epi) {
@@ -1557,100 +1570,28 @@ extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w,
     p.stats = epi->stats;
     p.stats_channels = epi->stats_channels > 0 ? epi->stats_channels : d.c_out;
     p.stats_c0 = epi->stats_c0;
+    p.in_norm = epi->in_norm;   // fused GroupNorm + SiLU of the input (warps 12..15)
   }
-  VDM_CHECK_ARG(!(p.stats && d.out_fp32), "vdm_conv3d: stats are only produced for bf16 outputs");
-  VDM_CHECK_ARG(!(p.residual && d.out_fp32), "vdm_conv3d: residual is only supported for bf16 outputs");
-  VDM_CHECK_ARG(!p.r_up || (d.depth % 2 == 0 && d.height % 2 == 0 && d.width % 2 == 0),
-                "vdm_conv3d: an up-sampled residual needs an even grid, got (%d,%d,%d)", d.depth, d.height, d.width);
-  p.debug_flags = g_debug_flags;
-
-  // d-marching schedule for the narrow layers whose input channels are one chunk (conv3d_march.cuh)
-  if (fold && !fold_streamed && p.k_chunks == 1 && g_debug_no_march == 0)
-    return launch_march(d, p, x, has_skip ? epi->skip_x : nullptr, has_xf ? epi->in_norm : nullptr, kc, halo, x_planes, has_residual,
-                        encode, stream);
+  p.res_depth = pl.res_depth; p.res_ring_off = pl.res_ring_off; p.xf_coef_off = pl.xf_coef_off;
+  p.m_units = pl.m_units; p.m_nseg = pl.m_nseg; p.m_seglen = pl.m_seglen;
+  p.debug_flags = pl.debug_flags;
 
   // activations: 4-D (W*8 channels-in-plane, H, D, B*planes), box (Wh*8, Hh, Hd, KC/8); out-of-bounds -> zeros.
   // The (w, 8ch) pair is ONE tensor-map dimension on purpose: the TMA unit issues requests per
   // innermost box row, and a 16-byte row (8 channels as their own dimension) capped the r01 kernel at
   // one 32-byte sector per ~9 cycles per SM (profiles/r01_conv_ncu.txt).  Rows are Wh*16 = 160 bytes now.
-  CUtensorMap tmx;
-  {
-    const cuuint64_t Dx = d.depth + 2 * halo, Hx = d.height + 2 * halo, Wx = d.width + 2 * halo;
-    const cuuint64_t V = Dx * Hx * Wx;
-    cuuint64_t gdim[4] = {Wx * 8, Hx, Dx, (cuuint64_t)d.batch * x_planes};
-    cuuint64_t gstr[3] = {Wx * 16, Hx * Wx * 16, V * 16};
-    cuuint32_t box[4] = {(cuuint32_t)p.Wh * 8, (cuuint32_t)p.Hh, (cuuint32_t)p.Hd, (cuuint32_t)(kc / 8)};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tmx, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(x), gdim, gstr, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d: cuTensorMapEncodeTiled(x) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
+  // The marching kernel loads one d-slice per stage.
+  const uint32_t box_d = march ? 1u : (uint32_t)p.Hd, planes = (uint32_t)(pl.kc / 8);
+  CUtensorMap tmx, tmx2;
+  int e = encode_planar(&tmx, x, d.width + 2 * halo, d.height + 2 * halo, d.depth + 2 * halo, (uint64_t)d.batch * x_planes,
+                        0, {(uint32_t)p.Wh, (uint32_t)p.Hh, box_d, planes}, "vdm_conv3d", march ? "x, marching" : "x");
+  if (e != VDM_OK) return e;
+  tmx2 = tmx;
+  if (has_skip) {   // fused 1x1x1 skip conv: the tile's own voxels, no halo
+    e = encode_planar(&tmx2, epi->skip_x, d.width, d.height, d.depth, (uint64_t)d.batch * x2_planes, 0,
+                      {(uint32_t)kTileW, (uint32_t)kTileH, march ? 1u : (uint32_t)pl.mt, planes}, "vdm_conv3d",
+                      march ? "skip_x, marching" : "skip_x");
+    if (e != VDM_OK) return e;
   }
-
-  CUtensorMap tmx2 = tmx;
-  if (p.skip_chunks > 0) {
-    const cuuint64_t V = (cuuint64_t)d.depth * d.height * d.width;
-    cuuint64_t gdim[4] = {(cuuint64_t)d.width * 8, (cuuint64_t)d.height, (cuuint64_t)d.depth, (cuuint64_t)d.batch * p.x2_planes};
-    cuuint64_t gstr[3] = {(cuuint64_t)d.width * 16, (cuuint64_t)d.height * d.width * 16, V * 16};
-    cuuint32_t box[4] = {(cuuint32_t)kTileW * 8, (cuuint32_t)kTileH, (cuuint32_t)mt, (cuuint32_t)(kc / 8)};   // no halo
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tmx2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(epi->skip_x), gdim, gstr, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d: cuTensorMapEncodeTiled(skip_x) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
-  }
-
-  // Halo stages: two are planned above; layers whose weights leave room get up to kMaxAStages.  A TMA box takes
-  // several thousand cycles to arrive from L2 / HBM, and where a chunk's MMAs are shorter than that (conv_in: 54 MMAs per
-  // tile, the 1x1x1 convs) two stages left the tensor core waiting for loads.
-  p.nsa = 2;
-  {
-    const int fixed = p.nsb * p.b_stage_bytes + p.skip_w_bytes + (has_residual ? 4 * kResSlotBytes : 0);
-    while (p.nsa < kMaxAStages && (p.nsa + 1) * p.a_stage_bytes + fixed <= smem_total) ++p.nsa;
-  }
-  const int used = p.nsa * p.a_stage_bytes + p.nsb * p.b_stage_bytes + p.skip_w_bytes;
-  if (has_residual) {
-    int depth = (smem_total - used) / kResSlotBytes;
-    p.res_depth = depth > 4 ? 4 : depth;
-    VDM_CHECK_ARG(p.res_depth >= 1, "vdm_conv3d: no shared memory left for the residual ring");
-    p.res_ring_off = used + (int)sizeof(ConvShared) + stat_part_bytes;
-    p.res_ring_off = (p.res_ring_off + 15) & ~15;
-  }
-  p.xf_coef_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 16 + p.res_depth * kResSlotBytes + 15) & ~15;
-  p.in_norm = has_xf ? epi->in_norm : nullptr;
-  p.c_in = d.c_in;
-  const size_t smem_bytes = (size_t)p.xf_coef_off + xf_bytes + 1024;
-  const int grid = p.n_tiles < num_sms() ? p.n_tiles : num_sms();
-  int rc = VDM_E_UNSUPPORTED;
-#define VDM_LAUNCH(MTv, KJv, NFv)                                                                              \
-  if (mt == MTv && kc == 16 * KJv && (fold ? p.n_cta : 0) == NFv) {                                            \
-    static bool configured = false;                                                                            \
-    if (!configured) {                                                                                         \
-      VDM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_planar_kernel<MTv, KJv, NFv>,                                 \
-                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));          \
-      configured = true;                                                                                       \
-    }                                                                                                          \
-    conv3d_planar_kernel<MTv, KJv, NFv><<<grid, kConvThreads, smem_bytes, stream>>>(tmx, tmx2, p);                   \
-    rc = VDM_OK;                                                                                               \
-  }
-  VDM_LAUNCH(1, 1, 0) VDM_LAUNCH(1, 2, 0) VDM_LAUNCH(1, 4, 0)
-  VDM_LAUNCH(2, 1, 0) VDM_LAUNCH(2, 2, 0) VDM_LAUNCH(2, 4, 0)
-  VDM_LAUNCH(3, 1, 0) VDM_LAUNCH(3, 2, 0) VDM_LAUNCH(3, 4, 0)
-  VDM_LAUNCH(4, 1, 0) VDM_LAUNCH(4, 2, 0) VDM_LAUNCH(4, 4, 0)
-  VDM_LAUNCH(4, 1, 16) VDM_LAUNCH(4, 1, 32) VDM_LAUNCH(4, 2, 16) VDM_LAUNCH(4, 2, 32) VDM_LAUNCH(4, 2, 64)
-  VDM_LAUNCH(3, 1, 16) VDM_LAUNCH(3, 1, 32) VDM_LAUNCH(3, 2, 16) VDM_LAUNCH(3, 2, 32)
-  VDM_LAUNCH(2, 1, 16) VDM_LAUNCH(2, 1, 32) VDM_LAUNCH(2, 2, 16) VDM_LAUNCH(2, 2, 32)
-#undef VDM_LAUNCH
-  if (rc != VDM_OK) {
-    set_error("vdm_conv3d: no kernel instance for MT=%d KC=%d", mt, kc);
-    return rc;
-  }
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return launch_conv(pl, tmx, tmx2, p, stream);
 }

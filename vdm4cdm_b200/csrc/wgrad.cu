@@ -20,10 +20,9 @@
 // Pipeline per CTA (6 warps): warp 0 TMA producer (halo slices of a + one tile of g per stage),
 // warp 1 MMA issuer (jobs x 8 K-steps of 16 voxels per tile), warps 2-5 final TMEM -> atomics.
 // Roofline: tensor-bound, algorithmic FLOPs = 2 * taps * Cin * Cout * B*D*H*W (same as the forward).
-#include <cudaTypedefs.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
+#include "tma_host.cuh"
 
 namespace vdm {
 
@@ -445,156 +444,53 @@ conv3d_wgrad_narrow_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
   }
 }
 
-static PFN_cuTensorMapEncodeTiled_v12000 wg_encode_fn() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = []() -> PFN_cuTensorMapEncodeTiled_v12000 {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return nullptr;
-    return reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(ptr);
-  }();
-  return fn;
-}
+// Launch plan of one weight-gradient layer: which kernel, its blocking, pipeline depth, grid and shared memory, written
+// into the kernel's parameters (the caller adds the operands).  Host arithmetic only.
+struct WgradPlan {
+  bool narrow;            // conv3d_wgrad_narrow_kernel (3x3x3, c_out <= 32) with `np`, else conv3d_wgrad_kernel with `gp`
+  WgradNarrowParams np;
+  WgradParams gp;
+  int grid;
+  size_t smem_bytes;
+};
 
-static int wg_num_sms() {
-  static int n = []() {
-    int dev = 0, v = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return kNumSMs;
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) return kNumSMs;
-    return v;
-  }();
-  return n;
-}
-
-static int g_wgrad_no_narrow = 0;
-
-static int launch_wgrad_narrow(const VdmWgradDesc& d, const void* a, const void* g, float* dw, int x_planes, int g_planes,
-                               int c_out16, PFN_cuTensorMapEncodeTiled_v12000 encode, cudaStream_t stream) {
-  WgradNarrowParams p;
-  memset(&p, 0, sizeof(p));
-  p.B = d.batch; p.D = d.depth; p.H = d.height; p.W = d.width;
-  p.c_in = d.c_in; p.c_out = d.c_out; p.n = c_out16;
-  int cpb = 32;
-  while (d.c_in % cpb != 0) cpb >>= 1;          // 32 or 16 (c_in is a multiple of 16)
-  p.cpb = cpb; p.S = 128 / cpb; p.n_cblocks = d.c_in / cpb;
-  p.n_slots = kWnLen + p.S - 1;
-  p.tiles_w = ceil_div(d.width, kWgTileW);
-  p.tiles_h = ceil_div(d.height, kWgTileH);
-  p.segs_d = ceil_div(d.depth, kWnLen);
-  const long long n_segs = (long long)d.batch * p.tiles_h * p.tiles_w * p.segs_d;
-  VDM_CHECK_ARG(n_segs < (1ll << 31), "vdm_conv3d_wgrad: too many segments");
-  p.n_segs = (int)n_segs;
-  int n_splits = wg_num_sms() / p.n_cblocks;
-  if (n_splits < 1) n_splits = 1;
-  if (n_splits > p.n_segs) n_splits = p.n_segs;
-  p.n_splits = n_splits;
-  p.slice_bytes = (cpb / 8) * (kWgTileH + 2) * (kWgTileW + 2) * 16;
-  p.g_tile_bytes = p.n * kWgTileH * kWgTileW * 2;
-  p.g_stage_bytes = 3 * p.g_tile_bytes;
-  p.x_planes = x_planes; p.x_plane0 = d.a_plane0;
-  p.a_shift = d.a_padded ? 1 : 0;
-  p.g_shift = d.g_padded ? 1 : 0;
-  p.g_planes = g_planes; p.g_plane0 = d.g_plane0;
-  p.dw = dw;
-  if (d.dw_stride_tap == 0 && d.dw_stride_ci == 0 && d.dw_stride_co == 0) {
-    p.st_tap = (long long)d.c_in * d.c_out; p.st_ci = d.c_out; p.st_co = 1; p.c_in_real = d.c_in;
-  } else {
-    VDM_CHECK_ARG(d.c_in_real >= 1 && d.c_in_real <= d.c_in, "vdm_conv3d_wgrad: c_in_real=%d out of [1, c_in]", d.c_in_real);
-    p.st_tap = d.dw_stride_tap; p.st_ci = d.dw_stride_ci; p.st_co = d.dw_stride_co; p.c_in_real = d.c_in_real;
-  }
-  const size_t smem_bytes = (size_t)p.n_slots * p.slice_bytes + (size_t)kWnGStages * p.g_stage_bytes +
-                            sizeof(WgradNarrowShared) + 1024;
-  VDM_CHECK_ARG(smem_bytes <= 227 * 1024, "vdm_conv3d_wgrad: narrow-layer plan needs %zu bytes of shared memory", smem_bytes);
-  CUtensorMap tma, tmg[3];
-  {
-    const cuuint64_t ah = d.a_padded ? 1 : 0;         // `a` with a one-voxel periodic halo: padded dims
-    const cuuint64_t Da = d.depth + 2 * ah, Ha = d.height + 2 * ah, Wa = d.width + 2 * ah;
-    cuuint64_t gdim[4] = {Wa * 8, Ha, Da, (cuuint64_t)d.batch * x_planes};
-    cuuint64_t gstr_a[3] = {Wa * 16, Ha * Wa * 16, Da * Ha * Wa * 16};
-    cuuint32_t box[4] = {(cuuint32_t)(kWgTileW + 2) * 8, (cuuint32_t)(kWgTileH + 2), 1u, (cuuint32_t)(cpb / 8)};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a), gdim, gstr_a, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled(a) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
-    // g: logical dims (W, H, D) always (positions beyond the grid read zeros); with a periodic halo the window
-    // of copy kw starts (2 - kw) voxels into the padded row (see the kernel), else all three maps are the same.
-    const cuuint64_t gh = d.g_padded ? 1 : 0;
-    const cuuint64_t Dg = d.depth + 2 * gh, Hg = d.height + 2 * gh, Wg = d.width + 2 * gh;
-    cuuint64_t gdim2[4] = {(cuuint64_t)d.width * 8, (cuuint64_t)d.height, (cuuint64_t)d.depth, (cuuint64_t)d.batch * g_planes};
-    cuuint64_t gstr_g[3] = {Wg * 16, Hg * Wg * 16, Dg * Hg * Wg * 16};
-    cuuint32_t box2[4] = {(cuuint32_t)kWgTileW * 8, (cuuint32_t)kWgTileH, 1u, (cuuint32_t)(p.n / 8)};
-    for (int kw = 0; kw < 3; ++kw) {
-      const char* base = static_cast<const char*>(g) + (gh ? ((Hg + 1) * Wg + (cuuint64_t)(2 - kw)) * 16 : 0);
-      r = encode(&tmg[kw], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<char*>(base), gdim2, gstr_g, box2, estr,
-                 CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (r != CUDA_SUCCESS) {
-        set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled(g) failed with %d", (int)r);
-        return VDM_E_DRIVER;
-      }
-    }
-  }
-  static bool configured = false;
-  if (!configured) {
-    VDM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_wgrad_narrow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    configured = true;
-  }
-  conv3d_wgrad_narrow_kernel<<<p.n_cblocks * p.n_splits, kWnThreads, smem_bytes, stream>>>(tma, tmg[0], tmg[1], tmg[2], p);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
-}
-
-}  // namespace vdm
-
-using namespace vdm;
-
-extern "C" int vdm_wgrad_debug_set(int key, int value) {
-  if (key == 0) { g_wgrad_no_narrow = value; return VDM_OK; }
-  set_error("vdm_wgrad_debug_set: unknown key %d", key);
-  return VDM_E_BADARG;
-}
-
-extern "C" int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const void* g, float* dw, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  VDM_CHECK_ARG(desc && a && g && dw, "vdm_conv3d_wgrad: NULL pointer argument");
-  const VdmWgradDesc& d = *desc;
-  VDM_CHECK_ARG(d.batch >= 1 && d.depth >= 1 && d.height >= 1 && d.width >= 1, "vdm_conv3d_wgrad: bad grid");
-  VDM_CHECK_ARG(d.c_in >= 16 && d.c_in % 16 == 0, "vdm_conv3d_wgrad: c_in=%d must be a multiple of 16", d.c_in);
-  VDM_CHECK_ARG(d.c_out >= 1 && d.c_out <= 256, "vdm_conv3d_wgrad: c_out=%d out of [1,256]", d.c_out);
-  VDM_CHECK_ARG(d.kernel == 3 || d.kernel == 1, "vdm_conv3d_wgrad: kernel size %d (3 or 1 supported)", d.kernel);
-  VDM_CHECK_ARG(!(d.kernel == 3 && d.a_padded && !d.g_padded), "vdm_conv3d_wgrad: a periodic `a` needs a periodic g (g_padded)");
-  const int x_planes = d.a_planes > 0 ? d.a_planes : d.c_in / 8;
-  const int c_out16 = (d.c_out + 15) / 16 * 16;
-  const int g_planes = d.g_planes > 0 ? d.g_planes : c_out16 / 8;
-  VDM_CHECK_ARG(d.a_plane0 >= 0 && d.a_plane0 + d.c_in / 8 <= x_planes, "vdm_conv3d_wgrad: a plane window out of range");
-  VDM_CHECK_ARG(d.g_plane0 >= 0 && d.g_plane0 + c_out16 / 8 <= g_planes,
-                "vdm_conv3d_wgrad: g plane window out of range (g must hold c_out rounded up to 16 channels)");
-  VDM_CHECK_ARG((reinterpret_cast<uintptr_t>(a) & 15) == 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0,
-                "vdm_conv3d_wgrad: pointers must be 16-byte aligned");
-  auto encode = wg_encode_fn();
-  if (!encode) {
-    set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled is not available from the driver");
-    return VDM_E_DRIVER;
+static int plan_wgrad(const VdmWgradDesc& d, int c_out16, int sms, WgradPlan& pl) {
+  pl = WgradPlan{};
+  pl.narrow = d.kernel == 3 && c_out16 <= 32 && d.depth >= 2;
+  if (pl.narrow) {
+    WgradNarrowParams& p = pl.np;
+    p.n = c_out16;
+    int cpb = 32;
+    while (d.c_in % cpb != 0) cpb >>= 1;          // 32 or 16 (c_in is a multiple of 16)
+    p.cpb = cpb; p.S = 128 / cpb; p.n_cblocks = d.c_in / cpb;
+    p.n_slots = kWnLen + p.S - 1;
+    p.tiles_w = ceil_div(d.width, kWgTileW);
+    p.tiles_h = ceil_div(d.height, kWgTileH);
+    p.segs_d = ceil_div(d.depth, kWnLen);
+    const long long n_segs = (long long)d.batch * p.tiles_h * p.tiles_w * p.segs_d;
+    VDM_CHECK_ARG(n_segs < (1ll << 31), "vdm_conv3d_wgrad: too many segments");
+    p.n_segs = (int)n_segs;
+    int n_splits = sms / p.n_cblocks;
+    if (n_splits < 1) n_splits = 1;
+    if (n_splits > p.n_segs) n_splits = p.n_segs;
+    p.n_splits = n_splits;
+    p.slice_bytes = (cpb / 8) * (kWgTileH + 2) * (kWgTileW + 2) * 16;
+    p.g_tile_bytes = p.n * kWgTileH * kWgTileW * 2;
+    p.g_stage_bytes = 3 * p.g_tile_bytes;
+    pl.smem_bytes = (size_t)p.n_slots * p.slice_bytes + (size_t)kWnGStages * p.g_stage_bytes + sizeof(WgradNarrowShared) + 1024;
+    VDM_CHECK_ARG(pl.smem_bytes <= 227 * 1024, "vdm_conv3d_wgrad: narrow-layer plan needs %zu bytes of shared memory",
+                  pl.smem_bytes);
+    pl.grid = p.n_cblocks * p.n_splits;
+    return VDM_OK;
   }
 
-  if (d.kernel == 3 && c_out16 <= 32 && d.depth >= 2 && g_wgrad_no_narrow == 0)
-    return launch_wgrad_narrow(d, a, g, dw, x_planes, g_planes, c_out16, encode, stream);
-
-  WgradParams p;
-  memset(&p, 0, sizeof(p));
-  p.B = d.batch; p.D = d.depth; p.H = d.height; p.W = d.width;
-  p.c_in = d.c_in; p.c_out = d.c_out;
+  WgradParams& p = pl.gp;
   p.kd_count = d.kernel; p.pad = d.kernel == 3 ? 1 : 0;
   p.n_khw = d.kernel * d.kernel;
   p.Hh = kWgTileH + 2 * p.pad; p.Wh = kWgTileW + 2 * p.pad;
   int cpb = 128;
   while (d.c_in % cpb != 0) cpb >>= 1;
-  p.cpb = cpb; p.S = 128 / cpb; p.n_cblocks = d.c_in / cpb;
+  p.S = 128 / cpb;
   int over_read = 0;
   if (d.kernel == 1) {
     // 1x1x1: there is no filter plane to fold into M, and the layer is HBM-bound: load each `a` slice ONCE.  One block
@@ -603,9 +499,10 @@ extern "C" int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const v
     // (r01r: 0.38 ms for the 96->32 skip conv with S = 4 slices loaded per tile, 4x its HBM floor.)
     cpb = 128;
     while (d.c_in % cpb != 0) cpb -= 16;
-    p.cpb = cpb; p.S = 1; p.n_cblocks = d.c_in / cpb;
+    p.S = 1;
     over_read = 16 * kWgTileH * kWgTileW * 16;
   }
+  p.cpb = cpb; p.n_cblocks = d.c_in / cpb;
   p.n_sblocks = (p.kd_count + p.S - 1) / p.S;
   p.n_jobs_total = p.n_sblocks * p.n_khw;
   p.n_split = c_out16 > 128 ? 2 : 1;
@@ -624,8 +521,7 @@ extern "C" int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const v
   VDM_CHECK_ARG(n_tiles < (1ll << 31), "vdm_conv3d_wgrad: too many tiles");
   p.n_tiles = (int)n_tiles;
   p.slice_bytes = (cpb / 8) * p.Hh * p.Wh * 16;
-  const int n_slices = p.n_sblocks * p.S;
-  p.a_stage_bytes = (n_slices * p.slice_bytes + 127) & ~127;
+  p.a_stage_bytes = (p.n_sblocks * p.S * p.slice_bytes + 127) & ~127;
   p.g_stage_bytes = p.n * kWgTileH * kWgTileW * 2;
   const int budget = 227 * 1024 - 1024 - (int)sizeof(WgradShared) - 256 - over_read;
   int stages = budget / (p.a_stage_bytes + p.g_stage_bytes);
@@ -635,69 +531,89 @@ extern "C" int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const v
   p.stages = stages;
   VDM_CHECK_ARG(16 * p.Hh * p.Wh <= 0x3FFF, "vdm_conv3d_wgrad: operand block too large for the descriptor");
   const int units = p.n_cblocks * p.n_jgroups * p.n_split;
-  int n_splits = (2 * wg_num_sms()) / units;          // about two CTAs' worth of work units per SM ...
+  int n_splits = (2 * sms) / units;          // about two CTAs' worth of work units per SM ...
   if (n_splits < 1) n_splits = 1;
   if (n_splits > p.n_tiles) n_splits = p.n_tiles;     // ... but at least one tile each
-  if (units * n_splits > wg_num_sms() && n_splits > 1) {
+  if (units * n_splits > sms && n_splits > 1) {
     // prefer exactly one wave when that keeps >= 8 tiles per CTA
-    const int one_wave = wg_num_sms() / units;
+    const int one_wave = sms / units;
     if (one_wave >= 1 && p.n_tiles / one_wave >= 8) n_splits = one_wave;
   }
   p.n_splits = n_splits;
-  p.x_planes = x_planes; p.x_plane0 = d.a_plane0;
-  p.a_shift = d.a_padded ? 1 : 0;
-  p.g_shift = d.g_padded ? 1 : 0;
-  p.g_planes = g_planes; p.g_plane0 = d.g_plane0;
-  p.dw = dw;
-  if (d.dw_stride_tap == 0 && d.dw_stride_ci == 0 && d.dw_stride_co == 0) {
-    p.st_tap = (long long)d.c_in * d.c_out; p.st_ci = d.c_out; p.st_co = 1; p.c_in_real = d.c_in;
-  } else {
-    VDM_CHECK_ARG(d.c_in_real >= 1 && d.c_in_real <= d.c_in, "vdm_conv3d_wgrad: c_in_real=%d out of [1, c_in]", d.c_in_real);
-    p.st_tap = d.dw_stride_tap; p.st_ci = d.dw_stride_ci; p.st_co = d.dw_stride_co; p.c_in_real = d.c_in_real;
+  pl.smem_bytes = (size_t)p.stages * (p.a_stage_bytes + p.g_stage_bytes) + sizeof(WgradShared) + 1024 + over_read;
+  pl.grid = units * n_splits;
+  return VDM_OK;
+}
+
+}  // namespace vdm
+
+using namespace vdm;
+
+extern "C" int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const void* g, float* dw, void* stream_) {
+  cudaStream_t stream = (cudaStream_t)stream_;
+  VDM_CHECK_ARG(desc && a && g && dw, "vdm_conv3d_wgrad: NULL pointer argument");
+  const VdmWgradDesc& d = *desc;
+  VDM_CHECK_ARG(d.batch >= 1 && d.depth >= 1 && d.height >= 1 && d.width >= 1, "vdm_conv3d_wgrad: bad grid");
+  VDM_CHECK_ARG(d.c_in >= 16 && d.c_in % 16 == 0, "vdm_conv3d_wgrad: c_in=%d must be a multiple of 16", d.c_in);
+  VDM_CHECK_ARG(d.c_out >= 1 && d.c_out <= 256, "vdm_conv3d_wgrad: c_out=%d out of [1,256]", d.c_out);
+  VDM_CHECK_ARG(d.kernel == 3 || d.kernel == 1, "vdm_conv3d_wgrad: kernel size %d (3 or 1 supported)", d.kernel);
+  VDM_CHECK_ARG(!(d.kernel == 3 && d.a_padded && !d.g_padded), "vdm_conv3d_wgrad: a periodic `a` needs a periodic g (g_padded)");
+  const int x_planes = d.a_planes > 0 ? d.a_planes : d.c_in / 8;
+  const int c_out16 = (d.c_out + 15) / 16 * 16;
+  const int g_planes = d.g_planes > 0 ? d.g_planes : c_out16 / 8;
+  VDM_CHECK_ARG(d.a_plane0 >= 0 && d.a_plane0 + d.c_in / 8 <= x_planes, "vdm_conv3d_wgrad: a plane window out of range");
+  VDM_CHECK_ARG(d.g_plane0 >= 0 && d.g_plane0 + c_out16 / 8 <= g_planes,
+                "vdm_conv3d_wgrad: g plane window out of range (g must hold c_out rounded up to 16 channels)");
+  VDM_CHECK_ARG((reinterpret_cast<uintptr_t>(a) & 15) == 0 && (reinterpret_cast<uintptr_t>(g) & 15) == 0,
+                "vdm_conv3d_wgrad: pointers must be 16-byte aligned");
+  const bool dense_dw = d.dw_stride_tap == 0 && d.dw_stride_ci == 0 && d.dw_stride_co == 0;
+  VDM_CHECK_ARG(dense_dw || (d.c_in_real >= 1 && d.c_in_real <= d.c_in), "vdm_conv3d_wgrad: c_in_real=%d out of [1, c_in]",
+                d.c_in_real);
+  if (!encode_fn()) {
+    set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled is not available from the driver");
+    return VDM_E_DRIVER;
   }
 
-  CUtensorMap tma, tmg;
-  {
-    const cuuint64_t ah = d.a_padded ? 1 : 0;         // `a` with a one-voxel periodic halo: padded dims
-    const cuuint64_t Da = d.depth + 2 * ah, Ha = d.height + 2 * ah, Wa = d.width + 2 * ah;
-    cuuint64_t gdim[4] = {Wa * 8, Ha, Da, (cuuint64_t)d.batch * x_planes};
-    cuuint64_t gstr_a[3] = {Wa * 16, Ha * Wa * 16, Da * Ha * Wa * 16};
-    cuuint32_t box[4] = {(cuuint32_t)p.Wh * 8, (cuuint32_t)p.Hh, 1u, (cuuint32_t)(cpb / 8)};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = encode(&tma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a), gdim, gstr_a, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled(a) failed with %d", (int)r);
-      return VDM_E_DRIVER;
+  WgradPlan pl;
+  int e = plan_wgrad(d, c_out16, num_sms(), pl);
+  if (e != VDM_OK) return e;
+  auto set_operands = [&](auto& p) {   // the fields both kernels' parameters share
+    p.B = d.batch; p.D = d.depth; p.H = d.height; p.W = d.width;
+    p.c_in = d.c_in; p.c_out = d.c_out;
+    p.x_planes = x_planes; p.x_plane0 = d.a_plane0;
+    p.a_shift = d.a_padded ? 1 : 0;
+    p.g_shift = d.g_padded ? 1 : 0;
+    p.g_planes = g_planes; p.g_plane0 = d.g_plane0;
+    p.dw = dw;
+    if (dense_dw) {
+      p.st_tap = (long long)d.c_in * d.c_out; p.st_ci = d.c_out; p.st_co = 1; p.c_in_real = d.c_in;
+    } else {
+      p.st_tap = d.dw_stride_tap; p.st_ci = d.dw_stride_ci; p.st_co = d.dw_stride_co; p.c_in_real = d.c_in_real;
     }
-    // g: logical dims (W, H, D) always (positions beyond the grid read zeros); with a periodic halo the window
-    // of copy kw starts (2 - kw) voxels into the padded row (see the kernel), else all three maps are the same.
-    // g: logical dims (W, H, D) (positions beyond the grid read zeros); with a periodic halo the window starts at
-    // the interior of the padded tensor
-    // g: logical dims (W, H, D) (positions beyond the grid read zeros); with a periodic halo the window starts at
-    // the interior of the padded tensor
-    const cuuint64_t gh = d.g_padded ? 1 : 0;
-    const cuuint64_t Dg = d.depth + 2 * gh, Hg = d.height + 2 * gh, Wg = d.width + 2 * gh;
-    cuuint64_t gdim2[4] = {(cuuint64_t)d.width * 8, (cuuint64_t)d.height, (cuuint64_t)d.depth, (cuuint64_t)d.batch * g_planes};
-    cuuint64_t gstr_g[3] = {Wg * 16, Hg * Wg * 16, Dg * Hg * Wg * 16};
-    cuuint32_t box2[4] = {(cuuint32_t)kWgTileW * 8, (cuuint32_t)kWgTileH, 1u, (cuuint32_t)(p.n / 8)};
-    const char* gbase = static_cast<const char*>(g) + (gh ? ((Hg + 1) * Wg + 1) * 16 : 0);
-    r = encode(&tmg, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<char*>(gbase), gdim2, gstr_g, box2, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("vdm_conv3d_wgrad: cuTensorMapEncodeTiled(g) failed with %d", (int)r);
-      return VDM_E_DRIVER;
-    }
+  };
+  if (pl.narrow) set_operands(pl.np);
+  else set_operands(pl.gp);
+
+  // `a` with a one-voxel periodic halo: the padded dims; one d-slice per box
+  const int ah = d.a_padded ? 1 : 0, pad = pl.narrow ? 1 : pl.gp.pad, cpb = pl.narrow ? pl.np.cpb : pl.gp.cpb;
+  CUtensorMap tma, tmg[3];
+  e = encode_planar(&tma, a, d.width + 2 * ah, d.height + 2 * ah, d.depth + 2 * ah, (uint64_t)d.batch * x_planes, 0,
+                    {(uint32_t)(kWgTileW + 2 * pad), (uint32_t)(kWgTileH + 2 * pad), 1u, (uint32_t)(cpb / 8)},
+                    "vdm_conv3d_wgrad", "a");
+  if (e != VDM_OK) return e;
+  // g: logical dims (W, H, D) always (positions beyond the grid read zeros).  With a periodic halo the window starts in
+  // the interior of the padded tensor; the narrow kernel reads three copies, copy kw starting (2 - kw) voxels into the
+  // padded row (see the kernel).  Without one, all three maps are the same.
+  const int gh = d.g_padded ? 1 : 0, n = pl.narrow ? pl.np.n : pl.gp.n;
+  const uint64_t Wg = d.width + 2 * gh, Hg = d.height + 2 * gh;
+  for (int kw = 0; kw < (pl.narrow ? 3 : 1); ++kw) {
+    const char* base = static_cast<const char*>(g) + (gh ? ((Hg + 1) * Wg + (pl.narrow ? 2 - kw : 1)) * 16 : 0);
+    e = encode_planar(&tmg[kw], base, d.width, d.height, d.depth, (uint64_t)d.batch * g_planes, gh,
+                      {(uint32_t)kWgTileW, (uint32_t)kWgTileH, 1u, (uint32_t)(n / 8)}, "vdm_conv3d_wgrad", "g");
+    if (e != VDM_OK) return e;
   }
-  const size_t smem_bytes = (size_t)p.stages * (p.a_stage_bytes + p.g_stage_bytes) + sizeof(WgradShared) + 1024 + over_read;
-  static bool configured = false;
-  if (!configured) {
-    VDM_CHECK_CUDA(cudaFuncSetAttribute(conv3d_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    configured = true;
-  }
-  conv3d_wgrad_kernel<<<units * n_splits, kWgThreads, smem_bytes, stream>>>(tma, tmg, p);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  if (pl.narrow)
+    return launch_kernel<conv3d_wgrad_narrow_kernel>(pl.grid, kWnThreads, pl.smem_bytes, stream, tma, tmg[0], tmg[1], tmg[2],
+                                                     pl.np);
+  return launch_kernel<conv3d_wgrad_kernel>(pl.grid, kWgThreads, pl.smem_bytes, stream, tma, tmg[0], pl.gp);
 }
