@@ -19,6 +19,10 @@
  *   conv weights: bf16 [tap][Cin/8][Cout_pad][8]  (element (tap, ci, co) at
  *                 ((tap*Cin/8 + ci/8)*Cout_pad + co)*8 + ci%8), Cout_pad % 16 == 0
  *   latent z    : fp32 [B][D][H][W] (the reference's (B,1,D,H,W))
+ *   TF32 mode   : the *_tf32 / *_f32 entry points take "fp32 channel-planar" activations [B][C/4][D][H][W][4]: 4 fp32
+ *                 channels = the same 16 bytes per voxel and plane, so plane counts and plane windows (x_planes,
+ *                 VdmTensor.planes, ...) count 4-channel planes there; conv weights are fp32 [tap][Cin/4][Cout_pad][4]
+ *                 (vdm_pack_conv_weight_f32).  vdm_pad_circular copies 16-byte units and works on either layout.
  *   chan stats  : double [B][C][2] = (sum, sum of squares) over the D*H*W voxels
  */
 #ifndef VDM4CDM_B200_H
@@ -115,6 +119,16 @@ typedef struct VdmConvEpilogue {
 VDM_API int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w, void* y,
                const VdmConvEpilogue* epi, void* stream);
 
+/* The same conv at TF32 precision (tcgen05.mma kind::tf32, fp32 accumulate): x, the residual and a planar y are fp32
+ * channel-planar (4 channels per plane; x_planes / y_planes / r_planes and the *_plane0 windows count those planes),
+ * w is vdm_pack_conv_weight_f32's layout; c_in is a multiple of 8.  The epilogue adds chan_add and the residual to the
+ * fp32 accumulator and stores it unrounded; statistics are those of the stored values.  out_fp32 = 1 writes fp32
+ * [B][c_out][D][H][W] as vdm_conv3d does.  in_norm, skip_x and residual_upsample are bf16-only: VDM_E_UNSUPPORTED.
+ * Inference precision option: a TF32 operand keeps 10 mantissa bits against bf16's 7, and activations are never
+ * rounded for storage. */
+VDM_API int vdm_conv3d_tf32(const VdmConvDesc* desc, const void* x, const void* w, void* y,
+                    const VdmConvEpilogue* epi, void* stream);
+
 #ifdef VDM_BRINGUP
 /* NOT part of the release library.  `make -C vdm4cdm_b200/csrc bringup` builds libvdm4cdm_b200_bringup.so with
  * -DVDM_BRINGUP, the only build in which this symbol and the ablation branches of the conv kernel exist
@@ -160,6 +174,10 @@ VDM_API int vdm_conv3d_wgrad(const VdmWgradDesc* desc, const void* a, const void
  * c_in_pad / c_out_pad are the padded sizes of the PACKED tensor's K and N dimensions (multiples of 16). */
 VDM_API int vdm_pack_conv_weight(const float* w, void* packed, int c_out, int c_in, int kernel, int transpose_flip,
                          int ci0, int n_ci, int c_in_pad, int c_out_pad, void* stream);
+/* Forward filter for vdm_conv3d_tf32: fp32 [k^3][c_in_pad/4][c_out_pad][4], every weight rounded to the nearest TF32
+ * value (cvt.rna.tf32.f32), zero padded; c_in_pad a multiple of 8, c_out_pad of 16. */
+VDM_API int vdm_pack_conv_weight_f32(const float* w, void* packed, int c_out, int c_in, int kernel, int c_in_pad,
+                             int c_out_pad, void* stream);
 
 /* The same for a whole network in ONE launch: `jobs_device` is an array of n_jobs descriptors IN DEVICE MEMORY (the
  * arguments of vdm_pack_conv_weight with k3 = kernel^3; pointers must stay valid, e.g. for a captured CUDA graph).
@@ -211,6 +229,11 @@ VDM_API int vdm_gn_silu_step(const VdmTensor* x, const VdmTensor* y, int batch, 
                      const double* stats, const float* gamma, const float* beta, float eps, float dropout_p,
                      uint64_t seed, const int32_t* seed_step, uint32_t layer_tag, void* stream);
 
+/* vdm_gn_silu on fp32 channel-planar views (4 channels per plane; channels a multiple of 4), without dropout.  SiLU is
+ * x / (1 + exp(-x)) in fp32 (not the ~2^-11 hardware tanh of the bf16 passes). */
+VDM_API int vdm_gn_silu_f32(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels, int groups,
+                    const double* stats, const float* gamma, const float* beta, float eps, void* stream);
+
 /* 2x2x2 average pooling of a (depth,height,width) grid; accumulates channel stats of y when stats != NULL. */
 VDM_API int vdm_avgpool2(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
                  int channels, double* stats, int stats_channels, int stats_c0, void* stream);
@@ -220,6 +243,11 @@ VDM_API int vdm_avgpool2(const VdmTensor* x, const VdmTensor* y, int batch, int 
  * Accumulates channel stats of y when stats != NULL. */
 VDM_API int vdm_upsample2(const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height, int width,
                   int channels, double* stats, int stats_channels, int stats_c0, void* stream);
+/* vdm_avgpool2 / vdm_upsample2 on fp32 channel-planar views (statistics of the fp32 values). */
+VDM_API int vdm_avgpool2_f32(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
+                     int channels, double* stats, int stats_channels, int stats_c0, void* stream);
+VDM_API int vdm_upsample2_f32(const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height, int width,
+                      int channels, double* stats, int stats_channels, int stats_c0, void* stream);
 
 /* ---- backward of the fused elementwise passes (autograd's native_group_norm_backward /
  *      silu_backward / dropout mask / avg_pool3d_backward / upsample_nearest3d_backward launches
@@ -302,7 +330,8 @@ VDM_API int vdm_loss_dpred(const float* pred, const float* noise, const float* c
                    int64_t total, void* stream);
 
 /* Periodic one-voxel halo: y[b][p][dp][hp][wp] = x[b][p][(dp-1) mod D][(hp-1) mod H][(wp-1) mod W] for
- * dp in [0, D+2) etc.  x: [B][planes][D][H][W][8] view, y: [B][planes][D+2][H+2][W+2][8] view. */
+ * dp in [0, D+2) etc.  x: [B][planes][D][H][W][8] view, y: [B][planes][D+2][H+2][W+2][8] view.  The kernel copies
+ * 16-byte units: an fp32 channel-planar tensor is padded by passing 2 * its channel count (= 8 * its planes). */
 VDM_API int vdm_pad_circular(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
                      int channels, void* stream);
 
@@ -310,6 +339,10 @@ VDM_API int vdm_pad_circular(const VdmTensor* x, const VdmTensor* y, int batch, 
  * z: fp32 [B][V]; cond: fp32 [B][n_cond][V] (NCDHW) or NULL; out: c_pad/8 planes; n_cond <= 7. */
 VDM_API int vdm_pack_input(const float* z, const float* cond, const VdmTensor* out, int batch, int64_t voxels,
                    int n_cond, int c_pad, void* stream);
+/* The same into an fp32 channel-planar tensor: planes 0 and 1 hold (z, cond_1..cond_n, 0...), the rest are 0;
+ * c_pad a multiple of 8, n_cond <= 7. */
+VDM_API int vdm_pack_input_f32(const float* z, const float* cond, const VdmTensor* out, int batch, int64_t voxels,
+                       int n_cond, int c_pad, void* stream);
 
 /* ---- fused VDM ancestral-sampler update ------------------------------------------------
  * VDM.sample_zs_given_zt (vdm_model.py:370-378): mean = alpha_s/alpha_t*(zt - c*sigma_t*eps_hat),

@@ -50,6 +50,9 @@ def main(mode="CV"):
                     help="smoke runs only: sample from random weights when the configured ckpt_path does not exist "
                          "(default: raise, like the reference's torch.load)")
     ap.add_argument("--configs", default=os.path.join(ROOT, "configs.yaml"))
+    ap.add_argument("--precision", choices=["bf16", "tf32"], default="bf16",
+                    help="denoiser precision: bf16 activations (default) or fp32 activations with TF32 convs, the "
+                         "reference's cuDNN TF32 class of accuracy (A/B comparisons of the generated statistics)")
     args = ap.parse_args()
     if "SFM" in args.model_name:
         raise NotImplementedError("This model is not implemented yet")       # generate_3D.py:16-17
@@ -61,6 +64,8 @@ def main(mode="CV"):
     if rank == 0:
         os.makedirs(args.save_path, exist_ok=True)
     model = utils.get_model(config, device=device, allow_random_init=args.allow_random_init).eval()
+    if args.precision != "bf16":
+        model.model.score_model.precision = args.precision        # the CUNet behind LightVDM -> VDM
     grid = int(config.get("cropsize", 128))
     n_params = int(config.get("conditioning_values", 6))
     if mode == "CV":

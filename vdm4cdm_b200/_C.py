@@ -74,6 +74,12 @@ _SIGNATURES = {
     "vdm_last_error_string": (c_char_p, []),
     "vdm_device_supported": (c_int, [c_int]),
     "vdm_conv3d": (c_int, [POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, POINTER(ConvEpilogue), c_void_p]),
+    "vdm_conv3d_tf32": (c_int, [POINTER(ConvDesc), c_void_p, c_void_p, c_void_p, POINTER(ConvEpilogue), c_void_p]),
+    "vdm_pack_conv_weight_f32": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "vdm_gn_silu_f32": (c_int, [_T, _T, c_int, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_float, c_void_p]),
+    "vdm_avgpool2_f32": (c_int, [_T, _T, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
+    "vdm_upsample2_f32": (c_int, [_T, _T, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_int, c_void_p]),
+    "vdm_pack_input_f32": (c_int, [c_void_p, c_void_p, _T, c_int, c_int64, c_int, c_int, c_void_p]),
     "vdm_conv3d_wgrad": (c_int, [POINTER(WgradDesc), c_void_p, c_void_p, c_void_p, c_void_p]),
     "vdm_pack_conv_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "vdm_pack_conv_weight_batched": (c_int, [c_void_p, c_int, c_void_p]),

@@ -100,6 +100,8 @@ __device__ __forceinline__ bf16x8 ld_stream(const bf16x8* p) {
   return r;
 }
 __device__ __forceinline__ void st_stream(bf16x8* p, const bf16x8& v) { __stcs(reinterpret_cast<uint4*>(p), v.u); }
+__device__ __forceinline__ float4 ld_stream(const float4* p) { return __ldcs(p); }
+__device__ __forceinline__ void st_stream(float4* p, const float4& v) { __stcs(p, v); }
 
 __device__ __forceinline__ float2 bf16pair_to_float2(uint32_t w) {
   return make_float2(__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u));
@@ -127,6 +129,15 @@ __device__ __forceinline__ bf16x8 pack8(const float (&f)[8]) {
   return p;
 }
 
+// The 16-byte unit of a channel-planar tensor as fp32 lanes: 8 bf16 channels, or 4 fp32 channels (the fp32 channel-planar
+// layout [B][C/4][D][H][W][4] of the TF32 inference mode).  Unit<F32>::T is the type, L its channel count.
+template <bool F32> struct Unit { using T = bf16x8; static constexpr int L = 8; };
+template <> struct Unit<true> { using T = float4; static constexpr int L = 4; };
+__device__ __forceinline__ void unpack_unit(const bf16x8& p, float (&f)[8]) { unpack8(p, f); }
+__device__ __forceinline__ void unpack_unit(const float4& p, float (&f)[4]) { f[0] = p.x; f[1] = p.y; f[2] = p.z; f[3] = p.w; }
+__device__ __forceinline__ void pack_unit(const float (&f)[8], bf16x8& p) { p = pack8(f); }
+__device__ __forceinline__ void pack_unit(const float (&f)[4], float4& p) { p = make_float4(f[0], f[1], f[2], f[3]); }
+
 // sigmoid via the hardware tanh (one MUFU op, ~2^-11 relative error: well inside the bf16 the results are stored in).
 // r01m: with exp + full-precision division the GroupNorm/SiLU kernels were issue-bound at 30-50% of the HBM roofline.
 __device__ __forceinline__ float fast_sigmoid(float x) {
@@ -143,6 +154,10 @@ __device__ __forceinline__ float silu_half(float h) {
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(h));
   return fmaf(h, t, h);
 }
+
+// silu in fp32 for the TF32 inference mode: x * sigmoid(x) with an exp-based sigmoid (a few ulp, where the hardware tanh
+// above is ~2^-11 -- the size of a whole TF32 rounding).
+__device__ __forceinline__ float silu_f32(float x) { return x / (1.0f + expf(-x)); }
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

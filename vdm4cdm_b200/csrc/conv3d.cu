@@ -497,11 +497,17 @@ __device__ __forceinline__ void transform_tiles(const ConvKernelParams& p, ConvS
 // bias row of a chunk lives in registers for the whole tile, the TMEM load of unit i+1 is issued before unit i is
 // processed, output pointers advance by adds, and shared memory is addressed as shared memory.
 constexpr int kEpiRes = 1, kEpiStats = 2, kEpiFp32 = 4;
+// fp32 channel-planar output [B][C/4][D][H][W][4] (the TF32 instances): a 16-channel unit is four 16-byte planes, the
+// residual is read in the same layout, and the statistics are those of the stored, un-rounded fp32 values.
+constexpr int kEpiF32Planar = 8;
 
 template <int MT, int MODE>
 __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvShared* sh, uint8_t* smem, float* stat_part,
                                                double* stat_acc, const uint32_t tmem_base) {
   constexpr bool RES = (MODE & kEpiRes) != 0, STATS = (MODE & kEpiStats) != 0, FP32 = (MODE & kEpiFp32) != 0;
+  constexpr bool F32P = (MODE & kEpiF32Planar) != 0;
+  constexpr int kUnitPlanes = F32P ? 4 : 2;     // 16-byte planes of one 16-channel unit of the planar output / residual
+  constexpr int kPlaneShift = F32P ? 2 : 3;     // log2(channels per plane)
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q = warp & 3;                       // TMEM lane quarter this warp may read
   const int ew = warp - (kEpiFirst >> 5);       // 0..7
@@ -536,7 +542,7 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
   // cp.async has no destination register; the only wait is cp.async.wait_group on the oldest group.
   constexpr int kResPrefetchTiles = 3;
   const int r_depth = p.res_depth;
-  uint4* r_ring = reinterpret_cast<uint4*>(smem + p.res_ring_off) + et;   // slot i, plane hf: r_ring[(2*i + hf) * kEpiThreads]
+  uint4* r_ring = reinterpret_cast<uint4*>(smem + p.res_ring_off) + et;   // slot i, plane k: r_ring[(kUnitPlanes*i + k) * kEpiThreads]
   int r_slot = 0;                                  // oldest slot == the one refilled next (the ring is always full)
   const uint4* res_base = reinterpret_cast<const uint4*>(p.residual);
   // residual grid: the output grid, or (r_up) its half-resolution parent (coordinates shifted right by one)
@@ -558,7 +564,7 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
         r_hw_ok = (hr < p.H) && (wr < p.W);
         r_d0 = tr.d0;
         r_cbase = tr.ns * n_cta;
-        r_ptr = res_base + ((long long)tr.b * p.r_planes + p.r_plane0 + (r_cbase >> 3) +
+        r_ptr = res_base + ((long long)tr.b * p.r_planes + p.r_plane0 + (r_cbase >> kPlaneShift) +
                             (((hr & 1) << 1) | (wr & 1)) * p.r_d2s_planes) * r_V +
                 (long long)(hr >> r_sh) * r_W + (wr >> r_sh);
         ru_s = s0; ru_ch = ch0;
@@ -571,12 +577,18 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
       ru_s += s_step;
       if (ru_s >= MT) { ru_s = s0; ru_ch += ch_step; }
       if (r_hw_ok && r_d0 + su < p.D) {
-        const uint4* src = r_ptr + (long long)(chu * 2 + (((r_d0 + su) & 1) << 2) * p.r_d2s_planes) * r_V +
+        const uint4* src = r_ptr + (long long)(chu * kUnitPlanes + (((r_d0 + su) & 1) << 2) * p.r_d2s_planes) * r_V +
                            (long long)((r_d0 + su) >> r_sh) * r_HW;
         const int cu = r_cbase + chu * 16;
-        uint4* dst = r_ring + (2 * slot) * kEpiThreads;
-        if (cu < p.c_out) ptx::cp_async16(dst, src);
-        if (cu + 8 < p.c_out) ptx::cp_async16(dst + kEpiThreads, src + r_V);
+        uint4* dst = r_ring + (kUnitPlanes * slot) * kEpiThreads;
+        if constexpr (F32P) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            if (cu + 4 * k < p.c_out) ptx::cp_async16(dst + k * kEpiThreads, src + k * r_V);
+        } else {
+          if (cu < p.c_out) ptx::cp_async16(dst, src);
+          if (cu + 8 < p.c_out) ptx::cp_async16(dst + kEpiThreads, src + r_V);
+        }
       }
     }
     ptx::cp_async_commit();                        // one group per unit, also when nothing was copied
@@ -598,14 +610,14 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
       if (pt < p.n_tiles) {
         const TileCoord tp = decode_tile(p, pt);
         const int pc0 = tp.ns * n_cta;
-        const int n_rows = (n_cta >> 3) * MT * 16;
-        const uint4* pbase = res_base + ((long long)tp.b * p.r_planes + p.r_plane0 + (pc0 >> 3)) * r_V + (tp.w0 >> r_sh);
+        const int n_rows = (n_cta >> kPlaneShift) * MT * 16;
+        const uint4* pbase = res_base + ((long long)tp.b * p.r_planes + p.r_plane0 + (pc0 >> kPlaneShift)) * r_V + (tp.w0 >> r_sh);
         for (int idx = et; idx < n_rows; idx += kEpiThreads) {
           const int hh = tp.h0 + (idx & 15);
           const int sp_ = idx >> 4;
           const int pp = sp_ / MT;
           const int dd = tp.d0 + (sp_ - pp * MT);
-          if (hh < p.H && dd < p.D && pc0 + pp * 8 < p.c_out && !(r_sh && ((hh | dd) & 1)))
+          if (hh < p.H && dd < p.D && pc0 + (pp << kPlaneShift) < p.c_out && !(r_sh && ((hh | dd) & 1)))
             ptx::prefetch_l2(pbase + (long long)pp * r_V + ((long long)(dd >> r_sh) * r_H + (hh >> r_sh)) * r_W);
         }
       }
@@ -647,14 +659,17 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
       }
       bf16x8* y_ch = reinterpret_cast<bf16x8*>(p.y) + ((long long)t.b * p.y_planes + p.y_plane0 + (c0 >> 3)) * V + vox0;
       float* y32_ch = static_cast<float*>(p.y) + ((long long)t.b * p.c_out + c0) * V + vox0;
+      float4* y4_ch = static_cast<float4*>(p.y) + ((long long)t.b * p.y_planes + p.y_plane0 + (c0 >> 2)) * V + vox0;
       auto process = [&](uint32_t (&raw)[16], int s) __attribute__((always_inline)) {
         const bool valid = hw_ok && (t.d0 + s < p.D);
         uint4 rcur0 = make_uint4(0, 0, 0, 0), rcur1 = make_uint4(0, 0, 0, 0);
+        uint4 rcur2 = make_uint4(0, 0, 0, 0), rcur3 = make_uint4(0, 0, 0, 0);   // (fp32 planar: planes 2, 3 of the unit)
         if (RES) {
           // the oldest slot is this unit's residual; refill it for the unit r_depth ahead
           ptx::cp_async_wait(r_depth - 1);
-          const uint4* slot = r_ring + (2 * r_slot) * kEpiThreads;
+          const uint4* slot = r_ring + (kUnitPlanes * r_slot) * kEpiThreads;
           rcur0 = slot[0]; rcur1 = slot[kEpiThreads];
+          if (F32P) { rcur2 = slot[2 * kEpiThreads]; rcur3 = slot[3 * kEpiThreads]; }
           res_issue(r_slot);
           r_slot = (r_slot + 1 == r_depth) ? 0 : r_slot + 1;
         }
@@ -674,6 +689,33 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
           return;
         }
         if (nhf == 0 || !valid) return;          // padded output channels (warp-uniform) / voxels beyond the grid
+        if (F32P) {
+          float4* yp = y4_ch + (long long)s * HW;
+#pragma unroll
+          for (int hf = 0; hf < 2; ++hf) {
+            if (hf == 1 && nhf < 2) break;
+            float g[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) g[j] = f[hf * 8 + j];
+            if (RES) {
+              const uint4 ra = hf == 0 ? rcur0 : rcur2, rb = hf == 0 ? rcur1 : rcur3;
+              add2(g[0], g[1], __uint_as_float(ra.x), __uint_as_float(ra.y));
+              add2(g[2], g[3], __uint_as_float(ra.z), __uint_as_float(ra.w));
+              add2(g[4], g[5], __uint_as_float(rb.x), __uint_as_float(rb.y));
+              add2(g[6], g[7], __uint_as_float(rb.z), __uint_as_float(rb.w));
+            }
+            yp[(long long)(2 * hf) * V] = make_float4(g[0], g[1], g[2], g[3]);
+            yp[(long long)(2 * hf + 1) * V] = make_float4(g[4], g[5], g[6], g[7]);
+            if (STATS) {
+#pragma unroll
+              for (int j = 0; j < 8; j += 2) {
+                add2(s1[hf * 8 + j], s1[hf * 8 + j + 1], g[j], g[j + 1]);
+                fma2_sq(s2[hf * 8 + j], s2[hf * 8 + j + 1], g[j], g[j + 1]);
+              }
+            }
+          }
+          return;
+        }
         bf16x8* yp = y_ch + (long long)s * HW;
 #pragma unroll
         for (int hf = 0; hf < 2; ++hf) {
@@ -792,14 +834,14 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
 // rate while L2 ran at 8 %.  Here the run-time part is per TAP (its halo offset from the tap table, its weight block: one
 // 64-bit descriptor for A and KJ for B), and the MT x KJ MMAs of a tap differ by IMMEDIATE offsets (PAD fixes the halo
 // geometry at compile time): one UIADD3.64 and the UTCHMMA per MMA.
-template <int MT, int KJ, int PAD, int TPS, bool RESIDENT>
+template <int MT, int KJ, int PAD, int TPS, bool RESIDENT, ptx::MmaKind KIND>
 __device__ __forceinline__ void issue_generic_tiles(const ConvKernelParams& p, ConvShared* sh, uint64_t* a_rdy, uint32_t a_base16,
                                                     uint32_t b_base16, uint32_t tmem_u, bool leader) {
   constexpr uint32_t Hh = kTileH + 2 * PAD, Wh = kTileW + 2 * PAD, Hd = MT + 2 * PAD;
   constexpr uint32_t slice16 = Hh * Wh;                      // one d-slice of a plane, 16-byte units
   constexpr uint32_t kstep_a16 = 2u * Hd * Hh * Wh;          // two planes (K = 16)
   const uint32_t n_cta = hold_u32((uint32_t)p.n_cta);
-  const uint32_t idesc = ptx::make_idesc_bf16(128, n_cta);
+  const uint32_t idesc = ptx::make_idesc_bf16<KIND>(128, n_cta);
   const uint64_t a_hi = make_planar_desc(0, Hd * Hh * Wh * 16u, Wh * 16u);
   const uint64_t b_hi = make_planar_desc(0, n_cta * 16u, 128u);
   const uint32_t a_stage16 = hold_u32((uint32_t)p.a_stage_bytes >> 4), b_stage16 = hold_u32((uint32_t)p.b_stage_bytes >> 4);
@@ -847,8 +889,8 @@ __device__ __forceinline__ void issue_generic_tiles(const ConvKernelParams& p, C
             for (int s = 0; s < MT; ++s) {
 #pragma unroll
               for (int j = 0; j < KJ; ++j)
-                ptx::umma_bf16_off64(d_tmem0, (uint32_t)s * n_cta, a_tap, (uint32_t)s * slice16 + (uint32_t)j * kstep_a16, b_tap[j], 0u,
-                                     idesc, j == 0 ? first : 1u);
+                ptx::umma_bf16_off64<KIND>(d_tmem0, (uint32_t)s * n_cta, a_tap, (uint32_t)s * slice16 + (uint32_t)j * kstep_a16, b_tap[j],
+                                           0u, idesc, j == 0 ? first : 1u);
             }
           }
           if (!resident) {
@@ -867,10 +909,16 @@ __device__ __forceinline__ void issue_generic_tiles(const ConvKernelParams& p, C
 // MT = d-slices (accumulators) per tile, KJ = K=16 MMAs per channel chunk (KC = 16*KJ), NF = 0 for the generic
 // path or Cout_pad for the kd-folded path: compile-time so that the MMA issue loops are straight lines of
 // tcgen05.mma with immediate offsets (r01a: a generic loop cost ~240 issue cycles per MMA).
-template <int MT, int KJ, int NF>
+// TF32: fp32 channel-planar activations [B][C/4][D][H][W][4] and fp32 weights [tap][Cin/4][Cout_pad][4], tcgen05.mma
+// kind::tf32.  A plane is 16 bytes and a K step 32 bytes in both element types, so everything up to the accumulator
+// (TMA boxes, weight copies, descriptors, the issue schedule) is that of the bf16 layer with twice the input channels;
+// only the MMA kind and the epilogue's output element differ.  Generic schedule only, no fused input transform.
+template <int MT, int KJ, int NF, bool TF32 = false>
 __global__ void __launch_bounds__(kConvThreads, 1)
 conv3d_planar_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_x2,
                      const __grid_constant__ ConvKernelParams p) {
+  static_assert(!TF32 || NF == 0, "the TF32 instances run the generic schedule only");
+  constexpr ptx::MmaKind kKind = TF32 ? ptx::MmaKind::kTF32 : ptx::MmaKind::kF16;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // Round the window up to 1024 bytes by POINTER ARITHMETIC on the __shared__ array: a round trip through uintptr_t
   // made nvcc lose the address space, and every access through `sh` / the residual ring compiled to generic LD / ST
@@ -1138,29 +1186,31 @@ conv3d_planar_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
       // (pad == 0 is the 1x1x1 conv: one tap per stage; tap subsets whose count is not a multiple of three too)
       const bool res = p.b_resident != 0;
       if (!p.pad) {
-        if (res) issue_generic_tiles<MT, KJ, 0, 1, true>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
-        else issue_generic_tiles<MT, KJ, 0, 1, false>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        if (res) issue_generic_tiles<MT, KJ, 0, 1, true, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        else issue_generic_tiles<MT, KJ, 0, 1, false, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
       } else if (p.taps_per_stage == 3) {
-        if (res) issue_generic_tiles<MT, KJ, 1, 3, true>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
-        else issue_generic_tiles<MT, KJ, 1, 3, false>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        if (res) issue_generic_tiles<MT, KJ, 1, 3, true, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        else issue_generic_tiles<MT, KJ, 1, 3, false, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
       } else {
-        if (res) issue_generic_tiles<MT, KJ, 1, 1, true>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
-        else issue_generic_tiles<MT, KJ, 1, 1, false>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        if (res) issue_generic_tiles<MT, KJ, 1, 1, true, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
+        else issue_generic_tiles<MT, KJ, 1, 1, false, kKind>(p, sh, a_rdy, a_base16, b_base16, tmem_u, leader);
       }
     }
   }
   } else if (warp >= 12) {
     // ===================== input transform (4 warps): see transform_tiles =====================
     ptx::setmaxnreg_dec<kRegsXf>();
-    if (p.in_norm) transform_tiles<MT, KJ>(p, sh, a_smem, reinterpret_cast<float*>(smem + p.xf_coef_off));
+    if constexpr (!TF32)
+      if (p.in_norm) transform_tiles<MT, KJ>(p, sh, a_smem, reinterpret_cast<float*>(smem + p.xf_coef_off));
   } else {
     // ===================== epilogue (8 warps; two per TMEM lane quarter): see epilogue_tiles =====================
     ptx::setmaxnreg_inc<kRegsEpi>();
+    constexpr int P = TF32 ? kEpiF32Planar : 0;     // planar output element: fp32 (TF32) or bf16
     if (p.out_fp32) epilogue_tiles<MT, kEpiFp32>(p, sh, smem, stat_part, stat_acc, tmem_base);
-    else if (p.residual && p.stats) epilogue_tiles<MT, kEpiRes | kEpiStats>(p, sh, smem, stat_part, stat_acc, tmem_base);
-    else if (p.residual) epilogue_tiles<MT, kEpiRes>(p, sh, smem, stat_part, stat_acc, tmem_base);
-    else if (p.stats) epilogue_tiles<MT, kEpiStats>(p, sh, smem, stat_part, stat_acc, tmem_base);
-    else epilogue_tiles<MT, 0>(p, sh, smem, stat_part, stat_acc, tmem_base);
+    else if (p.residual && p.stats) epilogue_tiles<MT, P | kEpiRes | kEpiStats>(p, sh, smem, stat_part, stat_acc, tmem_base);
+    else if (p.residual) epilogue_tiles<MT, P | kEpiRes>(p, sh, smem, stat_part, stat_acc, tmem_base);
+    else if (p.stats) epilogue_tiles<MT, P | kEpiStats>(p, sh, smem, stat_part, stat_acc, tmem_base);
+    else epilogue_tiles<MT, P>(p, sh, smem, stat_part, stat_acc, tmem_base);
   }
 
   ptx::tc_fence_before();
@@ -1217,7 +1267,9 @@ static int tap_cell(const VdmConvDesc& d, int t) {
 
 // Launch plan of one conv layer: schedule, tiling, pipeline depths and shared-memory layout.  Host arithmetic only (the
 // descriptor's ranges are checked by the caller); returns VDM_OK, or the code and message the layer is refused with.
-static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, bool has_xf, int skip_c_in, int sms,
+// A TF32 layer is planned as the byte-identical bf16 layer (`d` with twice its input channels) on the generic schedule;
+// its residual units are twice as large.
+static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, bool has_xf, int skip_c_in, int sms, bool tf32,
                      ConvPlan& pl) {
   const ConvOverrides& ov = g_overrides;
   pl = ConvPlan{};
@@ -1234,11 +1286,12 @@ static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, boo
     return VDM_E_UNSUPPORTED;
   }
   const int xf_bytes = has_xf ? ((d.c_in * 8 + 15) & ~15) : 0;      // (a, b) table of one sample
+  const int res_slot = tf32 ? 2 * kResSlotBytes : kResSlotBytes;     // one residual unit for every epilogue thread
   const int skip_w_bytes = has_skip ? skip_c_in * d.c_out_pad * 2 : 0;
 
   // ---- schedule ----
   // kd-folded schedules (issue_fold_tile): the full 3x3x3 stencil on a narrow layer
-  bool fold = d.n_taps == 27 && pad == 1 && (d.c_out_pad == 16 || d.c_out_pad == 32 || d.c_out_pad == 64) && d.depth >= 3 &&
+  bool fold = !tf32 && d.n_taps == 27 && pad == 1 && (d.c_out_pad == 16 || d.c_out_pad == 32 || d.c_out_pad == 64) && d.depth >= 3 &&
               ov.no_fold == 0 && ov.force_mt == 0 && ov.force_nsplit == 0;
   const bool streamed = d.c_out_pad == 64;
   int fold_mt = 0, fold_kc = 0;
@@ -1249,7 +1302,7 @@ static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, boo
   } else if (fold) {
     // all weights resident + two halo stages must fit; prefer tall tiles (halo efficiency), then wide chunks
     const int budget = 227 * 1024 - 1024 - (int)sizeof(ConvShared) - (2 * 2 * 8 * d.c_out_pad * 4 + 2 * d.c_out_pad * 8) - 256 -
-                       (has_residual ? 2 * kResSlotBytes : 0) - xf_bytes;      // room for at least two residual slots
+                       (has_residual ? 2 * res_slot : 0) - xf_bytes;      // room for at least two residual slots
     const int w_bytes = 27 * d.c_in * d.c_out_pad * 2 + skip_w_bytes;
     for (int m = 4; m >= 2 && !fold_mt; --m)
       for (int c = 32; c >= 16 && !fold_mt; c -= 16) {
@@ -1365,7 +1418,7 @@ static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, boo
   const int smem_total = 227 * 1024 - 1024 /*alignment slack*/ - (int)sizeof(ConvShared) - stat_part_bytes - 256 - xf_bytes;
   // layers with a residual keep a cp.async ring of it in shared memory: 4 units deep where the weights are streamed
   // anyway, at least 2 where they are resident (the fold search above left room)
-  const int smem_budget = smem_total - (has_residual ? (resident_fold ? 2 : 4) * kResSlotBytes : 0);
+  const int smem_budget = smem_total - (has_residual ? (resident_fold ? 2 : 4) * res_slot : 0);
   if (fold) {
     pl.kc = fold_kc;
     pl.a_stage_bytes = ((fold_kc / 8) * plane_bytes + 127) & ~127;
@@ -1403,17 +1456,17 @@ static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, boo
   // Halo stages: two are planned above; layers whose weights leave room get up to kMaxAStages.  A TMA box takes
   // several thousand cycles to arrive from L2 / HBM, and where a chunk's MMAs are shorter than that (conv_in: 54 MMAs per
   // tile, the 1x1x1 convs) two stages left the tensor core waiting for loads.
-  const int fixed = pl.nsb * pl.b_stage_bytes + skip_w_bytes + (has_residual ? 4 * kResSlotBytes : 0);
+  const int fixed = pl.nsb * pl.b_stage_bytes + skip_w_bytes + (has_residual ? 4 * res_slot : 0);
   pl.nsa = 2;
   while (pl.nsa < kMaxAStages && (pl.nsa + 1) * pl.a_stage_bytes + fixed <= smem_total) ++pl.nsa;
   const int used = pl.nsa * pl.a_stage_bytes + pl.nsb * pl.b_stage_bytes + skip_w_bytes;
   if (has_residual) {
-    const int depth = (smem_total - used) / kResSlotBytes;
+    const int depth = (smem_total - used) / res_slot;
     pl.res_depth = depth > 4 ? 4 : depth;
     VDM_CHECK_ARG(pl.res_depth >= 1, "vdm_conv3d: no shared memory left for the residual ring");
     pl.res_ring_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 15) & ~15;
   }
-  pl.xf_coef_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 16 + pl.res_depth * kResSlotBytes + 15) & ~15;
+  pl.xf_coef_off = (used + (int)sizeof(ConvShared) + stat_part_bytes + 16 + pl.res_depth * res_slot + 15) & ~15;
   pl.smem_bytes = (size_t)pl.xf_coef_off + xf_bytes + 1024;
   pl.grid = pl.n_tiles < sms ? pl.n_tiles : sms;
   return VDM_OK;
@@ -1421,7 +1474,7 @@ static int plan_conv(const VdmConvDesc& d, bool has_residual, bool has_skip, boo
 
 // The kernel instance of a plan.  Every instance compiled into the library is listed here.
 static int launch_conv(const ConvPlan& pl, const CUtensorMap& tmx, const CUtensorMap& tmx2, const ConvKernelParams& p,
-                       cudaStream_t stream) {
+                       bool tf32, cudaStream_t stream) {
   if (pl.schedule == ConvSchedule::kMarch) {
     const bool sk = p.skip_chunks > 0, xf = p.in_norm != nullptr;
 #define VDM_MARCH(KJv, NFv, SKv, XFv)                                                                          \
@@ -1435,6 +1488,18 @@ static int launch_conv(const ConvPlan& pl, const CUtensorMap& tmx, const CUtenso
     return VDM_E_UNSUPPORTED;
   }
   const int nf = pl.schedule == ConvSchedule::kTile ? 0 : pl.n_cta;
+  if (tf32) {
+#define VDM_TILE_TF32(MTv, KJv)                                                                                \
+    if (pl.mt == MTv && pl.kc == 16 * KJv && nf == 0)                                                          \
+      return launch_kernel<conv3d_planar_kernel<MTv, KJv, 0, true>>(pl.grid, kConvThreads, pl.smem_bytes, stream, tmx, tmx2, p);
+    VDM_TILE_TF32(1, 1) VDM_TILE_TF32(1, 2) VDM_TILE_TF32(1, 4)
+    VDM_TILE_TF32(2, 1) VDM_TILE_TF32(2, 2) VDM_TILE_TF32(2, 4)
+    VDM_TILE_TF32(3, 1) VDM_TILE_TF32(3, 2) VDM_TILE_TF32(3, 4)
+    VDM_TILE_TF32(4, 1) VDM_TILE_TF32(4, 2) VDM_TILE_TF32(4, 4)
+#undef VDM_TILE_TF32
+    set_error("vdm_conv3d_tf32: no kernel instance for MT=%d KC=%d", pl.mt, pl.kc / 2);
+    return VDM_E_UNSUPPORTED;
+  }
 #define VDM_TILE(MTv, KJv, NFv)                                                                                \
   if (pl.mt == MTv && pl.kc == 16 * KJv && nf == NFv)                                                          \
     return launch_kernel<conv3d_planar_kernel<MTv, KJv, NFv>>(pl.grid, kConvThreads, pl.smem_bytes, stream, tmx, tmx2, p);
@@ -1470,11 +1535,9 @@ extern "C" int vdm_debug_set(int key, int value) {
 }
 #endif
 
-extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w, void* y,
-                          const VdmConvEpilogue* epi, void* stream_) {
-  cudaStream_t stream = (cudaStream_t)stream_;
-  VDM_CHECK_ARG(desc && x && w && y, "vdm_conv3d: NULL pointer argument");
-  const VdmConvDesc& d = *desc;
+// vdm_conv3d, and vdm_conv3d_tf32 with `d` describing the byte-identical bf16 layer (see plan_conv).
+static int conv3d_run(const VdmConvDesc& d, const void* x, const void* w, void* y, const VdmConvEpilogue* epi, bool tf32,
+                      cudaStream_t stream) {
   VDM_CHECK_ARG(d.batch >= 1 && d.depth >= 1 && d.height >= 1 && d.width >= 1, "vdm_conv3d: bad grid");
   VDM_CHECK_ARG(d.c_in >= 16 && d.c_in % 16 == 0, "vdm_conv3d: c_in=%d must be a multiple of 16", d.c_in);
   VDM_CHECK_ARG(d.c_out_pad >= 16 && d.c_out_pad % 16 == 0 && d.c_out_pad <= 256,
@@ -1506,7 +1569,7 @@ extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w,
   }
 
   ConvPlan pl;
-  const int rc = plan_conv(d, has_residual, has_skip, has_xf, has_skip ? epi->skip_c_in : 0, num_sms(), pl);
+  const int rc = plan_conv(d, has_residual, has_skip, has_xf, has_skip ? epi->skip_c_in : 0, num_sms(), tf32, pl);
   if (rc != VDM_OK) return rc;
   // (checked after planning: a layer the planner refuses reports VDM_E_UNSUPPORTED, which callers answer with a fallback)
   const int x2_planes = !has_skip ? 0 : epi->skip_planes > 0 ? epi->skip_planes : epi->skip_c_in / 8;
@@ -1593,5 +1656,32 @@ extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w,
                       march ? "skip_x, marching" : "skip_x");
     if (e != VDM_OK) return e;
   }
-  return launch_conv(pl, tmx, tmx2, p, stream);
+  return launch_conv(pl, tmx, tmx2, p, tf32, stream);
+}
+
+extern "C" int vdm_conv3d(const VdmConvDesc* desc, const void* x, const void* w, void* y,
+                          const VdmConvEpilogue* epi, void* stream) {
+  VDM_CHECK_ARG(desc && x && w && y, "vdm_conv3d: NULL pointer argument");
+  return conv3d_run(*desc, x, w, y, epi, false, (cudaStream_t)stream);
+}
+
+extern "C" int vdm_conv3d_tf32(const VdmConvDesc* desc, const void* x, const void* w, void* y,
+                               const VdmConvEpilogue* epi, void* stream) {
+  VDM_CHECK_ARG(desc && x && w && y, "vdm_conv3d_tf32: NULL pointer argument");
+  const VdmConvDesc& d = *desc;
+  VDM_CHECK_ARG(d.c_in >= 8 && d.c_in % 8 == 0 && d.c_in <= 4096, "vdm_conv3d_tf32: c_in=%d must be a multiple of 8", d.c_in);
+  if (epi && (epi->in_norm || epi->skip_x || (epi->residual && epi->residual_upsample))) {
+    set_error("vdm_conv3d_tf32: the fused input transform, the fused skip conv and the up-sampled residual are bf16-only");
+    return VDM_E_UNSUPPORTED;
+  }
+  // Planes are 4 fp32 channels: the layer is the bf16 layer of 2 c_in channels; output and residual windows are counted
+  // in 4-channel planes here, so they are resolved before the bf16 checks see them.
+  VdmConvDesc d2 = d;
+  d2.c_in = 2 * d.c_in;
+  if (!d.out_fp32) {
+    d2.y_planes = d.y_planes > 0 ? d.y_planes : (d.c_out + 3) / 4;
+    VDM_CHECK_ARG(d.y_plane0 >= 0 && d.y_plane0 + d.c_out / 4 <= d2.y_planes, "vdm_conv3d_tf32: y plane window out of range");
+  }
+  d2.r_planes = d.r_planes > 0 ? d.r_planes : d.c_out / 4;
+  return conv3d_run(d2, x, w, y, epi, true, (cudaStream_t)stream);
 }

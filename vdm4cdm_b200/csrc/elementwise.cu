@@ -35,26 +35,29 @@ channel_stats_kernel(VdmTensor x, int planes, int64_t voxels, double* __restrict
 
 // STREAM: evict-first loads/stores for tensors far larger than L2 (level-0 activations: +20% on the 96-channel
 // layer, r01z); small tensors keep default caching so the conv that follows reads them from L2.
-template <bool STREAM>
+// F32: fp32 channel-planar tensors (TF32 inference mode), exp-based SiLU, no dropout.
+template <bool STREAM, bool F32 = false>
 __global__ void __launch_bounds__(kEwThreads)
 gn_silu_kernel(VdmTensor x, VdmTensor y, int planes, int64_t voxels, int groups, const double* __restrict__ stats,
                const float* __restrict__ gamma, const float* __restrict__ beta, float eps, float dropout_p,
                uint64_t seed, const int32_t* __restrict__ seed_step, uint32_t layer_tag) {
+  using T = typename Unit<F32>::T;
+  constexpr int L = Unit<F32>::L;
   if (seed_step) seed += (uint64_t)(uint32_t)(*seed_step);
-  __shared__ float s_scale[8], s_shift[8];
+  __shared__ float s_scale[L], s_shift[L];
   const int b = blockIdx.y / planes, pl = blockIdx.y % planes;
-  const int C = planes * 8;
-  plane_scale_shift(stats + (int64_t)b * C * 2, C, groups, pl, (double)voxels, gamma, beta, eps, s_scale, s_shift,
-                    nullptr, nullptr);
+  const int C = planes * L;
+  plane_scale_shift<L>(stats + (int64_t)b * C * 2, C, groups, pl, (double)voxels, gamma, beta, eps, s_scale, s_shift,
+                       nullptr, nullptr);
   __syncthreads();
-  float sc[8], sh[8];                      // halved: silu(y) = h + h tanh(h), h = y / 2 (silu_half)
+  float sc[L], sh[L];                      // bf16: halved, silu(y) = h + h tanh(h), h = y / 2 (silu_half)
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    sc[j] = 0.5f * s_scale[j];
-    sh[j] = 0.5f * s_shift[j];
+  for (int j = 0; j < L; ++j) {
+    sc[j] = F32 ? s_scale[j] : 0.5f * s_scale[j];
+    sh[j] = F32 ? s_shift[j] : 0.5f * s_shift[j];
   }
-  const bf16x8* xp = plane_ptr(x, b, pl, voxels);
-  bf16x8* yp = plane_ptr_mut(y, b, pl, voxels);
+  const T* xp = plane_ptr<T>(x, b, pl, voxels);
+  T* yp = plane_ptr_mut<T>(y, b, pl, voxels);
   const bool drop = dropout_p > 0.f;
   const uint32_t thresh16 = (uint32_t)(dropout_p * 65536.0f + 0.5f);
   const float keep_scale = drop ? 1.0f / (1.0f - dropout_p) : 1.0f;
@@ -64,7 +67,7 @@ gn_silu_kernel(VdmTensor x, VdmTensor y, int planes, int64_t voxels, int groups,
   constexpr int U = 4;
   const int64_t stride = (int64_t)gridDim.x * kEwThreads;
   for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < voxels; i += U * stride) {
-    bf16x8 v[U];
+    T v[U];
 #pragma unroll
     for (int k = 0; k < U; ++k) {
       const int64_t ii = i + k * stride;
@@ -74,17 +77,21 @@ gn_silu_kernel(VdmTensor x, VdmTensor y, int planes, int64_t voxels, int groups,
     for (int k = 0; k < U; ++k) {
       const int64_t ii = i + k * stride;
       if (ii >= voxels) break;
-      float f[8];
-      unpack8(v[k], f);
+      float f[L];
+      unpack_unit(v[k], f);
 #pragma unroll
-      for (int j = 0; j < 8; ++j) f[j] = silu_half(fmaf(f[j], sc[j], sh[j]));
-      if (drop) {
-        const uint32_t keep = dropout_keep8(chunk0 + (uint64_t)ii, layer_tag, seed, thresh16);
+      for (int j = 0; j < L; ++j) f[j] = F32 ? silu_f32(fmaf(f[j], sc[j], sh[j])) : silu_half(fmaf(f[j], sc[j], sh[j]));
+      if constexpr (!F32) {
+        if (drop) {
+          const uint32_t keep = dropout_keep8(chunk0 + (uint64_t)ii, layer_tag, seed, thresh16);
 #pragma unroll
-        for (int j = 0; j < 8; ++j) f[j] = ((keep >> j) & 1u) ? f[j] * keep_scale : 0.f;
+          for (int j = 0; j < 8; ++j) f[j] = ((keep >> j) & 1u) ? f[j] * keep_scale : 0.f;
+        }
       }
-      if (STREAM) st_stream(yp + ii, pack8(f));
-      else yp[ii] = pack8(f);
+      T out;
+      pack_unit(f, out);
+      if (STREAM) st_stream(yp + ii, out);
+      else yp[ii] = out;
     }
   }
 }
@@ -185,59 +192,68 @@ gn_silu_view_kernel(VdmTensor x, VdmTensor y, int planes, int c_off, int C_total
 }
 
 // ---- 2x2x2 average pooling (+ stats of the output) ---------------------------------------------
+// (F32: fp32 channel-planar, statistics of the fp32 values)
+template <bool F32 = false>
 __global__ void __launch_bounds__(kEwThreads)
 avgpool2_kernel(VdmTensor x, VdmTensor y, int planes, int D, int H, int W, double* __restrict__ stats,
                 int stats_channels, int stats_c0) {
+  using T = typename Unit<F32>::T;
+  constexpr int L = Unit<F32>::L;
   const int b = blockIdx.y / planes, pl = blockIdx.y % planes;
   const int Do = D >> 1, Ho = H >> 1, Wo = W >> 1;
   const int64_t vin = (int64_t)D * H * W, vout = (int64_t)Do * Ho * Wo;
-  const bf16x8* xp = plane_ptr(x, b, pl, vin);
-  bf16x8* yp = plane_ptr_mut(y, b, pl, vout);
-  float sum[8] = {0, 0, 0, 0, 0, 0, 0, 0}, sq[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  const T* xp = plane_ptr<T>(x, b, pl, vin);
+  T* yp = plane_ptr_mut<T>(y, b, pl, vout);
+  float sum[L] = {}, sq[L] = {};
   for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < vout; i += (int64_t)gridDim.x * kEwThreads) {
     unsigned v = (unsigned)i;
     const int wo = (int)(v % (unsigned)Wo); v /= (unsigned)Wo;
     const int ho = (int)(v % (unsigned)Ho);
     const int dz = (int)(v / (unsigned)Ho);
-    float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    float acc[L] = {};
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
       const int d = 2 * dz + (k >> 2), h = 2 * ho + ((k >> 1) & 1), w = 2 * wo + (k & 1);
-      float f[8];
-      unpack8(xp[((int64_t)d * H + h) * W + w], f);
+      float f[L];
+      unpack_unit(xp[((int64_t)d * H + h) * W + w], f);
 #pragma unroll
-      for (int j = 0; j < 8; ++j) acc[j] += f[j];
+      for (int j = 0; j < L; ++j) acc[j] += f[j];
     }
 #pragma unroll
-    for (int j = 0; j < 8; ++j) acc[j] *= 0.125f;
-    const bf16x8 packed = pack8(acc);
+    for (int j = 0; j < L; ++j) acc[j] *= 0.125f;
+    T packed;
+    pack_unit(acc, packed);
     yp[i] = packed;
     if (stats) {
-      float r[8];
-      unpack8(packed, r);  // statistics of the stored (rounded) tensor
+      float r[L];
+      unpack_unit(packed, r);  // statistics of the stored (rounded) tensor
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
+      for (int j = 0; j < L; ++j) {
         sum[j] += r[j];
         sq[j] += r[j] * r[j];
       }
     }
   }
-  if (stats) block_flush_stats(sum, sq, stats + ((int64_t)b * stats_channels + stats_c0 + pl * 8) * 2);
+  if (stats) block_flush_stats<L>(sum, sq, stats + ((int64_t)b * stats_channels + stats_c0 + pl * L) * 2);
 }
 
 // ---- nearest x2 up-sampling into a plane window of y (+ stats of the output) -------------------
 // (D, H, W) is the FINE grid.  One thread per FINE voxel: fully coalesced 16-byte stores (the 8x repeated
 // coarse reads hit L1/L2).  r01f: the one-thread-per-coarse-voxel version (8 scattered stores per thread)
 // ran at ~1.2 TB/s.
+// (F32: fp32 channel-planar)
+template <bool F32 = false>
 __global__ void __launch_bounds__(kEwThreads)
 upsample2_kernel(VdmTensor coarse, VdmTensor y, int planes, int D, int H, int W, double* __restrict__ stats,
                  int stats_channels, int stats_c0) {
+  using T = typename Unit<F32>::T;
+  constexpr int L = Unit<F32>::L;
   const int b = blockIdx.y / planes, pl = blockIdx.y % planes;
   const int Hc = H >> 1, Wc = W >> 1;
   const int64_t vc = (int64_t)(D >> 1) * Hc * Wc, vf = (int64_t)D * H * W;
-  const bf16x8* cp = plane_ptr(coarse, b, pl, vc);
-  bf16x8* yp = plane_ptr_mut(y, b, pl, vf);
-  float sum[8] = {0, 0, 0, 0, 0, 0, 0, 0}, sq[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  const T* cp = plane_ptr<T>(coarse, b, pl, vc);
+  T* yp = plane_ptr_mut<T>(y, b, pl, vf);
+  float sum[L] = {}, sq[L] = {};
   // one thread per (fine d, fine h, COARSE w): one 16-byte read, two adjacent 16-byte stores (32 contiguous bytes)
   const int64_t vh = vf >> 1;
   const bool big = vf * planes > ((int64_t)4 << 20);   // > 64 MB per sample: written once, read later from HBM anyway
@@ -246,21 +262,21 @@ upsample2_kernel(VdmTensor coarse, VdmTensor y, int planes, int D, int H, int W,
     const int wc = (int)(v % (unsigned)Wc); v /= (unsigned)Wc;
     const int h = (int)(v % (unsigned)H);
     const int d = (int)(v / (unsigned)H);
-    const bf16x8 val = cp[((int64_t)(d >> 1) * Hc + (h >> 1)) * Wc + wc];
-    bf16x8* dst = yp + ((int64_t)d * H + h) * W + 2 * wc;
+    const T val = cp[((int64_t)(d >> 1) * Hc + (h >> 1)) * Wc + wc];
+    T* dst = yp + ((int64_t)d * H + h) * W + 2 * wc;
     if (big) { st_stream(dst, val); st_stream(dst + 1, val); }
     else { dst[0] = val; dst[1] = val; }
     if (stats) {
-      float r[8];
-      unpack8(val, r);
+      float r[L];
+      unpack_unit(val, r);
 #pragma unroll
-      for (int j = 0; j < 8; ++j) {
+      for (int j = 0; j < L; ++j) {
         sum[j] += 2.f * r[j];
         sq[j] += 2.f * r[j] * r[j];
       }
     }
   }
-  if (stats) block_flush_stats(sum, sq, stats + ((int64_t)b * stats_channels + stats_c0 + pl * 8) * 2);
+  if (stats) block_flush_stats<L>(sum, sq, stats + ((int64_t)b * stats_channels + stats_c0 + pl * L) * 2);
 }
 
 // ---- periodic one-voxel halo (circular convolutions) ---------------------------------------------------
@@ -395,7 +411,7 @@ extern "C" int vdm_avgpool2(const VdmTensor* x, const VdmTensor* y, int batch, i
   if (stats_channels <= 0) stats_channels = channels;
   const int planes = channels / 8;
   const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);
-  avgpool2_kernel<<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+  avgpool2_kernel<false><<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
       *x, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
   VDM_CHECK_LAUNCH();
   return VDM_OK;
@@ -411,7 +427,59 @@ extern "C" int vdm_upsample2(const VdmTensor* coarse, const VdmTensor* y, int ba
   if (stats_channels <= 0) stats_channels = channels;
   const int planes = channels / 8;
   const int64_t vf = (int64_t)depth * height * width;
-  upsample2_kernel<<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+  upsample2_kernel<false><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+      *coarse, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
+// ---- fp32 channel-planar forms (TF32 inference mode): 4 channels per plane ----------------------------------------
+extern "C" int vdm_gn_silu_f32(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels, int groups,
+                               const double* stats, const float* gamma, const float* beta, float eps, void* stream) {
+  VDM_CHECK_ARG(view_ok_f32(x, channels) && view_ok_f32(y, channels) && stats && gamma && beta,
+                "vdm_gn_silu_f32: bad tensor argument");
+  VDM_CHECK_ARG(batch >= 1 && voxels >= 1, "vdm_gn_silu_f32: bad shape");
+  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_gn_silu_f32: batch * planes exceeds 65535");
+  VDM_CHECK_ARG(groups >= 1 && channels % groups == 0, "vdm_gn_silu_f32: %d channels not divisible into %d groups",
+                channels, groups);
+  const int planes = channels / 4;
+  if ((int64_t)batch * channels * voxels * 4 > (int64_t)96 << 20)
+    gn_silu_kernel<true, true><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+        *x, *y, planes, voxels, groups, stats, gamma, beta, eps, 0.f, 0, nullptr, 0);
+  else
+    gn_silu_kernel<false, true><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+        *x, *y, planes, voxels, groups, stats, gamma, beta, eps, 0.f, 0, nullptr, 0);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
+extern "C" int vdm_avgpool2_f32(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
+                                int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
+  VDM_CHECK_ARG(view_ok_f32(x, channels) && view_ok_f32(y, channels) && batch >= 1, "vdm_avgpool2_f32: bad argument");
+  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_avgpool2_f32: batch * planes exceeds 65535");
+  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_avgpool2_f32: grid too large for 32-bit voxel indices");
+  VDM_CHECK_ARG(depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0,
+                "vdm_avgpool2_f32: grid (%d,%d,%d) must be even", depth, height, width);
+  if (stats_channels <= 0) stats_channels = channels;
+  const int planes = channels / 4;
+  const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);
+  avgpool2_kernel<true><<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+      *x, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
+extern "C" int vdm_upsample2_f32(const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height, int width,
+                                 int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
+  VDM_CHECK_ARG(view_ok_f32(coarse, channels) && view_ok_f32(y, channels) && batch >= 1, "vdm_upsample2_f32: bad argument");
+  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_upsample2_f32: batch * planes exceeds 65535");
+  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_upsample2_f32: grid too large for 32-bit voxel indices");
+  VDM_CHECK_ARG(depth % 2 == 0 && height % 2 == 0 && width % 2 == 0 && depth >= 2 && height >= 2 && width >= 2,
+                "vdm_upsample2_f32: fine grid (%d,%d,%d) must be even", depth, height, width);
+  if (stats_channels <= 0) stats_channels = channels;
+  const int planes = channels / 4;
+  const int64_t vf = (int64_t)depth * height * width;
+  upsample2_kernel<true><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
       *coarse, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
   VDM_CHECK_LAUNCH();
   return VDM_OK;

@@ -10,48 +10,52 @@ namespace vdm {
 
 constexpr int kEwThreads = 256;
 
-// Reduce per-thread (sum[8], sq[8]) over the block, then 16 fp64 atomics into stats[c0..c0+8).
-__device__ __forceinline__ void block_flush_stats(float (&sum)[8], float (&sq)[8], double* __restrict__ stats8) {
-  __shared__ float s_part[kEwThreads / 32][16];
+// Reduce per-thread (sum[L], sq[L]) over the block, then 2L fp64 atomics into stats[c0..c0+L) (L = 8 bf16 or 4 fp32 lanes).
+template <int L = 8>
+__device__ __forceinline__ void block_flush_stats(float (&sum)[L], float (&sq)[L], double* __restrict__ stats8) {
+  __shared__ float s_part[kEwThreads / 32][2 * L];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-  for (int j = 0; j < 8; ++j) {
+  for (int j = 0; j < L; ++j) {
     sum[j] = warp_sum(sum[j]);
     sq[j] = warp_sum(sq[j]);
   }
   if (lane == 0) {
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
+    for (int j = 0; j < L; ++j) {
       s_part[warp][j] = sum[j];
-      s_part[warp][8 + j] = sq[j];
+      s_part[warp][L + j] = sq[j];
     }
   }
   __syncthreads();
-  if (threadIdx.x < 16) {
+  if (threadIdx.x < 2 * L) {
     float acc = 0.f;
 #pragma unroll
     for (int w = 0; w < kEwThreads / 32; ++w) acc += s_part[w][threadIdx.x];
-    // stats layout: [channel][2]; threadIdx.x < 8 -> sums, >= 8 -> sums of squares
-    atomicAdd(stats8 + 2 * (threadIdx.x & 7) + (threadIdx.x >> 3), (double)acc);
+    // stats layout: [channel][2]; threadIdx.x < L -> sums, >= L -> sums of squares
+    atomicAdd(stats8 + 2 * (threadIdx.x % L) + (threadIdx.x / L), (double)acc);
   }
   __syncthreads();
 }
 
-__device__ __forceinline__ const bf16x8* plane_ptr(const VdmTensor& t, int b, int plane, int64_t voxels) {
-  return reinterpret_cast<const bf16x8*>(t.data) + ((int64_t)b * t.planes + t.plane0 + plane) * voxels;
+template <typename T = bf16x8>
+__device__ __forceinline__ const T* plane_ptr(const VdmTensor& t, int b, int plane, int64_t voxels) {
+  return reinterpret_cast<const T*>(t.data) + ((int64_t)b * t.planes + t.plane0 + plane) * voxels;
 }
-__device__ __forceinline__ bf16x8* plane_ptr_mut(const VdmTensor& t, int b, int plane, int64_t voxels) {
-  return reinterpret_cast<bf16x8*>(t.data) + ((int64_t)b * t.planes + t.plane0 + plane) * voxels;
+template <typename T = bf16x8>
+__device__ __forceinline__ T* plane_ptr_mut(const VdmTensor& t, int b, int plane, int64_t voxels) {
+  return reinterpret_cast<T*>(t.data) + ((int64_t)b * t.planes + t.plane0 + plane) * voxels;
 }
 
-// ---- GroupNorm scale/shift of the 8 channels of one plane ------------------------------------
+// ---- GroupNorm scale/shift of the L (8 bf16 or 4 fp32) channels of one plane ----------------------
 // y = x*scale + shift  ==  gamma*(x-mean)*rstd + beta ; stats are [B][C][2] for exactly this tensor.
+template <int L = 8>
 __device__ __forceinline__ void plane_scale_shift(const double* __restrict__ stats_b, int C, int groups, int pl,
                                                   double voxels, const float* __restrict__ gamma,
                                                   const float* __restrict__ beta, float eps, float* s_scale,
                                                   float* s_shift, float* s_mean, float* s_rstd) {
-  if (threadIdx.x < 8) {
-    const int c = pl * 8 + threadIdx.x;
+  if (threadIdx.x < L) {
+    const int c = pl * L + threadIdx.x;
     const int cpg = C / groups;
     const int g0 = (c / cpg) * cpg;
     double s1 = 0.0, s2 = 0.0;
@@ -98,6 +102,11 @@ static inline dim3 ew_grid(int64_t voxels, int batch_planes) {
 
 static inline bool view_ok(const VdmTensor* t, int channels) {
   return t && t->data && channels >= 8 && channels % 8 == 0 && t->plane0 >= 0 && t->planes >= t->plane0 + channels / 8 &&
+         (reinterpret_cast<uintptr_t>(t->data) & 15) == 0;
+}
+// The same for an fp32 channel-planar view (4 channels per plane).
+static inline bool view_ok_f32(const VdmTensor* t, int channels) {
+  return t && t->data && channels >= 4 && channels % 4 == 0 && t->plane0 >= 0 && t->planes >= t->plane0 + channels / 4 &&
          (reinterpret_cast<uintptr_t>(t->data) & 15) == 0;
 }
 

@@ -165,60 +165,77 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem desc] * B[smem desc]; bf16 inputs, fp32 accumulate (kind::f16).
+// Operand type of a tcgen05.mma: bf16 (kind::f16) or tf32 (kind::tf32).  One K step is 32 bytes of each operand in both
+// kinds (K = 16 bf16 or K = 8 tf32), so the shared-memory descriptors of a K step are the same; only the instruction's
+// kind and the A / B format fields of the instruction descriptor differ.
+enum class MmaKind { kF16, kTF32 };
+#define VDM_UMMA_KIND_ASM(K, BODY) \
+  if constexpr (K == MmaKind::kTF32) asm volatile(BODY("tf32")); else asm volatile(BODY("f16"))
+
+// D[tmem] (+)= A[smem desc] * B[smem desc]; bf16 (or tf32) inputs, fp32 accumulate.
+#define VDM_UMMA_BODY(KIND)                                                                    \
+      "{\n\t"                                                                                  \
+      ".reg .pred p;\n\t"                                                                      \
+      "setp.ne.b32 p, %4, 0;\n\t"                                                              \
+      "tcgen05.mma.cta_group::1.kind::" KIND " [%0], %1, %2, %3, p;\n\t"                       \
+      "}" ::"r"(d_tmem),                                                                       \
+      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)                                    \
+      : "memory"
+template <MmaKind K = MmaKind::kF16>
 __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
                                           uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
+  VDM_UMMA_KIND_ASM(K, VDM_UMMA_BODY);
 }
+#undef VDM_UMMA_BODY
 // Same, with the descriptors assembled INSIDE the asm block from warp-uniform bases plus per-MMA offsets:
 //   a_desc = {a_lo + a_off, a_hi32}, b_desc = {b_lo + b_off, b_hi32}, d = d_tmem + d_off.
 // Keeping the adds next to the (volatile) MMA stops ptxas from pre-computing hundreds of descriptors into vector
 // registers and moving them back with R2UR (r01s: ~65 issue cycles per MMA in the unrolled schedule).
+#define VDM_UMMA_OFF_BODY(KIND)                                                                \
+      "{\n\t"                                                                                  \
+      ".reg .pred p;\n\t"                                                                      \
+      ".reg .b32 alo, blo, dd;\n\t"                                                            \
+      ".reg .b64 da, db;\n\t"                                                                  \
+      "add.u32 alo, %1, %2;\n\t"                                                               \
+      "add.u32 blo, %4, %5;\n\t"                                                               \
+      "add.u32 dd, %0, %9;\n\t"                                                                \
+      "mov.b64 da, {alo, %3};\n\t"                                                             \
+      "mov.b64 db, {blo, %6};\n\t"                                                             \
+      "setp.ne.b32 p, %8, 0;\n\t"                                                              \
+      "tcgen05.mma.cta_group::1.kind::" KIND " [dd], da, db, %7, p;\n\t"                       \
+      "}" ::"r"(d_tmem),                                                                       \
+      "r"(a_lo), "r"(a_off), "r"(a_hi32), "r"(b_lo), "r"(b_off), "r"(b_hi32), "r"(idesc), "r"(accumulate), "r"(d_off) \
+      : "memory"
+template <MmaKind K = MmaKind::kF16>
 __device__ __forceinline__ void umma_bf16_off(uint32_t d_tmem, uint32_t d_off, uint32_t a_lo, uint32_t a_off, uint32_t a_hi32,
                                               uint32_t b_lo, uint32_t b_off, uint32_t b_hi32, uint32_t idesc,
                                               uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      ".reg .b32 alo, blo, dd;\n\t"
-      ".reg .b64 da, db;\n\t"
-      "add.u32 alo, %1, %2;\n\t"
-      "add.u32 blo, %4, %5;\n\t"
-      "add.u32 dd, %0, %9;\n\t"
-      "mov.b64 da, {alo, %3};\n\t"
-      "mov.b64 db, {blo, %6};\n\t"
-      "setp.ne.b32 p, %8, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [dd], da, db, %7, p;\n\t"
-      "}" ::"r"(d_tmem),
-      "r"(a_lo), "r"(a_off), "r"(a_hi32), "r"(b_lo), "r"(b_off), "r"(b_hi32), "r"(idesc), "r"(accumulate), "r"(d_off)
-      : "memory");
+  VDM_UMMA_KIND_ASM(K, VDM_UMMA_OFF_BODY);
 }
+#undef VDM_UMMA_OFF_BODY
 // Same with whole 64-bit descriptors plus per-MMA offsets: ONE UIADD3.64 per descriptor in SASS (the 32-bit form above costs an
 // add for the low word and a move for the high word of every descriptor pair: R3e, 6 uniform instructions per MMA from a single
 // issuing thread that has ~56 cycles per MMA).  The low words (address >> 4 | LBO << 16) never carry into the high ones.
+#define VDM_UMMA_OFF64_BODY(KIND)                                                              \
+      "{\n\t"                                                                                  \
+      ".reg .pred p;\n\t"                                                                      \
+      ".reg .b32 dd;\n\t"                                                                      \
+      ".reg .b64 da, db;\n\t"                                                                  \
+      "add.u64 da, %1, %2;\n\t"                                                                \
+      "add.u64 db, %3, %4;\n\t"                                                                \
+      "add.u32 dd, %0, %7;\n\t"                                                                \
+      "setp.ne.b32 p, %6, 0;\n\t"                                                              \
+      "tcgen05.mma.cta_group::1.kind::" KIND " [dd], da, db, %5, p;\n\t"                       \
+      "}" ::"r"(d_tmem),                                                                       \
+      "l"(a_desc), "l"((uint64_t)a_off), "l"(b_desc), "l"((uint64_t)b_off), "r"(idesc), "r"(accumulate), "r"(d_off) \
+      : "memory"
+template <MmaKind K = MmaKind::kF16>
 __device__ __forceinline__ void umma_bf16_off64(uint32_t d_tmem, uint32_t d_off, uint64_t a_desc, uint32_t a_off, uint64_t b_desc,
                                                 uint32_t b_off, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      ".reg .b32 dd;\n\t"
-      ".reg .b64 da, db;\n\t"
-      "add.u64 da, %1, %2;\n\t"
-      "add.u64 db, %3, %4;\n\t"
-      "add.u32 dd, %0, %7;\n\t"
-      "setp.ne.b32 p, %6, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [dd], da, db, %5, p;\n\t"
-      "}" ::"r"(d_tmem),
-      "l"(a_desc), "l"((uint64_t)a_off), "l"(b_desc), "l"((uint64_t)b_off), "r"(idesc), "r"(accumulate), "r"(d_off)
-      : "memory");
+  VDM_UMMA_KIND_ASM(K, VDM_UMMA_OFF64_BODY);
 }
+#undef VDM_UMMA_OFF64_BODY
+#undef VDM_UMMA_KIND_ASM
 // Arrive on `bar` when all previously issued tcgen05.mma of this thread have completed.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -267,10 +284,12 @@ __device__ __forceinline__ uint64_t make_kmajor_desc(uint32_t smem_addr, uint32_
   d |= layout << 61;
   return d;
 }
-// Instruction descriptor (InstrDescriptor): D=f32 [4,6)=1, A=bf16 [7,10)=1, B=bf16 [10,13)=1,
-// A,B K-major (bits 15,16 = 0), N>>3 [17,23), M>>4 [24,29).
+// Instruction descriptor (InstrDescriptor): D=f32 [4,6)=1, A format [7,10), B format [10,13) (kind::f16: bf16 = 1;
+// kind::tf32: tf32 = 2), A,B K-major (bits 15,16 = 0), N>>3 [17,23), M>>4 [24,29).
+template <MmaKind K = MmaKind::kF16>
 __device__ __host__ __forceinline__ uint32_t make_idesc_bf16(uint32_t m, uint32_t n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+  constexpr uint32_t ab = K == MmaKind::kTF32 ? 2u : 1u;
+  return (1u << 4) | (ab << 7) | (ab << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
 }
 
 }  // namespace ptx

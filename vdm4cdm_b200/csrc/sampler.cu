@@ -95,22 +95,37 @@ philox_normal_kernel(float* __restrict__ out, int64_t voxels, uint64_t seed,
   }
 }
 
-// z fp32 + cond fp32 planes -> channel-planar bf16: plane 0 = (z, cond_1..cond_n, 0...), other planes 0
+// z fp32 + cond fp32 planes -> channel-planar bf16: plane 0 = (z, cond_1..cond_n, 0...), other planes 0.
+// F32: fp32 channel-planar, the same 8 channels in planes 0 and 1.
+template <bool F32 = false>
 __global__ void __launch_bounds__(256)
 pack_input_kernel(const float* __restrict__ z, const float* __restrict__ cond, VdmTensor out, int planes,
                   int64_t voxels, int n_cond) {
+  using T = typename Unit<F32>::T;
+  constexpr int L = Unit<F32>::L, P = 8 / L;       // planes holding (z, cond_1..cond_7)
   const int b = blockIdx.y;
-  bf16x8* ob = reinterpret_cast<bf16x8*>(out.data) + ((int64_t)b * out.planes + out.plane0) * voxels;
+  T* ob = reinterpret_cast<T*>(out.data) + ((int64_t)b * out.planes + out.plane0) * voxels;
   for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < voxels;
        v += (int64_t)gridDim.x * blockDim.x) {
-    float f[8];
 #pragma unroll
-    for (int j = 0; j < 8; ++j)
-      f[j] = (j == 0) ? z[(int64_t)b * voxels + v]
-                      : (j <= n_cond ? cond[((int64_t)b * n_cond + (j - 1)) * voxels + v] : 0.f);
-    ob[v] = pack8(f);
-    const float zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    for (int pl = 1; pl < planes; ++pl) ob[(int64_t)pl * voxels + v] = pack8(zero);
+    for (int q = 0; q < P; ++q) {
+      float f[L];
+#pragma unroll
+      for (int i = 0; i < L; ++i) {
+        const int j = q * L + i;
+        f[i] = (j == 0) ? z[(int64_t)b * voxels + v]
+                        : (j <= n_cond ? cond[((int64_t)b * n_cond + (j - 1)) * voxels + v] : 0.f);
+      }
+      T u;
+      pack_unit(f, u);
+      ob[(int64_t)q * voxels + v] = u;
+    }
+    const float zero[L] = {};
+    for (int pl = P; pl < planes; ++pl) {
+      T u;
+      pack_unit(zero, u);
+      ob[(int64_t)pl * voxels + v] = u;
+    }
   }
 }
 
@@ -162,7 +177,21 @@ extern "C" int vdm_pack_input(const float* z, const float* cond, const VdmTensor
                 "vdm_pack_input: bad c_pad %d / n_cond %d / plane window", c_pad, n_cond);
   VDM_CHECK_ARG(n_cond == 0 || cond, "vdm_pack_input: cond is NULL with n_cond=%d", n_cond);
   const dim3 grid = vdm::grid_for(voxels, batch, 256);
-  vdm::pack_input_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / 8, voxels, n_cond);
+  vdm::pack_input_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / 8, voxels, n_cond);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
+extern "C" int vdm_pack_input_f32(const float* z, const float* cond, const VdmTensor* out, int batch, int64_t voxels,
+                                  int n_cond, int c_pad, void* stream) {
+  VDM_CHECK_ARG(z && out && out->data && batch >= 1 && batch <= 65535 && voxels >= 1 &&
+                    (reinterpret_cast<uintptr_t>(out->data) & 15) == 0, "vdm_pack_input_f32: bad argument");
+  VDM_CHECK_ARG(c_pad >= 8 && c_pad % 8 == 0 && n_cond >= 0 && n_cond + 1 <= 8 && out->plane0 >= 0 &&
+                    out->planes >= out->plane0 + c_pad / 4,
+                "vdm_pack_input_f32: bad c_pad %d / n_cond %d / plane window", c_pad, n_cond);
+  VDM_CHECK_ARG(n_cond == 0 || cond, "vdm_pack_input_f32: cond is NULL with n_cond=%d", n_cond);
+  const dim3 grid = vdm::grid_for(voxels, batch, 256);
+  vdm::pack_input_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / 4, voxels, n_cond);
   VDM_CHECK_LAUNCH();
   return VDM_OK;
 }

@@ -99,8 +99,14 @@ class CUNet(nn.Module):
                  v_conditioning_dims: Sequence[int] = (), t_conditioning: bool = False, norm_groups: int = 8,
                  mid_attn: bool = False, dropout_prob: float = 0.1, conv_padding_mode: str = "zeros",
                  n_attention_heads: int = 4, t_embedding_dim: int = 64, v_embedding_dim: int = 64,
-                 out_channels: Optional[int] = None):
+                 out_channels: Optional[int] = None, precision: str = "bf16"):
         super().__init__()
+        # Inference precision of the convolutional trunk: "bf16" (bf16 channel-planar activations, bf16 tensor-core convs) or
+        # "tf32" (fp32 channel-planar activations, tcgen05 kind::tf32 convs -- the reference's own cuDNN TF32 class of
+        # accuracy, for A/B comparisons).  A plain attribute: it may be changed on a loaded model.  TF32 is inference-only
+        # and runs the unfused path (no fuse_gn / fuse_upsample / polyphase_up / fused skip conv).
+        self.precision = precision
+        self._check_precision()
         if len(shape) != 4:
             raise NotImplementedError("vdm4cdm_b200.CUNet covers the 3-D networks (shape=(C, D, H, W)) only")
         if mid_attn:
@@ -178,6 +184,30 @@ class CUNet(nn.Module):
         # device-side training-step counter added to the dropout seed (a captured CUDA graph draws new masks)
         self.register_buffer("drop_counter", torch.zeros(1, dtype=torch.int32), persistent=False)
 
+    PRECISIONS = ("bf16", "tf32")
+
+    def _check_precision(self) -> bool:
+        """True in TF32 mode; ValueError for an unknown ``precision``."""
+        if self.precision not in self.PRECISIONS:
+            raise ValueError(f"CUNet.precision must be one of {self.PRECISIONS}, got {self.precision!r}")
+        return self.precision == "tf32"
+
+    def _lanes(self) -> int:
+        """Channels per plane of the trunk's planar activations: 8 (bf16) or 4 (TF32 mode, fp32)."""
+        return 4 if self.precision == "tf32" else 8
+
+    def _planar(self, ar: "_Arena", name: str, b: int, ch: int, grid, dev) -> torch.Tensor:
+        """Arena buffer of a ``ch``-channel planar activation on ``grid`` in the trunk's precision: bf16 [b, ch/8, *grid, 8]
+        or (TF32) fp32 [b, ch/4, *grid, 4]."""
+        lanes = self._lanes()
+        if lanes == 4:       # own buffers: a CUDA graph captured in the other precision keeps valid pointers
+            return ar.get("f32." + name, (b, ch // 4) + tuple(grid) + (4,), torch.float32, dev)
+        return ar.get(name, (b, ch // 8) + tuple(grid) + (8,), torch.bfloat16, dev)
+
+    def input_channels_pad(self) -> int:
+        """Channels of the packed network input (``ops.pack_input``'s ``c_pad``): 16 bf16 or 8 fp32 = two planes."""
+        return 8 if self.precision == "tf32" else 16
+
     # ---- conditioning (tiny fp32 MLPs, torch) -------------------------------------------------
     def conditionings(self, batch: int, t, v_conditionings, device) -> Optional[List[torch.Tensor]]:
         """List of fp32 [..., B, dim] embeddings (time first, then one per parameter vector).
@@ -205,8 +235,26 @@ class CUNet(nn.Module):
 
     def _packed(self, name: str, conv: nn.Conv3d) -> torch.Tensor:
         """bf16 kernel-layout copy of ``conv.weight`` (one ``vdm_pack_conv_weight`` launch when the parameter changed;
-        the buffer is allocated once, so captured CUDA graphs keep a valid pointer)."""
+        the buffer is allocated once, so captured CUDA graphs keep a valid pointer).  In TF32 mode the fp32 filter of
+        ``vdm_conv3d_tf32``, kept in its own slot so that switching precision does not re-pack."""
+        if self.precision == "tf32":
+            return self._packed_f32(name, conv)
         return self._packed_any(name, conv, False, 0, conv.in_channels)
+
+    def _packed_f32(self, name: str, conv: nn.Conv3d) -> torch.Tensor:
+        w = conv.weight
+        key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
+        slot = name + ".f32"
+        hit = self._packed_cache.get(slot)
+        if hit is None or hit[0] != key:
+            with torch.no_grad():
+                shape = ops.packed_weight_shape(w.shape, dtype=torch.float32)
+                buf = hit[1] if hit is not None and tuple(hit[1].shape) == shape and hit[1].device == w.device else \
+                    torch.empty(shape, dtype=torch.float32, device=w.device)
+                ops.pack_conv_weight_into(w.detach().contiguous(), buf)
+                hit = (key, buf)
+            self._packed_cache[slot] = hit
+        return hit[1]
 
     def _packed_dgrad(self, name: str, conv: nn.Conv3d, c0: int, n: int) -> torch.Tensor:
         """bf16 dgrad filter (roles of Cin/Cout exchanged, taps mirrored) for input channels [c0, c0+n)."""
@@ -390,10 +438,11 @@ class CUNet(nn.Module):
         # marching schedule (four warps take whole slices in turn).  In between (narrow output, more than 32 input channels:
         # the kd-folded TILE schedule) the transform's LDS / STS traffic costs more than the HBM pass it replaces
         # (+0.55 ms on a 0.85 ms conv even as a plain copy, profiles/R2h_transform_ablation.txt).
-        fuse_ok = self.fuse_gn and tape is None and not self.circular and p_drop == 0.0
+        tf32 = self._check_precision()
+        fuse_ok = self.fuse_gn and tape is None and not self.circular and p_drop == 0.0 and not tf32
         fuse_gn = fuse_ok and (co >= self.fuse_gn_min_channels or (self.fuse_gn_narrow and co <= 32))      # net2 reads h (co channels)
         fuse_gn1 = fuse_ok and (co >= self.fuse_gn_min_channels or (self.fuse_gn_narrow and ci <= 32 and co <= 32))
-        h = ar.get(f"{own}h.{co}.{tag}", (b, co // 8) + grid + (8,), torch.bfloat16, dev)
+        h = self._planar(ar, f"{own}h.{co}.{tag}", b, co, grid, dev)
         h_stats = self._stats(f"{name}.h", b, co, dev)
         net1_kw = dict(out=h, chan_add=rows[name + ".net1"], step_ptr=step_ptr if rows[name + ".net1"].dim() == 3 else None,
                        stats=h_stats, circular=self.circular)
@@ -401,7 +450,7 @@ class CUNet(nn.Module):
             coef1 = ops.gn_coef(x_stats, n1.weight, n1.bias, g, voxels, n1.eps,
                                 out=ar.get(f"coef1.{name}.{b}", (b, ci, 2), torch.float32, dev))
             ops.conv3d(x, self._packed(name + ".net1", blk.net1[2]), co, x_plane0=x_plane0, c_in=ci, in_norm=coef1, **net1_kw)
-        elif up_from is not None and self.polyphase_up and not self.circular:
+        elif up_from is not None and self.polyphase_up and not self.circular and not tf32:
             xc, xc_plane0, c_up = up_from
             cgrid = tuple(n // 2 for n in grid)
             # silu(gn(.)) of the coarse channels at the COARSE resolution (statistics of the fine concat)
@@ -434,7 +483,7 @@ class CUNet(nn.Module):
                 ops.gn_silu_view(x, c_sk, c_up, ci, g, x_stats, n1.weight, n1.bias, n1.eps, a_s, x_plane0=x_plane0 + c_up // 8)
                 ops.conv3d(a_s, w_sk, co, residual=part, residual_upsample="d2s", **net1_kw)
         else:
-            a1 = ar.get(f"{own}a.{ci}.{tag}", (b, ci // 8) + grid + (8,), torch.bfloat16, dev)
+            a1 = self._planar(ar, f"{own}a.{ci}.{tag}", b, ci, grid, dev)
             if up_from is None:
                 ops.gn_silu(x, ci, g, x_stats, n1.weight, n1.bias, n1.eps, x_plane0=x_plane0, out=a1)
             else:
@@ -455,8 +504,7 @@ class CUNet(nn.Module):
                                    out=ar.get(f"coef2.{name}.{b}", (b, co, 2), torch.float32, dev))
         else:
             in_norm2 = None
-            a2 = ar.get(f"{own}a2.{co}.{tag}" if tape is not None else f"a.{co}.{tag}", (b, co // 8) + grid + (8,),
-                        torch.bfloat16, dev)
+            a2 = self._planar(ar, f"{own}a2.{co}.{tag}" if tape is not None else f"a.{co}.{tag}", b, co, grid, dev)
             ops.gn_silu(h, co, g, h_stats, n2.weight, n2.bias, n2.eps, out=a2, dropout_p=p_drop,
                         seed=self.dropout_seed, layer_tag=self._dropout_calls,
                         seed_step=self.drop_counter if p_drop > 0.0 else None)
@@ -473,7 +521,7 @@ class CUNet(nn.Module):
             ops.conv3d(xc, self._packed_in_slice(name + ".skip.up", blk.skip_conv, 0, c_up), co, taps=ops.TAPS_1X1X1,
                        x_plane0=xc_plane0, c_in=c_up, out=rc, chan_add=rows[name + ".skip"])
             w_skip = self._packed_in_slice(name + ".skip.skip", blk.skip_conv, c_up, ci - c_up)
-            if self._fused_skip_ok.get(name, True):
+            if self._fused_skip_ok.get(name, True) and not tf32:
                 # fine half fused into net2's conv as one more channel chunk (centre tap only): no separate 1x1x1 launch,
                 # and the residual the epilogue reads is the coarse tensor (1/8 of the bytes)
                 try:
@@ -484,12 +532,12 @@ class CUNet(nn.Module):
                     return
                 except ops.UnsupportedFusion:
                     self._fused_skip_ok[name] = False          # wide layer: keep the skip conv as its own launch
-            res = ar.get(f"{own}r.{co}.{tag}", (b, co // 8) + grid + (8,), torch.bfloat16, dev)
+            res = self._planar(ar, f"{own}r.{co}.{tag}", b, co, grid, dev)
             ops.conv3d(x, w_skip, co, taps=ops.TAPS_1X1X1, x_plane0=x_plane0 + c_up // 8, c_in=ci - c_up, out=res,
                        residual=rc, residual_upsample=True)
             res_plane0 = 0
         else:
-            res = ar.get(f"{own}r.{co}.{tag}", (b, co // 8) + grid + (8,), torch.bfloat16, dev)
+            res = self._planar(ar, f"{own}r.{co}.{tag}", b, co, grid, dev)
             ops.conv3d(x, self._packed(name + ".skip", blk.skip_conv), co, taps=ops.TAPS_1X1X1, x_plane0=x_plane0, c_in=ci,
                        out=res, chan_add=rows[name + ".skip"])
             res_plane0 = 0
@@ -506,7 +554,7 @@ class CUNet(nn.Module):
         d, h, w = x.shape[2:5]
         ar = self._arena if tape is None else self._train_arena
         name = (slot if tape is not None else "pad") + f".{ch}.{b}x{d}"
-        buf = ar.get(name, (b, ch // 8, d + 2, h + 2, w + 2, 8), torch.bfloat16, x.device)
+        buf = self._planar(ar, name, b, ch, (d + 2, h + 2, w + 2), x.device)
         ops.pad_circular(x, ch, x_plane0=x_plane0, out=buf)
         return buf, 0
 
@@ -524,7 +572,12 @@ class CUNet(nn.Module):
         """eps_hat fp32 (B, 1, D, H, W) from the packed network input (``ops.pack_input``).
 
         ``tape`` (a dict, training only): intermediates live in a separate arena, nothing is shared between
-        layers, and every tensor the backward pass needs is recorded in it (``vdm4cdm_b200.autograd``)."""
+        layers, and every tensor the backward pass needs is recorded in it (``vdm4cdm_b200.autograd``).
+        In TF32 mode ``packed`` is the fp32 planar input and ``tape`` is refused (the mode is inference-only)."""
+        tf32 = self._check_precision()
+        if tf32 and tape is not None:
+            raise NotImplementedError("CUNet precision='tf32' is inference-only (no training tape)")
+        lanes = self._lanes()
         b = packed.shape[0]
         dev = packed.device
         c = self.chs
@@ -537,12 +590,12 @@ class CUNet(nn.Module):
         self._dropout_calls = 0
 
         def buf(name, ch, lvl):
-            return ar.get(f"{name}.{b}", (b, ch // 8) + grids[lvl] + (8,), torch.bfloat16, dev)
+            return self._planar(ar, f"{name}.{b}", b, ch, grids[lvl], dev)
 
         # conv_in
         h = buf("h_in", c[0], 0)
         h_stats = self._stats("conv_in", b, c[0], dev)
-        packed_c, _ = self._conv_input(packed, 16, 0, "conv_in.xp", tape)
+        packed_c, _ = self._conv_input(packed, self.input_channels_pad(), 0, "conv_in.xp", tape)
         ops.conv3d(packed_c, self._packed("conv_in", self.conv_in), c[0], out=h, chan_add=rows["conv_in"], stats=h_stats,
                    circular=self.circular)
         x, x_plane0, x_stats = h, 0, h_stats
@@ -555,11 +608,11 @@ class CUNet(nn.Module):
                 cat = buf(f"cat{i}", c[i + 1] + c[i], i)
                 cst = self._stats(f"cat{i}", b, c[i + 1] + c[i], dev)
                 cats[i], cat_stats[i] = cat, cst
-                self._run_block(name, blk, x, x_plane0, x_stats, rows, step_ptr, cat, c[i + 1] // 8, cst, c[i + 1],
+                self._run_block(name, blk, x, x_plane0, x_stats, rows, step_ptr, cat, c[i + 1] // lanes, cst, c[i + 1],
                                 grids[i], training_dropout, tape)
                 pooled = buf(f"pool{i}", c[i], i + 1)
                 pst = self._stats(f"pool{i}", b, c[i], dev)
-                ops.avgpool2(cat, c[i], x_plane0=c[i + 1] // 8, out=pooled, stats=pst)
+                ops.avgpool2(cat, c[i], x_plane0=c[i + 1] // lanes, out=pooled, stats=pst)
                 x, x_plane0, x_stats = pooled, 0, pst
             else:
                 o = buf("bottom0", c[i], i)
@@ -579,7 +632,7 @@ class CUNet(nn.Module):
             cat, cst = cats[i], cat_stats[i]
             o = buf(f"up{i}", c[i], i)
             ost = self._stats(name + ".out", b, c[i], dev)
-            if self.fuse_upsample and tape is None and blk.skip_conv is not None:
+            if self.fuse_upsample and tape is None and blk.skip_conv is not None and not tf32:
                 # the up-sampled channels are never written (see _run_block); their sums are 8x the coarse tensor's
                 torch.mul(x_stats, 8.0, out=cst[:, :c[i + 1]])
                 self._run_block(name, blk, cat, 0, cst, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout, tape,
@@ -591,14 +644,13 @@ class CUNet(nn.Module):
         gn = self.conv_out[0]
         if out is None:
             out = torch.empty((b, 1) + grids[0], dtype=torch.float32, device=dev)
-        if self.fuse_gn and tape is None and not self.circular and (self.fuse_gn_narrow and c[0] <= 32 or self.fuse_gn_min_channels <= 1):
+        if self.fuse_gn and tape is None and not self.circular and not tf32 and (self.fuse_gn_narrow and c[0] <= 32 or self.fuse_gn_min_channels <= 1):
             coef = ops.gn_coef(x_stats, gn.weight, gn.bias, gn.num_groups, grids[0][0] * grids[0][1] * grids[0][2], gn.eps,
                                out=ar.get(f"coef.conv_out.{b}", (b, c[0], 2), torch.float32, dev))
             ops.conv3d(x, self._packed("conv_out", self.conv_out[2]), 1, x_plane0=x_plane0, c_in=c[0], out=out, out_fp32=True,
                        chan_add=rows["conv_out"], in_norm=coef)
             return out
-        a = ar.get(("conv_out." if tape is not None else "") + f"a.{c[0]}.{b}x{grids[0][0]}",
-                   (b, c[0] // 8) + grids[0] + (8,), torch.bfloat16, dev)
+        a = self._planar(ar, ("conv_out." if tape is not None else "") + f"a.{c[0]}.{b}x{grids[0][0]}", b, c[0], grids[0], dev)
         ops.gn_silu(x, c[0], gn.num_groups, x_stats, gn.weight, gn.bias, gn.eps, out=a)
         a_c, _ = self._conv_input(a, c[0], 0, "conv_out.ap", tape)
         if tape is not None:
@@ -611,14 +663,17 @@ class CUNet(nn.Module):
         """eps_hat / v_hat (B, 1, D, H, W) fp32.  Under ``torch.no_grad()`` this is the inference path; with
         gradients enabled it goes through ``vdm4cdm_b200.autograd.unet_forward`` (dropout active iff
         ``self.training``)."""
+        tf32 = self._check_precision()
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            if tf32:
+                raise NotImplementedError("CUNet precision='tf32' is inference-only: run it under torch.no_grad()")
             from .autograd import unet_forward
             return unet_forward(self, x, t, s_conditioning, v_conditionings)
         with torch.no_grad():
             b = x.shape[0]
             rows = self.chan_add_rows(b, t, v_conditionings, x.device)
             cond = None if s_conditioning is None else s_conditioning.contiguous().float()
-            packed = ops.pack_input(x.contiguous().float(), cond, 16,
-                                    out=self._arena.get(f"packed.{b}", (b, 2) + self.shape[1:] + (8,), torch.bfloat16,
-                                                        x.device))
+            packed = ops.pack_input(x.contiguous().float(), cond, self.input_channels_pad(),
+                                    out=self._planar(self._arena, f"packed.{b}", b, self.input_channels_pad(), self.shape[1:],
+                                                     x.device))
             return self.run_packed(packed, rows)

@@ -5,6 +5,11 @@ raises ``RuntimeError`` on failure.  There is no PyTorch fallback for any of the
 Channel-planar activations are torch bf16 tensors of shape ``[B, P, D, H, W, 8]`` (P planes of 8
 channels); a *view* ``(buf, plane0, channels)`` addresses ``channels`` consecutive channels of a
 wider buffer, which is how channel concatenation is expressed without copies.
+
+The TF32 inference mode uses fp32 channel-planar tensors ``[B, P, D, H, W, 4]`` (P planes of 4 channels, the same
+16 bytes per voxel and plane).  ``conv3d``, ``gn_silu``, ``avgpool2``, ``upsample2``, ``pad_circular``, ``pack_input``
+and ``pack_conv_weight_into`` dispatch on the planar tensors' dtype; mixing bf16 and fp32 in one call raises
+``ValueError``.
 """
 from __future__ import annotations
 
@@ -69,24 +74,42 @@ def _planar_ok(t: torch.Tensor, name: str) -> None:
           f"{name}: expected a contiguous CUDA bf16 [B,P,D,H,W,8] tensor, got {tuple(t.shape)} {t.dtype} {t.device}")
 
 
+_LANES = {torch.bfloat16: 8, torch.float32: 4}       # channels per 16-byte plane of a planar tensor
+
+
+def _planar_lanes(t: torch.Tensor, name: str) -> int:
+    """Channels per plane (8: bf16, 4: fp32) of a contiguous CUDA channel-planar tensor."""
+    lanes = _LANES.get(t.dtype)
+    _need(t.is_cuda and lanes is not None and t.dim() == 6 and t.shape[-1] == lanes and t.is_contiguous(),
+          f"{name}: expected a contiguous CUDA bf16 [B,P,D,H,W,8] or fp32 [B,P,D,H,W,4] tensor, got "
+          f"{tuple(t.shape)} {t.dtype} {t.device}")
+    return lanes
+
+
+def _same_lanes(lanes: int, t: torch.Tensor, name: str) -> None:
+    _need(_planar_lanes(t, name) == lanes, f"{name}: bf16 and fp32 planar tensors mixed in one call")
+
+
 def _view(t: torch.Tensor, plane0: int) -> _C.Tensor:
     return _C.Tensor(t.data_ptr(), t.shape[1], plane0)
 
 
 # ---- layout helpers (host-side glue; run on whatever device the tensor lives on) -------------------
-def to_planar(x: torch.Tensor, pad_to: int = 8) -> torch.Tensor:
-    """(B, C, D, H, W) any float dtype -> bf16 [B, ceil(C/pad_to)*pad_to/8, D, H, W, 8] (zero padded)."""
+def to_planar(x: torch.Tensor, pad_to: int = 8, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """(B, C, D, H, W) any float dtype -> bf16 [B, ceil(C/pad_to)*pad_to/8, D, H, W, 8] (zero padded), or with
+    ``dtype=torch.float32`` fp32 [B, ceil(C/pad_to)*pad_to/4, D, H, W, 4]."""
+    lanes = _LANES[dtype]
     b, c, d, h, w = x.shape
     cp = -(-c // pad_to) * pad_to
     if cp != c:
         x = torch.cat([x, x.new_zeros(b, cp - c, d, h, w)], dim=1)
-    return x.reshape(b, cp // 8, 8, d, h, w).permute(0, 1, 3, 4, 5, 2).contiguous().to(torch.bfloat16)
+    return x.reshape(b, cp // lanes, lanes, d, h, w).permute(0, 1, 3, 4, 5, 2).contiguous().to(dtype)
 
 
 def from_planar(x: torch.Tensor, channels: Optional[int] = None) -> torch.Tensor:
-    """bf16 [B, P, D, H, W, 8] -> fp32 (B, C, D, H, W)."""
-    b, p, d, h, w, _ = x.shape
-    y = x.permute(0, 1, 5, 2, 3, 4).reshape(b, p * 8, d, h, w).float()
+    """bf16 [B, P, D, H, W, 8] or fp32 [B, P, D, H, W, 4] -> fp32 (B, C, D, H, W)."""
+    b, p, d, h, w, lanes = x.shape
+    y = x.permute(0, 1, 5, 2, 3, 4).reshape(b, p * lanes, d, h, w).float()
     return y if channels is None else y[:, :channels]
 
 
@@ -108,9 +131,14 @@ def pack_conv_weight(w: torch.Tensor, c_in_pad: Optional[int] = None, c_out_pad:
     return full.reshape(kd * kh * kw, cip // 8, 8, cop).permute(0, 1, 3, 2).contiguous().to(torch.bfloat16)
 
 
-def packed_weight_shape(conv_weight_shape, transpose_flip: bool = False, n_ci: Optional[int] = None):
-    """Shape of the packed bf16 filter for a torch Conv3d weight (Cout, Cin, k, k, k)."""
+def packed_weight_shape(conv_weight_shape, transpose_flip: bool = False, n_ci: Optional[int] = None,
+                        dtype: torch.dtype = torch.bfloat16):
+    """Shape of the packed bf16 filter for a torch Conv3d weight (Cout, Cin, k, k, k); with ``dtype=torch.float32`` the
+    TF32 forward filter [k^3, ceil(Cin/8)*2, Cout_pad, 4]."""
     co, ci, k = conv_weight_shape[0], conv_weight_shape[1], conv_weight_shape[2]
+    if dtype == torch.float32:
+        _need(not transpose_flip, "packed_weight_shape: the fp32 (TF32) filter is forward-only")
+        return (k ** 3, -(-ci // 8) * 8 // 4, -(-co // 16) * 16, 4)
     if transpose_flip:
         kdim, ndim = co, (ci if n_ci is None else n_ci)
     else:
@@ -121,9 +149,19 @@ def packed_weight_shape(conv_weight_shape, transpose_flip: bool = False, n_ci: O
 def pack_conv_weight_into(w: torch.Tensor, out: torch.Tensor, transpose_flip: bool = False, ci0: int = 0,
                           n_ci: Optional[int] = None) -> torch.Tensor:
     """``vdm_pack_conv_weight``: fp32 CUDA Conv3d weight -> ``out`` (bf16 [k^3, K_pad/8, N_pad, 8]) in one launch.
-    With ``transpose_flip`` the dgrad filter of input channels [ci0, ci0 + n_ci) is packed."""
+    With ``transpose_flip`` the dgrad filter of input channels [ci0, ci0 + n_ci) is packed.  An fp32 ``out``
+    ([k^3, K_pad/4, N_pad, 4], ``packed_weight_shape(..., dtype=torch.float32)``) receives the TF32-rounded forward
+    filter of ``vdm_conv3d_tf32`` (``vdm_pack_conv_weight_f32``)."""
     _need(w.is_cuda and w.dtype == torch.float32 and w.is_contiguous() and w.dim() == 5, "pack_conv_weight_into: w must be contiguous CUDA fp32 (Cout, Cin, k, k, k)")
     co, ci, k = w.shape[0], w.shape[1], w.shape[2]
+    if out.dtype == torch.float32:
+        _need(not transpose_flip and ci0 == 0 and n_ci in (None, ci), "pack_conv_weight_into: the fp32 (TF32) filter is forward-only")
+        _need(out.is_cuda and out.is_contiguous() and tuple(out.shape) == packed_weight_shape(w.shape, dtype=torch.float32),
+              "pack_conv_weight_into: bad out tensor")
+        rc = _C.lib().vdm_pack_conv_weight_f32(w.data_ptr(), out.data_ptr(), co, ci, k, out.shape[1] * 4, out.shape[2], _stream())
+        _C.check(rc, "vdm_pack_conv_weight_f32")
+        _launched(1)
+        return out
     n_ci = ci if n_ci is None else n_ci
     _need(out.is_cuda and out.dtype == torch.bfloat16 and out.is_contiguous() and
           tuple(out.shape) == packed_weight_shape(w.shape, transpose_flip, n_ci), "pack_conv_weight_into: bad out tensor")
@@ -239,16 +277,22 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
     result is fp32 (B, c_out, D, H, W) instead.
     chan_add: fp32 [B, c_out] or [steps, B, c_out] (then ``step_ptr`` selects the row block on device).
     stats: double [B, Cs, 2], accumulated at channel ``stats_c0``.
+
+    fp32 planar ``x`` (TF32 mode, ``vdm_conv3d_tf32``): ``w_packed``, a planar ``out`` and ``residual`` are fp32 planar
+    too (plane windows count 4-channel planes); ``skip_x``, ``in_norm`` and ``residual_upsample`` raise
+    ``UnsupportedFusion``.
     """
-    _planar_ok(x, "conv3d x")
+    lanes = _planar_lanes(x, "conv3d x")
+    tf32 = lanes == 4
     b, xp, d, h, w_, _ = x.shape
     if circular:                       # x carries a one-voxel periodic halo (``pad_circular``)
         d, h, w_ = d - 2, h - 2, w_ - 2
-    n_taps, cin8, c_out_pad, eight = w_packed.shape
-    _need(w_packed.is_cuda and w_packed.dtype == torch.bfloat16 and w_packed.is_contiguous() and eight == 8,
-          "conv3d: w_packed must be a contiguous CUDA bf16 [taps, Cin/8, Cout_pad, 8] tensor")
-    c_in = cin8 * 8 if c_in is None else c_in
-    _need(c_in == cin8 * 8, f"conv3d: weight packs {cin8 * 8} input channels, c_in={c_in}")
+    n_taps, cin_pl, c_out_pad, w_lanes = w_packed.shape
+    _need(w_packed.is_cuda and _LANES.get(w_packed.dtype) == lanes and w_packed.is_contiguous() and w_lanes == lanes,
+          "conv3d: w_packed must be a contiguous CUDA bf16 [taps, Cin/8, Cout_pad, 8] tensor (fp32 [taps, Cin/4, Cout_pad, 4] "
+          "with an fp32 x)")
+    c_in = cin_pl * lanes if c_in is None else c_in
+    _need(c_in == cin_pl * lanes, f"conv3d: weight packs {cin_pl * lanes} input channels, c_in={c_in}")
     _need(n_taps == len(taps), f"conv3d: weight has {n_taps} taps, {len(taps)} offsets given")
     desc = _C.ConvDesc()
     desc.batch, desc.depth, desc.height, desc.width = b, d, h, w_
@@ -263,12 +307,12 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
         if out_fp32:
             out = torch.empty((b, c_out, d, h, w_), dtype=torch.float32, device=x.device)
         else:
-            out = torch.empty((b, c_out // 8, d, h, w_, 8), dtype=torch.bfloat16, device=x.device)
+            out = torch.empty((b, c_out // lanes, d, h, w_, lanes), dtype=x.dtype, device=x.device)
     if out_fp32:
         _need(out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (b, c_out, d, h, w_),
               "conv3d: fp32 output must be contiguous (B, c_out, D, H, W)")
     else:
-        _planar_ok(out, "conv3d out")
+        _same_lanes(lanes, out, "conv3d out")
         _need(tuple(out.shape[2:5]) == (d, h, w_) and out.shape[0] == b, "conv3d: out grid mismatch")
         desc.y_planes, desc.y_plane0 = out.shape[1], out_plane0
     epi = _C.ConvEpilogue()
@@ -281,7 +325,7 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
             _need(step_ptr.is_cuda and step_ptr.dtype == torch.int32, "conv3d: step_ptr must be a CUDA int32 tensor")
             epi.step_ptr = step_ptr.data_ptr()
     if residual is not None:
-        _planar_ok(residual, "conv3d residual")
+        _same_lanes(lanes, residual, "conv3d residual")
         r_grid = (d // 2, h // 2, w_ // 2) if residual_upsample else (d, h, w_)
         _need(tuple(residual.shape[2:5]) == r_grid and residual.shape[0] == b, "conv3d: residual grid mismatch")
         epi.residual = residual.data_ptr()
@@ -291,7 +335,7 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
             _need(c_out % 8 == 0 and residual.shape[1] >= residual_plane0 + c_out, "conv3d: a depth-to-space residual holds 8 x c_out channels")
         desc.r_planes, desc.r_plane0 = residual.shape[1], residual_plane0
     if skip_x is not None:
-        _planar_ok(skip_x, "conv3d skip_x")
+        _same_lanes(lanes, skip_x, "conv3d skip_x")
         _need(tuple(skip_x.shape[2:5]) == (d, h, w_) and skip_x.shape[0] == b, "conv3d: skip_x grid mismatch")
         _need(skip_w is not None and skip_w.is_cuda and skip_w.dtype == torch.bfloat16 and skip_w.is_contiguous() and
               skip_w.dim() == 4 and skip_w.shape[0] == 1 and skip_w.shape[2] == c_out_pad,
@@ -312,17 +356,17 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
     if prof is not None:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-    rc = _C.lib().vdm_conv3d(ctypes.byref(desc), x.data_ptr(), w_packed.data_ptr(), out.data_ptr(), ctypes.byref(epi),
-                             _stream())
-    if rc == _C.E_UNSUPPORTED and (skip_x is not None or in_norm is not None):
+    fn = _C.lib().vdm_conv3d_tf32 if tf32 else _C.lib().vdm_conv3d
+    rc = fn(ctypes.byref(desc), x.data_ptr(), w_packed.data_ptr(), out.data_ptr(), ctypes.byref(epi), _stream())
+    if rc == _C.E_UNSUPPORTED and (skip_x is not None or in_norm is not None or (tf32 and residual_upsample)):
         raise _C.UnsupportedFusion(_C.lib().vdm_last_error_string().decode("utf-8", "replace"))
-    _C.check(rc, "vdm_conv3d")
+    _C.check(rc, "vdm_conv3d_tf32" if tf32 else "vdm_conv3d")
     _launched(1)
     if prof is not None:
         e1.record()
         # algorithmic FLOPs: real (un-padded) output channels, the channels the caller says it reads
         prof.append((e0, e1, 2.0 * n_taps * c_in * c_out * b * d * h * w_,
-                     f"{_PROFILE_TAG}{c_in}->{c_out} taps={n_taps} grid={d}x{h}x{w_} B={b}"))
+                     f"{_PROFILE_TAG}{'tf32 ' if tf32 else ''}{c_in}->{c_out} taps={n_taps} grid={d}x{h}x{w_} B={b}"))
     return out
 
 
@@ -402,8 +446,9 @@ def channel_stats(x: torch.Tensor, channels: int, x_plane0: int = 0, stats: Opti
 def gn_silu(x: torch.Tensor, channels: int, groups: int, stats: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor,
             eps: float = 1e-5, *, x_plane0: int = 0, out: Optional[torch.Tensor] = None, out_plane0: int = 0,
             dropout_p: float = 0.0, seed: int = 0, layer_tag: int = 0, seed_step: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """y = dropout(silu(groupnorm(x))).  ``seed_step`` (device int32) is added to ``seed`` on the device."""
-    _planar_ok(x, "gn_silu x")
+    """y = dropout(silu(groupnorm(x))).  ``seed_step`` (device int32) is added to ``seed`` on the device.
+    fp32 planar tensors (TF32 mode): ``vdm_gn_silu_f32``, no dropout."""
+    lanes = _planar_lanes(x, "gn_silu x")
     b = x.shape[0]
     voxels = x.shape[2] * x.shape[3] * x.shape[4]
     _need(stats.dtype == torch.float64 and tuple(stats.shape) == (b, channels, 2) and stats.is_contiguous(),
@@ -411,9 +456,16 @@ def gn_silu(x: torch.Tensor, channels: int, groups: int, stats: torch.Tensor, ga
     _need(gamma.dtype == torch.float32 and beta.dtype == torch.float32 and gamma.numel() == channels and
           beta.numel() == channels and gamma.is_cuda and beta.is_cuda, "gn_silu: gamma/beta must be CUDA fp32 [channels]")
     if out is None:
-        out = torch.empty((b, channels // 8) + tuple(x.shape[2:]), dtype=torch.bfloat16, device=x.device)
-    _planar_ok(out, "gn_silu out")
+        out = torch.empty((b, channels // lanes) + tuple(x.shape[2:5]) + (lanes,), dtype=x.dtype, device=x.device)
+    _same_lanes(lanes, out, "gn_silu out")
     vx, vy = _view(x, x_plane0), _view(out, out_plane0)
+    if lanes == 4:
+        _need(dropout_p == 0.0, "gn_silu: the fp32 (TF32 inference) form has no dropout")
+        rc = _C.lib().vdm_gn_silu_f32(ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
+                                      gamma.data_ptr(), beta.data_ptr(), eps, _stream())
+        _C.check(rc, "vdm_gn_silu_f32")
+        _launched(1)
+        return out
     rc = _C.lib().vdm_gn_silu_step(ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
                                    gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag,
                                    _stream())
@@ -473,51 +525,57 @@ def gn_silu_view(x: torch.Tensor, channels: int, c_off: int, channels_total: int
 
 def avgpool2(x: torch.Tensor, channels: int, *, x_plane0: int = 0, out: Optional[torch.Tensor] = None,
              out_plane0: int = 0, stats: Optional[torch.Tensor] = None, stats_c0: int = 0) -> torch.Tensor:
-    _planar_ok(x, "avgpool2 x")
+    lanes = _planar_lanes(x, "avgpool2 x")
     b, _, d, h, w, _ = x.shape
     if out is None:
-        out = torch.empty((b, channels // 8, d // 2, h // 2, w // 2, 8), dtype=torch.bfloat16, device=x.device)
-    _planar_ok(out, "avgpool2 out")
+        out = torch.empty((b, channels // lanes, d // 2, h // 2, w // 2, lanes), dtype=x.dtype, device=x.device)
+    _same_lanes(lanes, out, "avgpool2 out")
     vx, vy = _view(x, x_plane0), _view(out, out_plane0)
-    rc = _C.lib().vdm_avgpool2(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats),
-                               0 if stats is None else stats.shape[1], stats_c0, _stream())
-    _C.check(rc, "vdm_avgpool2")
+    fn = _C.lib().vdm_avgpool2_f32 if lanes == 4 else _C.lib().vdm_avgpool2
+    rc = fn(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats), 0 if stats is None else stats.shape[1],
+            stats_c0, _stream())
+    _C.check(rc, "vdm_avgpool2_f32" if lanes == 4 else "vdm_avgpool2")
     _launched(1)
     return out
 
 
 def upsample2(coarse: torch.Tensor, channels: int, out: torch.Tensor, *, coarse_plane0: int = 0, out_plane0: int = 0,
               stats: Optional[torch.Tensor] = None, stats_c0: int = 0) -> torch.Tensor:
-    _planar_ok(coarse, "upsample2 coarse")
-    _planar_ok(out, "upsample2 out")
+    lanes = _planar_lanes(coarse, "upsample2 coarse")
+    _same_lanes(lanes, out, "upsample2 out")
     b, _, d, h, w, _ = out.shape
     _need(tuple(coarse.shape[2:5]) == (d // 2, h // 2, w // 2), "upsample2: coarse grid must be half the fine grid")
     vx, vy = _view(coarse, coarse_plane0), _view(out, out_plane0)
-    rc = _C.lib().vdm_upsample2(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats),
-                                0 if stats is None else stats.shape[1], stats_c0, _stream())
-    _C.check(rc, "vdm_upsample2")
+    fn = _C.lib().vdm_upsample2_f32 if lanes == 4 else _C.lib().vdm_upsample2
+    rc = fn(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats), 0 if stats is None else stats.shape[1],
+            stats_c0, _stream())
+    _C.check(rc, "vdm_upsample2_f32" if lanes == 4 else "vdm_upsample2")
     _launched(1)
     return out
 
 
 def pad_circular(x: torch.Tensor, channels: int, *, x_plane0: int = 0, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """``vdm_pad_circular``: planar [B, P, D, H, W, 8] -> [B, channels/8, D+2, H+2, W+2, 8] with a periodic one-voxel halo."""
-    _planar_ok(x, "pad_circular x")
+    """``vdm_pad_circular``: planar [B, P, D, H, W, L] -> [B, channels/L, D+2, H+2, W+2, L] with a periodic one-voxel halo
+    (L = 8 bf16 or 4 fp32 channels per plane; the kernel copies 16-byte units)."""
+    lanes = _planar_lanes(x, "pad_circular x")
     b, _, d, h, w, _ = x.shape
     if out is None:
-        out = torch.empty((b, channels // 8, d + 2, h + 2, w + 2, 8), dtype=torch.bfloat16, device=x.device)
-    _planar_ok(out, "pad_circular out")
+        out = torch.empty((b, channels // lanes, d + 2, h + 2, w + 2, lanes), dtype=x.dtype, device=x.device)
+    _same_lanes(lanes, out, "pad_circular out")
     _need(tuple(out.shape[2:5]) == (d + 2, h + 2, w + 2) and out.shape[0] == b, "pad_circular: out must have the padded grid")
+    _need(channels % lanes == 0, f"pad_circular: channels={channels} is not a whole number of planes")
     vx, vy = _view(x, x_plane0), _view(out, 0)
-    rc = _C.lib().vdm_pad_circular(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _stream())
+    # the C entry point counts 8 channels per 16-byte plane
+    rc = _C.lib().vdm_pad_circular(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels * 8 // lanes, _stream())
     _C.check(rc, "vdm_pad_circular")
     _launched(1)
     return out
 
 
 def pack_input(z: torch.Tensor, cond: Optional[torch.Tensor], c_pad: int = 16,
-               out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """z: fp32 (B, 1, D, H, W) or (B, D, H, W); cond: fp32 (B, n_cond, D, H, W) -> planar [B, c_pad/8, D, H, W, 8]."""
+               out: Optional[torch.Tensor] = None, dtype: torch.dtype = torch.bfloat16) -> torch.Tensor:
+    """z: fp32 (B, 1, D, H, W) or (B, D, H, W); cond: fp32 (B, n_cond, D, H, W) -> planar [B, c_pad/8, D, H, W, 8], or
+    fp32 planar [B, c_pad/4, D, H, W, 4] when ``out`` (or, without ``out``, ``dtype``) is fp32."""
     _need(z.is_cuda and z.dtype == torch.float32 and z.is_contiguous(), "pack_input: z must be contiguous CUDA fp32")
     if z.dim() == 5:
         _need(z.shape[1] == 1, "pack_input: z must have one channel")
@@ -530,11 +588,13 @@ def pack_input(z: torch.Tensor, cond: Optional[torch.Tensor], c_pad: int = 16,
               tuple(cond.shape[2:]) == (d, h, w) and cond.shape[0] == b, "pack_input: cond must be fp32 (B, n, D, H, W)")
         n_cond = cond.shape[1]
     if out is None:
-        out = torch.empty((b, c_pad // 8, d, h, w, 8), dtype=torch.bfloat16, device=z.device)
-    _planar_ok(out, "pack_input out")
+        lanes = _LANES[dtype]
+        out = torch.empty((b, c_pad // lanes, d, h, w, lanes), dtype=dtype, device=z.device)
+    lanes = _planar_lanes(out, "pack_input out")
     vo = _view(out, 0)
-    rc = _C.lib().vdm_pack_input(z.data_ptr(), _ptr(cond), ctypes.byref(vo), b, d * h * w, n_cond, c_pad, _stream())
-    _C.check(rc, "vdm_pack_input")
+    fn = _C.lib().vdm_pack_input_f32 if lanes == 4 else _C.lib().vdm_pack_input
+    rc = fn(z.data_ptr(), _ptr(cond), ctypes.byref(vo), b, d * h * w, n_cond, c_pad, _stream())
+    _C.check(rc, "vdm_pack_input_f32" if lanes == 4 else "vdm_pack_input")
     _launched(1)
     return out
 

@@ -232,7 +232,8 @@ class VDM(nn.Module):
     def session(self, batch_size, n_sampling_steps, device, **kw) -> "SamplerSession":
         """A (cached) ``SamplerSession`` for this batch size / step count, reset to a new chain."""
         key = (batch_size, n_sampling_steps, str(device), kw.get("s_conditioning") is not None,
-               0 if kw.get("v_conditionings") is None else len(kw["v_conditionings"]))
+               0 if kw.get("v_conditionings") is None else len(kw["v_conditionings"]),
+               getattr(self.score_model, "precision", "bf16"))
         cache = self.__dict__.setdefault("_sessions", {})
         sess = cache.get(key)
         if sess is None:
@@ -306,7 +307,12 @@ class SamplerSession:
         self.eps = torch.empty(self.shape, dtype=torch.float32, device=dev)
         self.noise_buf = torch.empty(self.shape, dtype=torch.float32, device=dev)
         self.cond_buf = None
-        self.packed = torch.empty((batch_size, 2) + tuple(self.net.shape[1:]) + (8,), dtype=torch.bfloat16, device=dev)
+        # packed network input in the net's precision (bf16 [B, 2, D, H, W, 8] or, TF32, fp32 [B, 2, D, H, W, 4])
+        self.tf32 = getattr(self.net, "precision", "bf16") == "tf32"
+        self.c_pad = self.net.input_channels_pad()
+        lanes = 4 if self.tf32 else 8
+        self.packed = torch.empty((batch_size, self.c_pad // lanes) + tuple(self.net.shape[1:]) + (lanes,),
+                                  dtype=torch.float32 if self.tf32 else torch.bfloat16, device=dev)
         self.step_idx = torch.zeros(1, dtype=torch.int32, device=dev)
         self.rid_buf = torch.zeros(batch_size, dtype=torch.int32, device=dev)
         self.steps = torch.linspace(1.0, 0.0, n_sampling_steps + 1, device=dev)
@@ -354,7 +360,7 @@ class SamplerSession:
                 self.cond_buf.copy_(c)
         elif self.cond_buf is not None:
             raise ValueError("a session created with spatial conditioning must be reset with one")
-        ops.pack_input(self.z, self.cond_buf, 16, out=self.packed)
+        ops.pack_input(self.z, self.cond_buf, self.c_pad, out=self.packed)
         self.step_idx.zero_()
         self.done = 0
         # the graph bakes in pointers and the (seed, injected-noise or Philox) choice, nothing else
@@ -373,10 +379,13 @@ class SamplerSession:
         self.kernels_per_step = ops.launch_count() - n0
 
     def _update(self):
+        # (TF32: the fused update writes bf16 input planes only, so the fp32 input is re-packed by its own launch)
         ops.sampler_step(self.z, self.eps, self.coef, out=self.z, step_ptr=self.step_idx, seed=self.seed,
                          realisation_id=self.rid_buf, draw_base=1,
                          noise=self.noise_buf if self.noise_fn is not None else None, cond=self.cond_buf,
-                         packed_out=self.packed)
+                         packed_out=None if self.tf32 else self.packed)
+        if self.tf32:
+            ops.pack_input(self.z, self.cond_buf, self.c_pad, out=self.packed)
         ops.increment(self.step_idx)
 
     @torch.no_grad()
