@@ -132,7 +132,7 @@ def test_batched_pack_equals_the_single_filter_launches():
     from vdm4cdm_b200.networks import CUNet
     net = CUNet(shape=(1, 16, 16, 16), chs=[16, 32], s_conditioning_channels=1, v_conditioning_dims=[], t_conditioning=True).to(dev)
     net.refresh_packed()
-    before = {slot: hit[1].clone() for slot, hit in net._packed_cache.items()}
+    before = {slot: f.buf.clone() for slot, f in net._packed_cache.items()}
     with torch.no_grad():
         for p_ in net.parameters():
             p_.mul_(1.5)
@@ -142,8 +142,8 @@ def test_batched_pack_equals_the_single_filter_launches():
     assert ops.launch_count() - launches0 == 1
     torch.cuda.synchronize()
     for name, conv in net._convs():
-        assert torch.equal(net._packed_cache[name][1], ops.pack_conv_weight(conv.weight.detach()))
-        assert not torch.equal(net._packed_cache[name][1], before[name])
+        assert torch.equal(net._packed_cache[name].buf, ops.pack_conv_weight(conv.weight.detach()))
+        assert not torch.equal(net._packed_cache[name].buf, before[name])
 
 
 def test_dgrad_wide_input_in_two_launches():

@@ -231,6 +231,29 @@ def test_sampler_chain_matches_oracle_per_step_and_graph_equals_eager():
     assert _rel_l2(x_folded, full) < 5 * BF16_RTOL
 
 
+def test_graph_replay_after_new_weights_matches_a_fresh_model():
+    """A captured sampler graph reads the packed filters without packing lazily, so ``SamplerSession.reset`` must
+    re-pack every slot (the up blocks' polyphase and input-channel-slice filters too): after ``load_state_dict`` a
+    replayed chain with the same seed and noise equals a fresh VDM with the new weights."""
+    from vdm4cdm_b200.vdm_model import VDM
+    shape, chs, batch, n_steps = (1, 16, 16, 16), (16, 32), 2, 4
+    _, net = _models(shape, chs)
+    _, net_new = _models(shape, chs, seed=1)
+    vdm, vdm_new = VDM(net).cuda().eval(), VDM(net_new).cuda().eval()
+    g = torch.Generator().manual_seed(3)
+    noises = [torch.randn((batch,) + shape, generator=g).cuda() for _ in range(n_steps + 1)]
+    kw = dict(seed=0, noise_fn=lambda d, s: noises[d], s_conditioning=torch.randn((batch,) + shape, generator=g).cuda(),
+              v_conditionings=[torch.rand(batch, 6, generator=g).cuda()])
+    vdm.use_cuda_graph = vdm_new.use_cuda_graph = True
+    old = vdm.sample(batch, n_steps, "cuda:0", **kw).cpu()          # eager first step, then the graph is captured
+    assert vdm._sessions and next(iter(vdm._sessions.values())).graph is not None
+    vdm.load_state_dict(vdm_new.state_dict())
+    got = vdm.sample(batch, n_steps, "cuda:0", **kw).cpu()          # replays the graph captured above
+    want = vdm_new.sample(batch, n_steps, "cuda:0", **kw).cpu()
+    assert _rel_l2(old, want) > 1e-2                                # the weights differ enough to tell
+    assert _rel_l2(got, want) < 1e-3, _rel_l2(got, want)
+
+
 def test_philox_sampling_is_batch_independent():
     from vdm4cdm_b200.vdm_model import VDM
     shape, chs = (1, 16, 16, 16), (16, 32)

@@ -238,7 +238,7 @@ class _UNetFn(torch.autograd.Function):
         packed = ops.pack_input(x.detach().contiguous().float(), cond, 16,
                                 out=ar.get(f"packed.{b}", (b, 2) + tuple(net.shape[1:]) + (8,), torch.bfloat16, x.device))
         tape: dict = {}
-        net.refresh_packed()
+        net.refresh_packed(training=True)
         out = net.run_packed(packed, rows, training_dropout=net.training and net.dropout_prob > 0.0, tape=tape)
         ctx.net, ctx.tape, ctx.row_names, ctx.param_names = net, tape, row_names, param_names
         ctx.need_dx = x.requires_grad

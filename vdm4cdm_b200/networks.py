@@ -21,7 +21,6 @@ fallback for the convolutional path; autograd support lives in ``vdm4cdm_b200.au
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional, Sequence
 
 import torch
@@ -94,6 +93,76 @@ class _Arena:
         return t
 
 
+class _PackedFilter:
+    """A slot of ``CUNet._packed_cache``: ``buf``, a kernel-layout copy of (part of) ``conv.weight``; the ``key`` of the
+    weights it was packed from; the recipe that packs it again.  ``buf`` is allocated once and re-packed in place, so
+    captured CUDA graphs keep a valid pointer.  Recipes, ``kind`` (``args``):
+      "bf16" (transpose_flip, c0, n): the forward filter, or the dgrad filter of input channels [c0, c0 + n);
+      "f32" (): the fp32 forward filter of ``vdm_conv3d_tf32`` (own slots: switching precision does not re-pack);
+      "slice" (c0, n): the bf16 forward filter of input channels [c0, c0 + n) (halves of an up block's convs);
+      "poly" (c_up, group, n_par): the bf16 polyphase parity group of the first ``c_up`` input channels
+          (``ops.polyphase_group``) and its ``taps``; the effective taps are summed in fp32 and rounded to bf16 once."""
+
+    def __init__(self, conv: nn.Conv3d, kind: str, args: tuple):
+        self.conv, self.kind, self.args = conv, kind, args
+        self.key = self.buf = self.taps = None
+
+    def weights_key(self, epoch: int) -> tuple:
+        w = self.conv.weight
+        return (w.data_ptr(), w._version, w.device, epoch)
+
+    @torch.no_grad()
+    def refresh(self, epoch: int) -> "_PackedFilter":
+        """Re-pack ``buf`` if the weights changed since it was packed (``epoch``: ``CUNet.invalidate_packed`` count)."""
+        key = self.weights_key(epoch)
+        if key == self.key:
+            return self
+        w = self.conv.weight.detach()
+        if self.kind == "poly":
+            c_up, group, n_par = self.args
+            part, self.taps = ops.polyphase_group(w[:, :c_up], group, n_par)
+            packed = ops.pack_conv_weight(part)
+            if self._fits(packed.shape, w.device):
+                self.buf.copy_(packed)
+            else:
+                self.buf = packed
+        else:
+            if self.kind == "slice":
+                w = w[:, self.args[0]:self.args[0] + self.args[1]]
+            transpose_flip, c0, n = self.args if self.kind == "bf16" else (False, 0, None)
+            dtype = torch.float32 if self.kind == "f32" else torch.bfloat16
+            shape = ops.packed_weight_shape(w.shape, transpose_flip, n, dtype=dtype)
+            if not self._fits(shape, w.device):
+                self.buf = torch.empty(shape, dtype=dtype, device=w.device)
+            ops.pack_conv_weight_into(w.contiguous(), self.buf, transpose_flip, c0, n)
+        self.key = key
+        return self
+
+    def _fits(self, shape, device) -> bool:
+        return self.buf is not None and tuple(self.buf.shape) == tuple(shape) and self.buf.device == device
+
+
+class _Forms:
+    """The fused forms one ``CUNet.run_packed`` call may use: bf16 inference only (training keeps every intermediate
+    for the backward pass; TF32 runs the unfused path).  The ``CUNet`` switches turn them off one by one."""
+
+    def __init__(self, net: "CUNet", tape: Optional[dict], training_dropout: bool):
+        fused = tape is None and net.precision == "bf16"
+        # GroupNorm + SiLU applied by the consumer conv to its input tiles (ops.conv3d in_norm): no dropout, zero padding
+        self.gn = fused and net.fuse_gn and not training_dropout and not net.circular
+        self.gn_min_channels = net.fuse_gn_min_channels
+        # up blocks read the coarse tensor (see CUNet._run_block); only then is their skip conv tried fused into net2's
+        self.read_coarse = fused and net.fuse_upsample
+        self.polyphase = self.read_coarse and net.polyphase_up and not net.circular
+
+    def gn_in_conv(self, c_in: int, c_out: int) -> bool:
+        """Whether a ``c_in`` -> ``c_out`` conv normalises its own input: layers of at least ``fuse_gn_min_channels``
+        outputs (tile kernel, four warps share every halo stage) and the narrow layers of the marching schedule (at most
+        32 channels in and out; R4k, 128^3 x 8: 12.40 -> 11.81 ms per step).  In between (the kd-folded TILE schedule) the
+        transform's LDS / STS traffic costs more than the HBM pass it replaces (profiles/R2h_transform_ablation.txt)."""
+        return self.gn and (c_out >= self.gn_min_channels or (c_in <= 32 and c_out <= 32))
+
+
 class CUNet(nn.Module):
     def __init__(self, shape=(1, 128, 128, 128), chs=(32, 64, 128, 256), s_conditioning_channels: int = 0,
                  v_conditioning_dims: Sequence[int] = (), t_conditioning: bool = False, norm_groups: int = 8,
@@ -127,13 +196,9 @@ class CUNet(nn.Module):
         self.circular = conv_padding_mode == "circular"     # the cropsize == 256 models (src/utils.py:460)
         self.fuse_upsample = True       # inference: up blocks read the coarse tensor instead of its up-sampled copy
         # inference: GroupNorm + SiLU in front of a conv is applied by the conv kernel to its input tile (ops.conv3d
-        # in_norm) instead of by a separate read + write pass over the tensor
+        # in_norm) instead of by a separate read + write pass over the tensor, for the layers _Forms.gn_in_conv picks
         self.fuse_gn = True
         self.fuse_gn_min_channels = 64
-        # ... and for the narrow layers that run the d-marching schedule (at most 32 channels in and out), where warps 12..15
-        # transform whole input slices (R4k, 128^3 x 8: 12.40 -> 11.81 ms per step; the convs get 0.2 ms slower each, the
-        # 0.34 ms GroupNorm passes go).  VDM4CDM_FUSE_GN_NARROW=0 switches it off (A/B measurements).
-        self.fuse_gn_narrow = os.environ.get("VDM4CDM_FUSE_GN_NARROW", "1") != "0"
         # inference, up blocks: conv3x3x3 over the up-sampled half of cat([interpolate(h), skip]) in its polyphase form --
         # eight 2x2x2-tap convolutions of the COARSE tensor, one per output parity (8/27 of the multiply-adds, the
         # up-sampled activations are never written); the skip half is a plain conv that adds them as its residual
@@ -176,9 +241,9 @@ class CUNet(nn.Module):
                                       nn.Conv3d(c[0], 1, 3, padding=1, padding_mode=pm))
         self._arena = _Arena()
         self._train_arena = _Arena()
-        self._packed_cache: Dict[str, tuple] = {}
-        self._pack_meta: Dict[str, tuple] = {}        # slot -> (conv, transpose_flip, c0, n) of the filters repack_all handles
+        self._packed_cache: Dict[str, _PackedFilter] = {}
         self._pack_tables: Dict[tuple, torch.Tensor] = {}
+        self._weights_epoch = 0
         self.dropout_seed = 0
         self._dropout_calls = 0
         # device-side training-step counter added to the dropout seed (a captured CUDA graph draws new masks)
@@ -227,116 +292,61 @@ class CUNet(nn.Module):
             out.append(emb(v.to(torch.float32)))
         return out if len(out) else None
 
-    # ---- packed weights (bf16, kernel layout), rebuilt when the fp32 parameter changes ------------
+    # ---- packed weights (kernel layout), re-packed in place when the fp32 parameter changes ------------
     def invalidate_packed(self) -> None:
-        """Tell the bf16 weight caches that the fp32 parameters changed behind torch's back (the fused
+        """Tell the weight caches that the fp32 parameters changed behind torch's back (the fused
         optimizer kernel writes through raw pointers, which does not bump ``Tensor._version``)."""
-        self._weights_epoch = getattr(self, "_weights_epoch", 0) + 1
+        self._weights_epoch += 1
+
+    def _slot(self, slot: str, conv: nn.Conv3d, kind: str, *args) -> _PackedFilter:
+        """Cache slot ``slot`` (recipe ``kind``, ``args`` of ``_PackedFilter``), packed on first use, up to date."""
+        f = self._packed_cache.get(slot)
+        if f is None:
+            f = self._packed_cache[slot] = _PackedFilter(conv, kind, args)
+        return f.refresh(self._weights_epoch)
 
     def _packed(self, name: str, conv: nn.Conv3d) -> torch.Tensor:
-        """bf16 kernel-layout copy of ``conv.weight`` (one ``vdm_pack_conv_weight`` launch when the parameter changed;
-        the buffer is allocated once, so captured CUDA graphs keep a valid pointer).  In TF32 mode the fp32 filter of
-        ``vdm_conv3d_tf32``, kept in its own slot so that switching precision does not re-pack."""
+        """Forward filter of ``conv`` in the trunk's precision: bf16, or in TF32 mode the fp32 filter of ``vdm_conv3d_tf32``."""
         if self.precision == "tf32":
-            return self._packed_f32(name, conv)
-        return self._packed_any(name, conv, False, 0, conv.in_channels)
-
-    def _packed_f32(self, name: str, conv: nn.Conv3d) -> torch.Tensor:
-        w = conv.weight
-        key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
-        slot = name + ".f32"
-        hit = self._packed_cache.get(slot)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                shape = ops.packed_weight_shape(w.shape, dtype=torch.float32)
-                buf = hit[1] if hit is not None and tuple(hit[1].shape) == shape and hit[1].device == w.device else \
-                    torch.empty(shape, dtype=torch.float32, device=w.device)
-                ops.pack_conv_weight_into(w.detach().contiguous(), buf)
-                hit = (key, buf)
-            self._packed_cache[slot] = hit
-        return hit[1]
+            return self._slot(name + ".f32", conv, "f32").buf
+        return self._slot(name, conv, "bf16", False, 0, conv.in_channels).buf
 
     def _packed_dgrad(self, name: str, conv: nn.Conv3d, c0: int, n: int) -> torch.Tensor:
         """bf16 dgrad filter (roles of Cin/Cout exchanged, taps mirrored) for input channels [c0, c0+n)."""
-        return self._packed_any(f"{name}.dgrad.{c0}.{n}", conv, True, c0, n)
-
-    def _packed_any(self, slot: str, conv: nn.Conv3d, transpose_flip: bool, c0: int, n: int) -> torch.Tensor:
-        w = conv.weight
-        key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
-        hit = self._packed_cache.get(slot)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                shape = ops.packed_weight_shape(w.shape, transpose_flip, n)
-                buf = hit[1] if hit is not None and tuple(hit[1].shape) == shape and hit[1].device == w.device else \
-                    torch.empty(shape, dtype=torch.bfloat16, device=w.device)
-                ops.pack_conv_weight_into(w.detach().contiguous(), buf, transpose_flip, c0, n)
-                hit = (key, buf)
-            self._packed_cache[slot] = hit
-            self._pack_meta[slot] = (conv, transpose_flip, c0, n)
-        return hit[1]
+        return self._slot(f"{name}.dgrad.{c0}.{n}", conv, "bf16", True, c0, n).buf
 
     def repack_all(self) -> None:
-        """Re-pack EVERY stale filter the trunk has used so far (forward and dgrad variants) in one
-        ``vdm_pack_conv_weight_batched`` launch -- the training step calls this after each optimizer update instead of
-        letting ~56 lazy single-filter launches happen.  Filters seen for the first time are still packed lazily."""
-        stale = []
-        for slot, (conv, transpose_flip, c0, n) in self._pack_meta.items():
-            w = conv.weight
-            key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
-            hit = self._packed_cache.get(slot)
-            if hit is None or not w.is_cuda or not w.is_contiguous() or hit[1].device != w.device:
-                continue
-            if hit[0] != key:
-                stale.append((slot, key, w, hit[1], transpose_flip, c0, n))
+        """Re-pack every stale whole-weight bf16 filter the trunk has used so far (forward and dgrad variants) in one
+        ``vdm_pack_conv_weight_batched`` launch -- the training step does this after each optimizer update instead of
+        letting ~56 lazy single-filter launches happen."""
+        e = self._weights_epoch
+        stale = [(slot, f) for slot, f in self._packed_cache.items() if f.kind == "bf16" and f.conv.weight.is_cuda and
+                 f.conv.weight.is_contiguous() and f.buf.device == f.conv.weight.device and f.key != f.weights_key(e)]
         if not stale:
             return
-        tkey = tuple((slot, key[0], buf.data_ptr()) for slot, key, _, buf, _, _, _ in stale)
+        tkey = tuple((slot, f.conv.weight.data_ptr(), f.buf.data_ptr()) for slot, f in stale)
         table = self._pack_tables.get(tkey)
         if table is None:
             self._pack_tables.clear()
-            table = ops.pack_job_table([(w.detach(), buf, tf, c0, n) for _, _, w, buf, tf, c0, n in stale], stale[0][2].device)
+            table = ops.pack_job_table([(f.conv.weight.detach(), f.buf, *f.args) for _, f in stale], stale[0][1].buf.device)
             self._pack_tables[tkey] = table
         with torch.no_grad():
             ops.pack_conv_weights_batched(table, len(stale))
-        for slot, key, _, buf, _, _, _ in stale:
-            self._packed_cache[slot] = (key, buf)
+        for _, f in stale:
+            f.key = f.weights_key(e)
 
-    def _packed_in_slice(self, slot: str, conv: nn.Conv3d, c0: int, n: int) -> torch.Tensor:
-        """bf16 filter of the conv restricted to INPUT channels [c0, c0 + n) (the two halves of an up block's 1x1x1
-        skip conv over the concatenation, see ``_run_block``)."""
-        w = conv.weight
-        key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
-        hit = self._packed_cache.get(slot)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                part = w.detach()[:, c0:c0 + n].contiguous()
-                shape = ops.packed_weight_shape(part.shape)
-                buf = hit[1] if hit is not None and tuple(hit[1].shape) == shape and hit[1].device == w.device else \
-                    torch.empty(shape, dtype=torch.bfloat16, device=w.device)
-                ops.pack_conv_weight_into(part, buf)
-                hit = (key, buf)
-            self._packed_cache[slot] = hit
-        return hit[1]
-
-    def _packed_poly(self, slot: str, conv: nn.Conv3d, c_up: int, group: int, n_par: int):
-        """(bf16 packed filter, taps) of the polyphase parity group ``group`` (``ops.polyphase_group``: ``n_par`` output
-        parities stacked along N) for the first ``c_up`` (up-sampled) input channels of a 3x3x3 conv; the effective taps
-        are sums of the original ones, formed in fp32 and rounded to bf16 once.  Re-packed in place when the parameter
-        changes (captured CUDA graphs keep the pointer)."""
-        w = conv.weight
-        key = (w.data_ptr(), w._version, w.device, getattr(self, "_weights_epoch", 0))
-        slot = f"{slot}.poly.{n_par}.{group}"
-        hit = self._packed_cache.get(slot)
-        if hit is None or hit[0] != key:
-            with torch.no_grad():
-                part, taps = ops.polyphase_group(w.detach()[:, :c_up], group, n_par)
-                packed = ops.pack_conv_weight(part)
-                if hit is not None and tuple(hit[1].shape) == tuple(packed.shape) and hit[1].device == w.device:
-                    hit[1].copy_(packed)
-                    packed = hit[1]
-                hit = (key, packed, taps)
-            self._packed_cache[slot] = hit
-        return hit[1], hit[2]
+    def refresh_packed(self, training: bool = False) -> None:
+        """Re-pack (in place) every cached filter whose fp32 parameter changed since it was packed, and pack the trunk's
+        forward filters in the current precision if missing: the whole-weight bf16 filters in one batched launch
+        (``repack_all``), every other slot by its own recipe.  A captured sampler graph reads the slots without packing
+        lazily, so ``SamplerSession.reset`` calls this.  ``training=True`` (every training forward) skips the slots that
+        only inference reads (fp32, slices, polyphase groups): they are re-packed when next used."""
+        self.repack_all()
+        for name, conv in self._convs():
+            self._packed(name, conv)
+        if not training:
+            for f in self._packed_cache.values():
+                f.refresh(self._weights_epoch)
 
     def trunk_parameters(self):
         """(name, parameter) of everything the convolutional trunk differentiates itself: conv filters and
@@ -360,13 +370,6 @@ class CUNet(nn.Module):
             if blk.skip_conv is not None:
                 out.append((name + ".skip", blk.skip_conv))
         return out
-
-    def refresh_packed(self) -> None:
-        """Re-pack (in place) every conv filter whose fp32 parameter changed since it was packed: one batched launch for
-        the filters packed before (``repack_all``), single launches for new ones."""
-        self.repack_all()
-        for name, conv in self._convs():
-            self._packed(name, conv)
 
     def conv_flops_per_sample(self) -> float:
         """Algorithmic conv FLOPs of one forward for one sample: sum of 2 k^3 Cin Cout D H W over the
@@ -413,8 +416,8 @@ class CUNet(nn.Module):
         return rows
 
     # ---- the convolutional trunk on channel-planar buffers --------------------------------------
-    def _run_block(self, name, blk: ResNetBlock, x, x_plane0, x_stats, rows, step_ptr, out, out_plane0, out_stats,
-                   out_stats_c0, grid, training_dropout, tape=None, up_from=None):
+    def _run_block(self, name, blk: ResNetBlock, forms: _Forms, x, x_plane0, x_stats, rows, step_ptr, out, out_plane0,
+                   out_stats, out_stats_c0, grid, training_dropout, tape=None, up_from=None):
         """out[window] = block(x[window]).  x_stats: double [B, ch_in, 2] of x.  With a ``tape`` (training)
         every intermediate gets its own buffer and is recorded for the backward pass.
 
@@ -433,25 +436,17 @@ class CUNet(nn.Module):
         n1 = blk.net1[0]
         voxels = grid[0] * grid[1] * grid[2]
         p_drop = blk.dropout_prob if training_dropout else 0.0
-        # inference without dropout and with zero padding: the convs normalise their own input tiles (fuse_gn) -- for layers
-        # of at least 64 output channels (tile kernel, four warps share every halo stage) and for the narrow layers of the
-        # marching schedule (four warps take whole slices in turn).  In between (narrow output, more than 32 input channels:
-        # the kd-folded TILE schedule) the transform's LDS / STS traffic costs more than the HBM pass it replaces
-        # (+0.55 ms on a 0.85 ms conv even as a plain copy, profiles/R2h_transform_ablation.txt).
-        tf32 = self._check_precision()
-        fuse_ok = self.fuse_gn and tape is None and not self.circular and p_drop == 0.0 and not tf32
-        fuse_gn = fuse_ok and (co >= self.fuse_gn_min_channels or (self.fuse_gn_narrow and co <= 32))      # net2 reads h (co channels)
-        fuse_gn1 = fuse_ok and (co >= self.fuse_gn_min_channels or (self.fuse_gn_narrow and ci <= 32 and co <= 32))
+        xc, xc_plane0, c_up = up_from or (None, 0, 0)
+        c_sk = ci - c_up                            # channels of the block input held by x
         h = self._planar(ar, f"{own}h.{co}.{tag}", b, co, grid, dev)
         h_stats = self._stats(f"{name}.h", b, co, dev)
         net1_kw = dict(out=h, chan_add=rows[name + ".net1"], step_ptr=step_ptr if rows[name + ".net1"].dim() == 3 else None,
                        stats=h_stats, circular=self.circular)
-        if fuse_gn1 and up_from is None:
+        if up_from is None and forms.gn_in_conv(ci, co):
             coef1 = ops.gn_coef(x_stats, n1.weight, n1.bias, g, voxels, n1.eps,
                                 out=ar.get(f"coef1.{name}.{b}", (b, ci, 2), torch.float32, dev))
             ops.conv3d(x, self._packed(name + ".net1", blk.net1[2]), co, x_plane0=x_plane0, c_in=ci, in_norm=coef1, **net1_kw)
-        elif up_from is not None and self.polyphase_up and not self.circular and not tf32:
-            xc, xc_plane0, c_up = up_from
+        elif up_from is not None and forms.polyphase:
             cgrid = tuple(n // 2 for n in grid)
             # silu(gn(.)) of the coarse channels at the COARSE resolution (statistics of the fine concat)
             ac = ar.get(f"ac.{c_up}.{b}x{cgrid[0]}", (b, c_up // 8) + cgrid + (8,), torch.bfloat16, dev)
@@ -464,12 +459,11 @@ class CUNet(nn.Module):
             #  channels: 2 parities (N = 256), 0.25 ms in 4 launches vs 0.30 in 8)
             n_par = 4 if co <= 32 else 2
             for grp in range(8 // n_par):
-                wp, taps = self._packed_poly(name + ".net1", blk.net1[2], c_up, grp, n_par)
-                ops.conv3d(ac, wp, n_par * co, taps=taps, out=part, out_plane0=grp * n_par * (co // 8))
+                poly = self._slot(f"{name}.net1.poly.{n_par}.{grp}", blk.net1[2], "poly", c_up, grp, n_par)
+                ops.conv3d(ac, poly.buf, n_par * co, taps=poly.taps, out=part, out_plane0=grp * n_par * (co // 8))
             # the skip channels at the fine resolution; the partial sums come in through the depth-to-space residual
-            c_sk = ci - c_up
-            w_sk = self._packed_in_slice(name + ".net1.skiphalf", blk.net1[2], c_up, c_sk)
-            if fuse_ok and (co >= self.fuse_gn_min_channels or (self.fuse_gn_narrow and c_sk <= 32 and co <= 32)):
+            w_sk = self._slot(name + ".net1.skiphalf", blk.net1[2], "slice", c_up, c_sk).buf
+            if forms.gn_in_conv(c_sk, co):
                 # GroupNorm + SiLU of the skip channels applied by the conv to its input tiles: (a, b) of all ci channels of
                 # the concat norm (groups straddle the two halves), the skip channels' rows handed to the conv
                 coef = ops.gn_coef(x_stats, n1.weight, n1.bias, g, voxels, n1.eps,
@@ -487,17 +481,16 @@ class CUNet(nn.Module):
             if up_from is None:
                 ops.gn_silu(x, ci, g, x_stats, n1.weight, n1.bias, n1.eps, x_plane0=x_plane0, out=a1)
             else:
-                xc, xc_plane0, c_up = up_from
                 ops.gn_silu_view(xc, c_up, 0, ci, g, x_stats, n1.weight, n1.bias, n1.eps, a1, x_plane0=xc_plane0,
                                  out_plane0=0, upsample=True)
-                ops.gn_silu_view(x, ci - c_up, c_up, ci, g, x_stats, n1.weight, n1.bias, n1.eps, a1,
+                ops.gn_silu_view(x, c_sk, c_up, ci, g, x_stats, n1.weight, n1.bias, n1.eps, a1,
                                  x_plane0=x_plane0 + c_up // 8, out_plane0=c_up // 8)
             a1c, _ = self._conv_input(a1, ci, 0, name + ".a1p", tape)
             ops.conv3d(a1c, self._packed(name + ".net1", blk.net1[2]), co, **net1_kw)
         if p_drop > 0.0:
             self._dropout_calls += 1
         n2 = blk.net2[0]
-        if fuse_gn:
+        if forms.gn_in_conv(co, co):
             # net2's conv reads h itself; (a, b) per (sample, channel) from h's statistics
             a2c = h
             in_norm2 = ops.gn_coef(h_stats, n2.weight, n2.bias, g, voxels, n2.eps,
@@ -515,13 +508,12 @@ class CUNet(nn.Module):
         if blk.skip_conv is None:
             res, res_plane0 = x, x_plane0
         elif up_from is not None:
-            xc, xc_plane0, c_up = up_from
             # coarse half of the skip conv (with the skip conv's bias): a small 1x1x1 conv on the half-resolution grid
             rc = ar.get(f"rc.{co}.{b}x{grid[0] // 2}", (b, co // 8) + tuple(n // 2 for n in grid) + (8,), torch.bfloat16, dev)
-            ops.conv3d(xc, self._packed_in_slice(name + ".skip.up", blk.skip_conv, 0, c_up), co, taps=ops.TAPS_1X1X1,
+            ops.conv3d(xc, self._slot(name + ".skip.up", blk.skip_conv, "slice", 0, c_up).buf, co, taps=ops.TAPS_1X1X1,
                        x_plane0=xc_plane0, c_in=c_up, out=rc, chan_add=rows[name + ".skip"])
-            w_skip = self._packed_in_slice(name + ".skip.skip", blk.skip_conv, c_up, ci - c_up)
-            if self._fused_skip_ok.get(name, True) and not tf32:
+            w_skip = self._slot(name + ".skip.skip", blk.skip_conv, "slice", c_up, c_sk).buf
+            if self._fused_skip_ok.get(name, True):
                 # fine half fused into net2's conv as one more channel chunk (centre tap only): no separate 1x1x1 launch,
                 # and the residual the epilogue reads is the coarse tensor (1/8 of the bytes)
                 try:
@@ -533,7 +525,7 @@ class CUNet(nn.Module):
                 except ops.UnsupportedFusion:
                     self._fused_skip_ok[name] = False          # wide layer: keep the skip conv as its own launch
             res = self._planar(ar, f"{own}r.{co}.{tag}", b, co, grid, dev)
-            ops.conv3d(x, w_skip, co, taps=ops.TAPS_1X1X1, x_plane0=x_plane0 + c_up // 8, c_in=ci - c_up, out=res,
+            ops.conv3d(x, w_skip, co, taps=ops.TAPS_1X1X1, x_plane0=x_plane0 + c_up // 8, c_in=c_sk, out=res,
                        residual=rc, residual_upsample=True)
             res_plane0 = 0
         else:
@@ -574,9 +566,9 @@ class CUNet(nn.Module):
         ``tape`` (a dict, training only): intermediates live in a separate arena, nothing is shared between
         layers, and every tensor the backward pass needs is recorded in it (``vdm4cdm_b200.autograd``).
         In TF32 mode ``packed`` is the fp32 planar input and ``tape`` is refused (the mode is inference-only)."""
-        tf32 = self._check_precision()
-        if tf32 and tape is not None:
+        if self._check_precision() and tape is not None:
             raise NotImplementedError("CUNet precision='tf32' is inference-only (no training tape)")
+        forms = _Forms(self, tape, training_dropout)
         lanes = self._lanes()
         b = packed.shape[0]
         dev = packed.device
@@ -608,7 +600,7 @@ class CUNet(nn.Module):
                 cat = buf(f"cat{i}", c[i + 1] + c[i], i)
                 cst = self._stats(f"cat{i}", b, c[i + 1] + c[i], dev)
                 cats[i], cat_stats[i] = cat, cst
-                self._run_block(name, blk, x, x_plane0, x_stats, rows, step_ptr, cat, c[i + 1] // lanes, cst, c[i + 1],
+                self._run_block(name, blk, forms, x, x_plane0, x_stats, rows, step_ptr, cat, c[i + 1] // lanes, cst, c[i + 1],
                                 grids[i], training_dropout, tape)
                 pooled = buf(f"pool{i}", c[i], i + 1)
                 pst = self._stats(f"pool{i}", b, c[i], dev)
@@ -617,13 +609,13 @@ class CUNet(nn.Module):
             else:
                 o = buf("bottom0", c[i], i)
                 ost = self._stats("bottom0", b, c[i], dev)
-                self._run_block(name, blk, x, x_plane0, x_stats, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout,
+                self._run_block(name, blk, forms, x, x_plane0, x_stats, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout,
                                 tape)
                 x, x_plane0, x_stats = o, 0, ost
         for j, (name, blk) in enumerate((("mid1", self.mid1), ("mid2", self.mid2))):
             o = buf(f"bottom{1 + j}", c[-1], nl - 1)
             ost = self._stats(name + ".out", b, c[-1], dev)
-            self._run_block(name, blk, x, x_plane0, x_stats, rows, step_ptr, o, 0, ost, 0, grids[-1], training_dropout,
+            self._run_block(name, blk, forms, x, x_plane0, x_stats, rows, step_ptr, o, 0, ost, 0, grids[-1], training_dropout,
                             tape)
             x, x_plane0, x_stats = o, 0, ost
         for k, i in enumerate(reversed(range(nl - 1))):
@@ -632,19 +624,19 @@ class CUNet(nn.Module):
             cat, cst = cats[i], cat_stats[i]
             o = buf(f"up{i}", c[i], i)
             ost = self._stats(name + ".out", b, c[i], dev)
-            if self.fuse_upsample and tape is None and blk.skip_conv is not None and not tf32:
+            if forms.read_coarse and blk.skip_conv is not None:
                 # the up-sampled channels are never written (see _run_block); their sums are 8x the coarse tensor's
                 torch.mul(x_stats, 8.0, out=cst[:, :c[i + 1]])
-                self._run_block(name, blk, cat, 0, cst, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout, tape,
+                self._run_block(name, blk, forms, cat, 0, cst, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout, tape,
                                 up_from=(x, x_plane0, c[i + 1]))
             else:
                 ops.upsample2(x, c[i + 1], cat, coarse_plane0=x_plane0, out_plane0=0, stats=cst, stats_c0=0)
-                self._run_block(name, blk, cat, 0, cst, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout, tape)
+                self._run_block(name, blk, forms, cat, 0, cst, rows, step_ptr, o, 0, ost, 0, grids[i], training_dropout, tape)
             x, x_plane0, x_stats = o, 0, ost
         gn = self.conv_out[0]
         if out is None:
             out = torch.empty((b, 1) + grids[0], dtype=torch.float32, device=dev)
-        if self.fuse_gn and tape is None and not self.circular and not tf32 and (self.fuse_gn_narrow and c[0] <= 32 or self.fuse_gn_min_channels <= 1):
+        if forms.gn_in_conv(c[0], 1):
             coef = ops.gn_coef(x_stats, gn.weight, gn.bias, gn.num_groups, grids[0][0] * grids[0][1] * grids[0][2], gn.eps,
                                out=ar.get(f"coef.conv_out.{b}", (b, c[0], 2), torch.float32, dev))
             ops.conv3d(x, self._packed("conv_out", self.conv_out[2]), 1, x_plane0=x_plane0, c_in=c[0], out=out, out_fp32=True,
