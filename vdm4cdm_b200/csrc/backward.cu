@@ -354,12 +354,8 @@ using namespace vdm;
 static int gn_bwd_common(const char* who, const VdmTensor* x, const VdmTensor* dy, int batch, int64_t voxels, int channels,
                          int groups, const double* stats, const float* gamma, const float* beta, float dropout_p,
                          const double* sums) {
-  VDM_CHECK_ARG(view_ok(x, channels) && view_ok(dy, channels) && stats && gamma && beta && sums, "%s: bad tensor argument", who);
-  VDM_CHECK_ARG(batch >= 1 && voxels >= 1, "%s: bad shape", who);
-  VDM_CHECK_ARG((int64_t)batch * (channels / 8) <= 65535, "%s: batch * planes exceeds 65535", who);
-  VDM_CHECK_ARG(groups >= 1 && channels % groups == 0, "%s: %d channels not divisible into %d groups", who, channels, groups);
-  VDM_CHECK_ARG(dropout_p >= 0.f && dropout_p < 1.f, "%s: dropout_p %f out of [0,1)", who, dropout_p);
-  return VDM_OK;
+  VDM_CHECK_ARG(sums, "%s: bad tensor argument", who);
+  return check_gn<8>(who, x, dy, batch, voxels, channels, groups, stats, gamma, beta, dropout_p);
 }
 
 extern "C" int vdm_gn_silu_bwd_reduce(const VdmTensor* x, const VdmTensor* dy, int batch, int64_t voxels, int channels,
@@ -394,7 +390,7 @@ extern "C" int vdm_gn_silu_bwd_apply(const VdmTensor* x, const VdmTensor* dy, co
   const int rc = gn_bwd_common("vdm_gn_silu_bwd_apply", x, dy, batch, voxels, channels, groups, stats, gamma, beta,
                                dropout_p, sums);
   if (rc != VDM_OK) return rc;
-  VDM_CHECK_ARG(view_ok(dx, channels) && (add == nullptr || view_ok(add, channels)), "vdm_gn_silu_bwd_apply: bad dx/add view");
+  VDM_CHECK_ARG(view_ok<8>(dx, channels) && (add == nullptr || view_ok<8>(add, channels)), "vdm_gn_silu_bwd_apply: bad dx/add view");
   GnBwdArgs a;
   memset(&a, 0, sizeof(a));
   a.x = *x; a.dy = *dy; a.dx = *dx; a.planes = channels / 8; a.voxels = voxels; a.groups = groups; a.stats = stats;
@@ -418,11 +414,9 @@ extern "C" int vdm_gn_silu_bwd_apply(const VdmTensor* x, const VdmTensor* dy, co
 extern "C" int vdm_avgpool2_bwd(const VdmTensor* dy, const VdmTensor* dx, int batch, int depth, int height, int width,
                                 int channels, int accumulate, double* stats, int stats_channels, int stats_c0,
                                 void* stream) {
-  VDM_CHECK_ARG(view_ok(dy, channels) && view_ok(dx, channels) && batch >= 1, "vdm_avgpool2_bwd: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_avgpool2_bwd");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_avgpool2_bwd: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0,
-                "vdm_avgpool2_bwd: fine grid (%d,%d,%d) must be even", depth, height, width);
+  VDM_CHECK_ARG(view_ok<8>(dy, channels) && view_ok<8>(dx, channels) && batch >= 1, "vdm_avgpool2_bwd: bad argument");
+  VDM_CHECK_PLANES(8, batch, channels, "vdm_avgpool2_bwd");
+  if (const int rc = check_grid("vdm_avgpool2_bwd", "fine grid", depth, height, width, true)) return rc;
   if (stats_channels <= 0) stats_channels = channels;
   const int planes = channels / 8;
   const int64_t vf = (int64_t)depth * height * width;
@@ -434,11 +428,9 @@ extern "C" int vdm_avgpool2_bwd(const VdmTensor* dy, const VdmTensor* dx, int ba
 
 extern "C" int vdm_upsample2_bwd(const VdmTensor* dy, const VdmTensor* dcoarse, int batch, int depth, int height,
                                  int width, int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok(dy, channels) && view_ok(dcoarse, channels) && batch >= 1, "vdm_upsample2_bwd: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_upsample2_bwd");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_upsample2_bwd: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0,
-                "vdm_upsample2_bwd: fine grid (%d,%d,%d) must be even", depth, height, width);
+  VDM_CHECK_ARG(view_ok<8>(dy, channels) && view_ok<8>(dcoarse, channels) && batch >= 1, "vdm_upsample2_bwd: bad argument");
+  VDM_CHECK_PLANES(8, batch, channels, "vdm_upsample2_bwd");
+  if (const int rc = check_grid("vdm_upsample2_bwd", "fine grid", depth, height, width, true)) return rc;
   if (stats_channels <= 0) stats_channels = channels;
   const int planes = channels / 8;
   const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);

@@ -306,8 +306,8 @@ using namespace vdm;
 
 extern "C" int vdm_pad_circular(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
                                 int channels, void* stream) {
-  VDM_CHECK_ARG(view_ok(x, channels) && view_ok(y, channels) && batch >= 1, "vdm_pad_circular: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_pad_circular");
+  VDM_CHECK_ARG(view_ok<8>(x, channels) && view_ok<8>(y, channels) && batch >= 1, "vdm_pad_circular: bad argument");
+  VDM_CHECK_PLANES(8, batch, channels, "vdm_pad_circular");
   VDM_CHECK_ARG(depth >= 1 && height >= 1 && width >= 1 && (int64_t)(depth + 2) * (height + 2) * (width + 2) < ((int64_t)1 << 31),
                 "vdm_pad_circular: bad grid (%d,%d,%d)", depth, height, width);
   const int planes = channels / 8;
@@ -319,8 +319,8 @@ extern "C" int vdm_pad_circular(const VdmTensor* x, const VdmTensor* y, int batc
 
 extern "C" int vdm_channel_stats(const VdmTensor* x, int batch, int64_t voxels, int channels, double* stats,
                                  int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok(x, channels) && stats && batch >= 1 && voxels >= 1, "vdm_channel_stats: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_channel_stats");
+  VDM_CHECK_ARG(view_ok<8>(x, channels) && stats && batch >= 1 && voxels >= 1, "vdm_channel_stats: bad argument");
+  VDM_CHECK_PLANES(8, batch, channels, "vdm_channel_stats");
   if (stats_channels <= 0) stats_channels = channels;
   const int planes = channels / 8;
   channel_stats_kernel<<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
@@ -329,31 +329,44 @@ extern "C" int vdm_channel_stats(const VdmTensor* x, int batch, int64_t voxels, 
   return VDM_OK;
 }
 
-extern "C" int vdm_gn_silu_step(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels,
-                                int groups, const double* stats, const float* gamma, const float* beta, float eps,
-                                float dropout_p, uint64_t seed, const int32_t* seed_step, uint32_t layer_tag, void* stream) {
-  VDM_CHECK_ARG(view_ok(x, channels) && view_ok(y, channels) && stats && gamma && beta, "vdm_gn_silu: bad tensor argument");
-  VDM_CHECK_ARG(batch >= 1 && voxels >= 1, "vdm_gn_silu: bad shape");
-  VDM_CHECK_PLANES(batch, channels, "vdm_gn_silu");
-  VDM_CHECK_ARG(groups >= 1 && channels % groups == 0, "vdm_gn_silu: %d channels not divisible into %d groups",
-                channels, groups);
-  VDM_CHECK_ARG(dropout_p >= 0.f && dropout_p < 1.f, "vdm_gn_silu: dropout_p %f out of [0,1)", dropout_p);
-  const int planes = channels / 8;
-  if ((int64_t)batch * channels * voxels * 2 > (int64_t)96 << 20)
-    gn_silu_kernel<true><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+// bf16 (vdm_gn_silu, vdm_gn_silu_step) and fp32 (vdm_gn_silu_f32, no dropout) GroupNorm + SiLU.
+template <bool F32>
+static int gn_silu_launch(const char* who, const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels,
+                          int groups, const double* stats, const float* gamma, const float* beta, float eps,
+                          float dropout_p, uint64_t seed, const int32_t* seed_step, uint32_t layer_tag, void* stream) {
+  constexpr int L = Unit<F32>::L;
+  if (const int rc = check_gn<L>(who, x, y, batch, voxels, channels, groups, stats, gamma, beta, dropout_p)) return rc;
+  const int planes = channels / L;
+  const dim3 grid = ew_grid(voxels, batch * planes);
+  constexpr int kElemBytes = 16 / L;
+  if ((int64_t)batch * channels * voxels * kElemBytes > (int64_t)96 << 20)
+    gn_silu_kernel<true, F32><<<grid, kEwThreads, 0, (cudaStream_t)stream>>>(
         *x, *y, planes, voxels, groups, stats, gamma, beta, eps, dropout_p, seed, seed_step, layer_tag);
   else
-    gn_silu_kernel<false><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+    gn_silu_kernel<false, F32><<<grid, kEwThreads, 0, (cudaStream_t)stream>>>(
         *x, *y, planes, voxels, groups, stats, gamma, beta, eps, dropout_p, seed, seed_step, layer_tag);
   VDM_CHECK_LAUNCH();
   return VDM_OK;
 }
 
+extern "C" int vdm_gn_silu_step(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels,
+                                int groups, const double* stats, const float* gamma, const float* beta, float eps,
+                                float dropout_p, uint64_t seed, const int32_t* seed_step, uint32_t layer_tag, void* stream) {
+  return gn_silu_launch<false>("vdm_gn_silu", x, y, batch, voxels, channels, groups, stats, gamma, beta, eps, dropout_p,
+                               seed, seed_step, layer_tag, stream);
+}
+
 extern "C" int vdm_gn_silu(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels, int groups,
                            const double* stats, const float* gamma, const float* beta, float eps, float dropout_p,
                            uint64_t seed, uint32_t layer_tag, void* stream) {
-  return vdm_gn_silu_step(x, y, batch, voxels, channels, groups, stats, gamma, beta, eps, dropout_p, seed, nullptr,
-                          layer_tag, stream);
+  return gn_silu_launch<false>("vdm_gn_silu", x, y, batch, voxels, channels, groups, stats, gamma, beta, eps, dropout_p,
+                               seed, nullptr, layer_tag, stream);
+}
+
+extern "C" int vdm_gn_silu_f32(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels, int groups,
+                               const double* stats, const float* gamma, const float* beta, float eps, void* stream) {
+  return gn_silu_launch<true>("vdm_gn_silu_f32", x, y, batch, voxels, channels, groups, stats, gamma, beta, eps, 0.f, 0,
+                              nullptr, 0, stream);
 }
 
 extern "C" int vdm_gn_coef(const double* stats, int batch, int channels, int groups, int64_t voxels, const float* gamma,
@@ -370,21 +383,17 @@ extern "C" int vdm_gn_coef(const double* stats, int batch, int channels, int gro
 extern "C" int vdm_gn_silu_view(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
                                 int channels, int c_off, int channels_total, int groups, const double* stats,
                                 const float* gamma, const float* beta, float eps, int upsample, void* stream) {
-  VDM_CHECK_ARG(view_ok(x, channels) && view_ok(y, channels) && stats && gamma && beta, "vdm_gn_silu_view: bad tensor argument");
+  VDM_CHECK_ARG(view_ok<8>(x, channels) && view_ok<8>(y, channels) && stats && gamma && beta, "vdm_gn_silu_view: bad tensor argument");
   VDM_CHECK_ARG(batch >= 1 && depth >= 1 && height >= 1 && width >= 1, "vdm_gn_silu_view: bad shape");
-  VDM_CHECK_PLANES(batch, channels, "vdm_gn_silu_view");
+  VDM_CHECK_PLANES(8, batch, channels, "vdm_gn_silu_view");
   VDM_CHECK_ARG(c_off >= 0 && c_off % 8 == 0 && c_off + channels <= channels_total,
                 "vdm_gn_silu_view: channel window [%d, %d) outside the %d-channel norm (c_off must be a multiple of 8)", c_off,
                 c_off + channels, channels_total);
   VDM_CHECK_ARG(groups >= 1 && channels_total % groups == 0, "vdm_gn_silu_view: %d channels not divisible into %d groups",
                 channels_total, groups);
+  if (const int rc = check_grid("vdm_gn_silu_view", "fine grid", depth, height, width, upsample != 0)) return rc;
   const int64_t vf = (int64_t)depth * height * width;
-  VDM_CHECK_ARG(vf < ((int64_t)1 << 31), "vdm_gn_silu_view: grid too large for 32-bit voxel indices");
   const int planes = channels / 8;
-  if (upsample) {
-    VDM_CHECK_ARG(depth % 2 == 0 && height % 2 == 0 && width % 2 == 0, "vdm_gn_silu_view: fine grid (%d,%d,%d) must be even",
-                  depth, height, width);
-  }
   if (upsample == 1) {
     gn_silu_view_kernel<true><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
         *x, *y, planes, c_off, channels_total, groups, depth, height, width, stats, gamma, beta, eps, (double)vf);
@@ -401,86 +410,61 @@ extern "C" int vdm_gn_silu_view(const VdmTensor* x, const VdmTensor* y, int batc
   return VDM_OK;
 }
 
+// 2x2x2 average pooling of a bf16 (vdm_avgpool2) or fp32 (vdm_avgpool2_f32) planar tensor.
+template <bool F32>
+static int avgpool2_launch(const char* who, const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height,
+                           int width, int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
+  constexpr int L = Unit<F32>::L;
+  VDM_CHECK_ARG(view_ok<L>(x, channels) && view_ok<L>(y, channels) && batch >= 1, "%s: bad argument", who);
+  VDM_CHECK_PLANES(L, batch, channels, who);
+  if (const int rc = check_grid(who, "grid", depth, height, width, true)) return rc;
+  if (stats_channels <= 0) stats_channels = channels;
+  const int planes = channels / L;
+  const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);
+  avgpool2_kernel<F32><<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+      *x, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
 extern "C" int vdm_avgpool2(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
                             int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok(x, channels) && view_ok(y, channels) && batch >= 1, "vdm_avgpool2: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_avgpool2");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_avgpool2: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0,
-                "vdm_avgpool2: grid (%d,%d,%d) must be even", depth, height, width);
+  return avgpool2_launch<false>("vdm_avgpool2", x, y, batch, depth, height, width, channels, stats, stats_channels,
+                                stats_c0, stream);
+}
+
+extern "C" int vdm_avgpool2_f32(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
+                                int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
+  return avgpool2_launch<true>("vdm_avgpool2_f32", x, y, batch, depth, height, width, channels, stats, stats_channels,
+                               stats_c0, stream);
+}
+
+// Nearest x2 up-sampling of a bf16 (vdm_upsample2) or fp32 (vdm_upsample2_f32) planar tensor; (depth, height, width) is
+// the fine grid.
+template <bool F32>
+static int upsample2_launch(const char* who, const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height,
+                            int width, int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
+  constexpr int L = Unit<F32>::L;
+  VDM_CHECK_ARG(view_ok<L>(coarse, channels) && view_ok<L>(y, channels) && batch >= 1, "%s: bad argument", who);
+  VDM_CHECK_PLANES(L, batch, channels, who);
+  if (const int rc = check_grid(who, "fine grid", depth, height, width, true)) return rc;
   if (stats_channels <= 0) stats_channels = channels;
-  const int planes = channels / 8;
-  const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);
-  avgpool2_kernel<false><<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-      *x, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
+  const int planes = channels / L;
+  const int64_t vf = (int64_t)depth * height * width;
+  upsample2_kernel<F32><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
+      *coarse, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
   VDM_CHECK_LAUNCH();
   return VDM_OK;
 }
 
 extern "C" int vdm_upsample2(const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height, int width,
                              int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok(coarse, channels) && view_ok(y, channels) && batch >= 1, "vdm_upsample2: bad argument");
-  VDM_CHECK_PLANES(batch, channels, "vdm_upsample2");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_upsample2: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth % 2 == 0 && height % 2 == 0 && width % 2 == 0 && depth >= 2 && height >= 2 && width >= 2,
-                "vdm_upsample2: fine grid (%d,%d,%d) must be even", depth, height, width);
-  if (stats_channels <= 0) stats_channels = channels;
-  const int planes = channels / 8;
-  const int64_t vf = (int64_t)depth * height * width;
-  upsample2_kernel<false><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-      *coarse, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
-}
-
-// ---- fp32 channel-planar forms (TF32 inference mode): 4 channels per plane ----------------------------------------
-extern "C" int vdm_gn_silu_f32(const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels, int groups,
-                               const double* stats, const float* gamma, const float* beta, float eps, void* stream) {
-  VDM_CHECK_ARG(view_ok_f32(x, channels) && view_ok_f32(y, channels) && stats && gamma && beta,
-                "vdm_gn_silu_f32: bad tensor argument");
-  VDM_CHECK_ARG(batch >= 1 && voxels >= 1, "vdm_gn_silu_f32: bad shape");
-  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_gn_silu_f32: batch * planes exceeds 65535");
-  VDM_CHECK_ARG(groups >= 1 && channels % groups == 0, "vdm_gn_silu_f32: %d channels not divisible into %d groups",
-                channels, groups);
-  const int planes = channels / 4;
-  if ((int64_t)batch * channels * voxels * 4 > (int64_t)96 << 20)
-    gn_silu_kernel<true, true><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-        *x, *y, planes, voxels, groups, stats, gamma, beta, eps, 0.f, 0, nullptr, 0);
-  else
-    gn_silu_kernel<false, true><<<ew_grid(voxels, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-        *x, *y, planes, voxels, groups, stats, gamma, beta, eps, 0.f, 0, nullptr, 0);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
-}
-
-extern "C" int vdm_avgpool2_f32(const VdmTensor* x, const VdmTensor* y, int batch, int depth, int height, int width,
-                                int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok_f32(x, channels) && view_ok_f32(y, channels) && batch >= 1, "vdm_avgpool2_f32: bad argument");
-  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_avgpool2_f32: batch * planes exceeds 65535");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_avgpool2_f32: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0,
-                "vdm_avgpool2_f32: grid (%d,%d,%d) must be even", depth, height, width);
-  if (stats_channels <= 0) stats_channels = channels;
-  const int planes = channels / 4;
-  const int64_t vout = (int64_t)(depth / 2) * (height / 2) * (width / 2);
-  avgpool2_kernel<true><<<ew_grid(vout, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-      *x, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return upsample2_launch<false>("vdm_upsample2", coarse, y, batch, depth, height, width, channels, stats, stats_channels,
+                                 stats_c0, stream);
 }
 
 extern "C" int vdm_upsample2_f32(const VdmTensor* coarse, const VdmTensor* y, int batch, int depth, int height, int width,
                                  int channels, double* stats, int stats_channels, int stats_c0, void* stream) {
-  VDM_CHECK_ARG(view_ok_f32(coarse, channels) && view_ok_f32(y, channels) && batch >= 1, "vdm_upsample2_f32: bad argument");
-  VDM_CHECK_ARG((int64_t)batch * (channels / 4) <= 65535, "vdm_upsample2_f32: batch * planes exceeds 65535");
-  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "vdm_upsample2_f32: grid too large for 32-bit voxel indices");
-  VDM_CHECK_ARG(depth % 2 == 0 && height % 2 == 0 && width % 2 == 0 && depth >= 2 && height >= 2 && width >= 2,
-                "vdm_upsample2_f32: fine grid (%d,%d,%d) must be even", depth, height, width);
-  if (stats_channels <= 0) stats_channels = channels;
-  const int planes = channels / 4;
-  const int64_t vf = (int64_t)depth * height * width;
-  upsample2_kernel<true><<<ew_grid(vf / 2, batch * planes), kEwThreads, 0, (cudaStream_t)stream>>>(
-      *coarse, *y, planes, depth, height, width, stats, stats_channels, stats_c0);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return upsample2_launch<true>("vdm_upsample2_f32", coarse, y, batch, depth, height, width, channels, stats,
+                                stats_channels, stats_c0, stream);
 }

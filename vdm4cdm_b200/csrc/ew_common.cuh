@@ -100,18 +100,36 @@ static inline dim3 ew_grid(int64_t voxels, int batch_planes) {
   return dim3((unsigned)blocks, (unsigned)batch_planes);
 }
 
+// A window of `channels` channels, L per 16-byte plane (8 bf16 or 4 fp32), inside a 16-byte aligned planar buffer.
+template <int L>
 static inline bool view_ok(const VdmTensor* t, int channels) {
-  return t && t->data && channels >= 8 && channels % 8 == 0 && t->plane0 >= 0 && t->planes >= t->plane0 + channels / 8 &&
-         (reinterpret_cast<uintptr_t>(t->data) & 15) == 0;
-}
-// The same for an fp32 channel-planar view (4 channels per plane).
-static inline bool view_ok_f32(const VdmTensor* t, int channels) {
-  return t && t->data && channels >= 4 && channels % 4 == 0 && t->plane0 >= 0 && t->planes >= t->plane0 + channels / 4 &&
+  return t && t->data && channels >= L && channels % L == 0 && t->plane0 >= 0 && t->planes >= t->plane0 + channels / L &&
          (reinterpret_cast<uintptr_t>(t->data) & 15) == 0;
 }
 
+// blockIdx.y = (sample, plane) of an L-lane tensor must fit the 65535 limit of gridDim.y.
+#define VDM_CHECK_PLANES(L, batch, channels, who) \
+  VDM_CHECK_ARG((int64_t)(batch) * ((channels) / (L)) <= 65535, "%s: batch * planes exceeds 65535", who)
 
-#define VDM_CHECK_PLANES(batch, channels, name) \
-  VDM_CHECK_ARG((int64_t)(batch) * ((channels) / 8) <= 65535, name ": batch * planes exceeds 65535")
+// Arguments of the GroupNorm + SiLU passes, forward (x, y) and backward (x, dy).
+template <int L>
+static inline int check_gn(const char* who, const VdmTensor* x, const VdmTensor* y, int batch, int64_t voxels, int channels,
+                           int groups, const double* stats, const float* gamma, const float* beta, float dropout_p) {
+  VDM_CHECK_ARG(view_ok<L>(x, channels) && view_ok<L>(y, channels) && stats && gamma && beta, "%s: bad tensor argument", who);
+  VDM_CHECK_ARG(batch >= 1 && voxels >= 1, "%s: bad shape", who);
+  VDM_CHECK_PLANES(L, batch, channels, who);
+  VDM_CHECK_ARG(groups >= 1 && channels % groups == 0, "%s: %d channels not divisible into %d groups", who, channels, groups);
+  VDM_CHECK_ARG(dropout_p >= 0.f && dropout_p < 1.f, "%s: dropout_p %f out of [0,1)", who, dropout_p);
+  return VDM_OK;
+}
+
+// Pooling and up-sampling grids: fewer than 2^31 voxels (the kernels split a plane index with 32-bit divisions) and, when
+// `even`, every extent even.  `noun` ("grid" or "fine grid") names the grid in the message.
+static inline int check_grid(const char* who, const char* noun, int depth, int height, int width, bool even) {
+  VDM_CHECK_ARG((int64_t)depth * height * width < ((int64_t)1 << 31), "%s: grid too large for 32-bit voxel indices", who);
+  VDM_CHECK_ARG(!even || (depth >= 2 && height >= 2 && width >= 2 && depth % 2 == 0 && height % 2 == 0 && width % 2 == 0),
+                "%s: %s (%d,%d,%d) must be even", who, noun, depth, height, width);
+  return VDM_OK;
+}
 
 }  // namespace vdm

@@ -68,43 +68,44 @@ pack_conv_weight_batched_kernel(const VdmPackJob* __restrict__ jobs) {
 
 using namespace vdm;
 
-extern "C" int vdm_pack_conv_weight(const float* w, void* packed, int c_out, int c_in, int kernel, int transpose_flip,
-                                    int ci0, int n_ci, int c_in_pad, int c_out_pad, void* stream) {
-  VDM_CHECK_ARG(w && packed && c_out >= 1 && c_in >= 1 && kernel >= 1 && kernel <= 3, "vdm_pack_conv_weight: bad argument");
-  VDM_CHECK_ARG(c_in_pad % 16 == 0 && c_out_pad % 16 == 0 && c_in_pad >= 16 && c_out_pad >= 16,
-                "vdm_pack_conv_weight: padded sizes (%d, %d) must be multiples of 16", c_in_pad, c_out_pad);
-  VDM_CHECK_ARG((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "vdm_pack_conv_weight: packed must be 16-byte aligned");
+// One filter as bf16 (vdm_pack_conv_weight: forward or dgrad slice) or TF32-rounded fp32 (vdm_pack_conv_weight_f32: forward
+// only, transpose_flip = 0).  c_in_pad is a whole number of 32-byte K steps: 16 bf16 or 8 fp32 channels.
+template <bool F32>
+static int pack_conv_weight_launch(const char* who, const float* w, void* packed, int c_out, int c_in, int kernel,
+                                   int transpose_flip, int ci0, int n_ci, int c_in_pad, int c_out_pad, void* stream) {
+  using Chunk = std::conditional_t<F32, uint4, bf16x8>;
+  constexpr int L = F32 ? 4 : 8;       // K values per 16-byte chunk
+  VDM_CHECK_ARG(w && packed && c_out >= 1 && c_in >= 1 && kernel >= 1 && kernel <= 3, "%s: bad argument", who);
+  VDM_CHECK_ARG(c_in_pad % (2 * L) == 0 && c_out_pad % 16 == 0 && c_in_pad >= 2 * L && c_out_pad >= 16,
+                F32 ? "%s: padded sizes (%d, %d) must be multiples of 8 and 16" : "%s: padded sizes (%d, %d) must be multiples of 16",
+                who, c_in_pad, c_out_pad);
+  VDM_CHECK_ARG((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "%s: packed must be 16-byte aligned", who);
   if (!transpose_flip) {
-    VDM_CHECK_ARG(c_in <= c_in_pad && c_out <= c_out_pad, "vdm_pack_conv_weight: padded sizes smaller than the filter");
+    VDM_CHECK_ARG(c_in <= c_in_pad && c_out <= c_out_pad, "%s: padded sizes smaller than the filter", who);
   } else {
     VDM_CHECK_ARG(ci0 >= 0 && n_ci >= 1 && ci0 + n_ci <= c_in && c_out <= c_in_pad && n_ci <= c_out_pad,
-                  "vdm_pack_conv_weight: dgrad slice [%d, %d) of %d input channels does not fit", ci0, ci0 + n_ci, c_in);
+                  "%s: dgrad slice [%d, %d) of %d input channels does not fit", who, ci0, ci0 + n_ci, c_in);
   }
   const int k3 = kernel * kernel * kernel;
-  const int64_t total = (int64_t)k3 * (c_in_pad / 8) * c_out_pad;
+  const int64_t total = (int64_t)k3 * (c_in_pad / L) * c_out_pad;
   int64_t blocks = (total + 255) / 256;
   if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
   pack_conv_weight_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-      w, static_cast<bf16x8*>(packed), c_out, c_in, k3, transpose_flip, ci0, n_ci, c_in_pad, c_out_pad);
+      w, static_cast<Chunk*>(packed), c_out, c_in, k3, transpose_flip, ci0, n_ci, c_in_pad, c_out_pad);
   VDM_CHECK_LAUNCH();
   return VDM_OK;
 }
 
+extern "C" int vdm_pack_conv_weight(const float* w, void* packed, int c_out, int c_in, int kernel, int transpose_flip,
+                                    int ci0, int n_ci, int c_in_pad, int c_out_pad, void* stream) {
+  return pack_conv_weight_launch<false>("vdm_pack_conv_weight", w, packed, c_out, c_in, kernel, transpose_flip, ci0, n_ci,
+                                        c_in_pad, c_out_pad, stream);
+}
+
 extern "C" int vdm_pack_conv_weight_f32(const float* w, void* packed, int c_out, int c_in, int kernel, int c_in_pad,
                                         int c_out_pad, void* stream) {
-  VDM_CHECK_ARG(w && packed && c_out >= 1 && c_in >= 1 && kernel >= 1 && kernel <= 3, "vdm_pack_conv_weight_f32: bad argument");
-  VDM_CHECK_ARG(c_in_pad % 8 == 0 && c_out_pad % 16 == 0 && c_in_pad >= 8 && c_out_pad >= 16,
-                "vdm_pack_conv_weight_f32: padded sizes (%d, %d) must be multiples of 8 and 16", c_in_pad, c_out_pad);
-  VDM_CHECK_ARG(c_in <= c_in_pad && c_out <= c_out_pad, "vdm_pack_conv_weight_f32: padded sizes smaller than the filter");
-  VDM_CHECK_ARG((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "vdm_pack_conv_weight_f32: packed must be 16-byte aligned");
-  const int k3 = kernel * kernel * kernel;
-  const int64_t total = (int64_t)k3 * (c_in_pad / 4) * c_out_pad;
-  int64_t blocks = (total + 255) / 256;
-  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
-  pack_conv_weight_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(w, static_cast<uint4*>(packed), c_out, c_in, k3, 0, 0,
-                                                                              c_out, c_in_pad, c_out_pad);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return pack_conv_weight_launch<true>("vdm_pack_conv_weight_f32", w, packed, c_out, c_in, kernel, 0, 0, c_out, c_in_pad,
+                                       c_out_pad, stream);
 }
 
 extern "C" int vdm_pack_conv_weight_batched(const VdmPackJob* jobs_device, int n_jobs, void* stream) {

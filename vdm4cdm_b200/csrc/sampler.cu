@@ -137,6 +137,23 @@ static inline dim3 grid_for(int64_t work_items, int batch, int threads) {
   return dim3((unsigned)blocks, (unsigned)batch);
 }
 
+// The packed network input as bf16 (vdm_pack_input) or fp32 (vdm_pack_input_f32) planes; the kernel stores 16-byte units.
+template <bool F32>
+static int pack_input_launch(const char* who, const float* z, const float* cond, const VdmTensor* out, int batch,
+                             int64_t voxels, int n_cond, int c_pad, void* stream) {
+  constexpr int L = Unit<F32>::L;
+  VDM_CHECK_ARG(z && out && out->data && batch >= 1 && batch <= 65535 && voxels >= 1 &&
+                    (reinterpret_cast<uintptr_t>(out->data) & 15) == 0, "%s: bad argument", who);
+  VDM_CHECK_ARG(c_pad >= 8 && c_pad % 8 == 0 && n_cond >= 0 && n_cond + 1 <= 8 && out->plane0 >= 0 &&
+                    out->planes >= out->plane0 + c_pad / L,
+                "%s: bad c_pad %d / n_cond %d / plane window", who, c_pad, n_cond);
+  VDM_CHECK_ARG(n_cond == 0 || cond, "%s: cond is NULL with n_cond=%d", who, n_cond);
+  const dim3 grid = grid_for(voxels, batch, 256);
+  pack_input_kernel<F32><<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / L, voxels, n_cond);
+  VDM_CHECK_LAUNCH();
+  return VDM_OK;
+}
+
 }  // namespace vdm
 
 extern "C" int vdm_sampler_step(const float* z, const float* eps_hat, float* z_out, int batch, int64_t voxels,
@@ -171,27 +188,10 @@ extern "C" int vdm_philox_normal(float* out, int batch, int64_t voxels, uint64_t
 
 extern "C" int vdm_pack_input(const float* z, const float* cond, const VdmTensor* out, int batch, int64_t voxels,
                               int n_cond, int c_pad, void* stream) {
-  VDM_CHECK_ARG(z && out && out->data && batch >= 1 && batch <= 65535 && voxels >= 1, "vdm_pack_input: bad argument");
-  VDM_CHECK_ARG(c_pad >= 8 && c_pad % 8 == 0 && n_cond >= 0 && n_cond + 1 <= 8 && out->plane0 >= 0 &&
-                    out->planes >= out->plane0 + c_pad / 8,
-                "vdm_pack_input: bad c_pad %d / n_cond %d / plane window", c_pad, n_cond);
-  VDM_CHECK_ARG(n_cond == 0 || cond, "vdm_pack_input: cond is NULL with n_cond=%d", n_cond);
-  const dim3 grid = vdm::grid_for(voxels, batch, 256);
-  vdm::pack_input_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / 8, voxels, n_cond);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return vdm::pack_input_launch<false>("vdm_pack_input", z, cond, out, batch, voxels, n_cond, c_pad, stream);
 }
 
 extern "C" int vdm_pack_input_f32(const float* z, const float* cond, const VdmTensor* out, int batch, int64_t voxels,
                                   int n_cond, int c_pad, void* stream) {
-  VDM_CHECK_ARG(z && out && out->data && batch >= 1 && batch <= 65535 && voxels >= 1 &&
-                    (reinterpret_cast<uintptr_t>(out->data) & 15) == 0, "vdm_pack_input_f32: bad argument");
-  VDM_CHECK_ARG(c_pad >= 8 && c_pad % 8 == 0 && n_cond >= 0 && n_cond + 1 <= 8 && out->plane0 >= 0 &&
-                    out->planes >= out->plane0 + c_pad / 4,
-                "vdm_pack_input_f32: bad c_pad %d / n_cond %d / plane window", c_pad, n_cond);
-  VDM_CHECK_ARG(n_cond == 0 || cond, "vdm_pack_input_f32: cond is NULL with n_cond=%d", n_cond);
-  const dim3 grid = vdm::grid_for(voxels, batch, 256);
-  vdm::pack_input_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(z, cond, *out, c_pad / 4, voxels, n_cond);
-  VDM_CHECK_LAUNCH();
-  return VDM_OK;
+  return vdm::pack_input_launch<true>("vdm_pack_input_f32", z, cond, out, batch, voxels, n_cond, c_pad, stream);
 }

@@ -32,9 +32,16 @@ def launch_count() -> int:
     return _LAUNCHES
 
 
-def _launched(n: int = 1) -> None:
+def _call(name: str, *args, launches: int = 1, fused: bool = False) -> None:
+    """Calls the C entry point ``name`` and counts the ``launches`` kernels it issues.  A refusal or launch error raises
+    ``RuntimeError``; with ``fused`` (an optional fused form was asked for), ``VDM_E_UNSUPPORTED`` raises
+    ``UnsupportedFusion`` so the caller can run the unfused launches instead."""
     global _LAUNCHES
-    _LAUNCHES += n
+    rc = getattr(_C.lib(), name)(*args)
+    if fused and rc == _C.E_UNSUPPORTED:
+        raise _C.UnsupportedFusion(_C.lib().vdm_last_error_string().decode("utf-8", "replace"))
+    _C.check(rc, name)
+    _LAUNCHES += launches
 
 
 _CONV_PROFILE = None
@@ -56,6 +63,20 @@ def set_profile_tag(tag: str) -> None:
     _PROFILE_TAG = tag
 
 
+def _conv_profiled(launch, label: str, n_taps: int, c_in: int, c_out: int, b: int, d: int, h: int, w: int) -> None:
+    """Runs ``launch()``; while ``set_conv_profiler`` is on, brackets it with events on the launching stream and records
+    them with the algorithmic FLOPs (real, un-padded output channels; the input channels the caller says it reads)."""
+    prof = _CONV_PROFILE
+    if prof is None:
+        return launch()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    launch()
+    e1.record()
+    prof.append((e0, e1, 2.0 * n_taps * c_in * c_out * b * d * h * w,
+                 f"{label}{c_in}->{c_out} taps={n_taps} grid={d}x{h}x{w} B={b}"))
+
+
 def _stream() -> int:
     return torch.cuda.current_stream().cuda_stream
 
@@ -69,25 +90,27 @@ def _need(cond: bool, msg: str) -> None:
         raise ValueError(msg)
 
 
-def _planar_ok(t: torch.Tensor, name: str) -> None:
-    _need(t.is_cuda and t.dtype == torch.bfloat16 and t.dim() == 6 and t.shape[-1] == 8 and t.is_contiguous(),
-          f"{name}: expected a contiguous CUDA bf16 [B,P,D,H,W,8] tensor, got {tuple(t.shape)} {t.dtype} {t.device}")
-
-
 _LANES = {torch.bfloat16: 8, torch.float32: 4}       # channels per 16-byte plane of a planar tensor
+_LAYOUTS = {8: "bf16 [B,P,D,H,W,8]", 4: "fp32 [B,P,D,H,W,4]"}
 
 
-def _planar_lanes(t: torch.Tensor, name: str) -> int:
-    """Channels per plane (8: bf16, 4: fp32) of a contiguous CUDA channel-planar tensor."""
-    lanes = _LANES.get(t.dtype)
-    _need(t.is_cuda and lanes is not None and t.dim() == 6 and t.shape[-1] == lanes and t.is_contiguous(),
-          f"{name}: expected a contiguous CUDA bf16 [B,P,D,H,W,8] or fp32 [B,P,D,H,W,4] tensor, got "
-          f"{tuple(t.shape)} {t.dtype} {t.device}")
-    return lanes
+def _planar_lanes(t: torch.Tensor, name: str, lanes: Optional[int] = None) -> int:
+    """Channels per plane (8: bf16, 4: fp32) of a contiguous CUDA channel-planar tensor; ``lanes`` admits one layout only."""
+    got = _LANES.get(t.dtype)
+    if not (t.is_cuda and got is not None and lanes in (None, got) and t.dim() == 6 and t.shape[-1] == got and
+            t.is_contiguous()):
+        want = " or ".join(_LAYOUTS.values()) if lanes is None else _LAYOUTS[lanes]
+        raise ValueError(f"{name}: expected a contiguous CUDA {want} tensor, got {tuple(t.shape)} {t.dtype} {t.device}")
+    return got
 
 
 def _same_lanes(lanes: int, t: torch.Tensor, name: str) -> None:
     _need(_planar_lanes(t, name) == lanes, f"{name}: bf16 and fp32 planar tensors mixed in one call")
+
+
+def _by_lanes(name: str, lanes: int) -> str:
+    """The C entry point ``name`` (bf16 planar tensors) or its ``_f32`` form (fp32 planar tensors, 4 lanes)."""
+    return name + "_f32" if lanes == 4 else name
 
 
 def _view(t: torch.Tensor, plane0: int) -> _C.Tensor:
@@ -158,17 +181,13 @@ def pack_conv_weight_into(w: torch.Tensor, out: torch.Tensor, transpose_flip: bo
         _need(not transpose_flip and ci0 == 0 and n_ci in (None, ci), "pack_conv_weight_into: the fp32 (TF32) filter is forward-only")
         _need(out.is_cuda and out.is_contiguous() and tuple(out.shape) == packed_weight_shape(w.shape, dtype=torch.float32),
               "pack_conv_weight_into: bad out tensor")
-        rc = _C.lib().vdm_pack_conv_weight_f32(w.data_ptr(), out.data_ptr(), co, ci, k, out.shape[1] * 4, out.shape[2], _stream())
-        _C.check(rc, "vdm_pack_conv_weight_f32")
-        _launched(1)
+        _call("vdm_pack_conv_weight_f32", w.data_ptr(), out.data_ptr(), co, ci, k, out.shape[1] * 4, out.shape[2], _stream())
         return out
     n_ci = ci if n_ci is None else n_ci
     _need(out.is_cuda and out.dtype == torch.bfloat16 and out.is_contiguous() and
           tuple(out.shape) == packed_weight_shape(w.shape, transpose_flip, n_ci), "pack_conv_weight_into: bad out tensor")
-    rc = _C.lib().vdm_pack_conv_weight(w.data_ptr(), out.data_ptr(), co, ci, k, 1 if transpose_flip else 0, ci0, n_ci,
-                                       out.shape[1] * 8, out.shape[2], _stream())
-    _C.check(rc, "vdm_pack_conv_weight")
-    _launched(1)
+    _call("vdm_pack_conv_weight", w.data_ptr(), out.data_ptr(), co, ci, k, 1 if transpose_flip else 0, ci0, n_ci,
+          out.shape[1] * 8, out.shape[2], _stream())
     return out
 
 
@@ -190,9 +209,7 @@ def pack_job_table(jobs, device) -> torch.Tensor:
 
 def pack_conv_weights_batched(table: torch.Tensor, n_jobs: int) -> None:
     """``vdm_pack_conv_weight_batched``: every job of ``pack_job_table`` in one launch."""
-    rc = _C.lib().vdm_pack_conv_weight_batched(table.data_ptr(), n_jobs, _stream())
-    _C.check(rc, "vdm_pack_conv_weight_batched")
-    _launched(1)
+    _call("vdm_pack_conv_weight_batched", table.data_ptr(), n_jobs, _stream())
 
 
 # ---- VDM training loss (csrc/vdm_loss.cu) ---------------------------------------------------------------
@@ -209,10 +226,8 @@ def loss_zt(x, noise, times, gamma_b, gamma_w, learned: bool) -> torch.Tensor:
     """``vdm_loss_zt``: z_t = alpha_t x + sigma_t noise, schedule parameters read on the device."""
     b, n = _loss_args_ok(x, noise)
     zt = torch.empty_like(x)
-    rc = _C.lib().vdm_loss_zt(x.data_ptr(), noise.data_ptr(), times.data_ptr(), gamma_b.data_ptr(), gamma_w.data_ptr(),
-                              1 if learned else 0, zt.data_ptr(), b, n, _stream())
-    _C.check(rc, "vdm_loss_zt")
-    _launched(1)
+    _call("vdm_loss_zt", x.data_ptr(), noise.data_ptr(), times.data_ptr(), gamma_b.data_ptr(), gamma_w.data_ptr(),
+          1 if learned else 0, zt.data_ptr(), b, n, _stream())
     return zt
 
 
@@ -221,10 +236,8 @@ def loss_zt_bwd(g_zt, x, noise, times, gamma_b, gamma_w, learned: bool) -> torch
     b, n = _loss_args_ok(g_zt, x, noise)
     work = torch.empty(2 * b, dtype=torch.float64, device=x.device)
     out = torch.empty(2, dtype=torch.float32, device=x.device)
-    rc = _C.lib().vdm_loss_zt_bwd(g_zt.data_ptr(), x.data_ptr(), noise.data_ptr(), times.data_ptr(), gamma_b.data_ptr(),
-                                  gamma_w.data_ptr(), 1 if learned else 0, work.data_ptr(), out.data_ptr(), b, n, _stream())
-    _C.check(rc, "vdm_loss_zt_bwd")
-    _launched(2)
+    _call("vdm_loss_zt_bwd", g_zt.data_ptr(), x.data_ptr(), noise.data_ptr(), times.data_ptr(), gamma_b.data_ptr(),
+          gamma_w.data_ptr(), 1 if learned else 0, work.data_ptr(), out.data_ptr(), b, n, _stream(), launches=2)
     return out
 
 
@@ -233,11 +246,9 @@ def loss_terms(pred, noise, x, noise0, gamma_b, gamma_w, learned: bool, data_noi
     b, n = _loss_args_ok(pred, noise, x, noise0)
     work = torch.empty(3 * b, dtype=torch.float64, device=x.device)
     out = torch.empty(8, dtype=torch.float32, device=x.device)
-    rc = _C.lib().vdm_loss_terms(pred.data_ptr(), noise.data_ptr(), x.data_ptr(), noise0.data_ptr(), gamma_b.data_ptr(),
-                                 gamma_w.data_ptr(), 1 if learned else 0, float(data_noise), work.data_ptr(), out.data_ptr(),
-                                 b, n, _stream())
-    _C.check(rc, "vdm_loss_terms")
-    _launched(2)
+    _call("vdm_loss_terms", pred.data_ptr(), noise.data_ptr(), x.data_ptr(), noise0.data_ptr(), gamma_b.data_ptr(),
+          gamma_w.data_ptr(), 1 if learned else 0, float(data_noise), work.data_ptr(), out.data_ptr(), b, n, _stream(),
+          launches=2)
     return out
 
 
@@ -245,10 +256,8 @@ def loss_dpred(pred, noise, coef, g_loss) -> torch.Tensor:
     """``vdm_loss_dpred``: d eps_hat = g_loss * coef * (eps_hat - eps) (coef, g_loss: one-element fp32 CUDA tensors)."""
     _loss_args_ok(pred, noise)
     d = torch.empty_like(pred)
-    rc = _C.lib().vdm_loss_dpred(pred.data_ptr(), noise.data_ptr(), coef.data_ptr(), g_loss.data_ptr(), d.data_ptr(),
-                                 pred.numel(), _stream())
-    _C.check(rc, "vdm_loss_dpred")
-    _launched(1)
+    _call("vdm_loss_dpred", pred.data_ptr(), noise.data_ptr(), coef.data_ptr(), g_loss.data_ptr(), d.data_ptr(), pred.numel(),
+          _stream())
     return d
 
 
@@ -352,21 +361,10 @@ def conv3d(x: torch.Tensor, w_packed: torch.Tensor, c_out: int, *, taps: Sequenc
         epi.stats = stats.data_ptr()
         epi.stats_channels = stats.shape[1]
         epi.stats_c0 = stats_c0
-    prof = _CONV_PROFILE
-    if prof is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-    fn = _C.lib().vdm_conv3d_tf32 if tf32 else _C.lib().vdm_conv3d
-    rc = fn(ctypes.byref(desc), x.data_ptr(), w_packed.data_ptr(), out.data_ptr(), ctypes.byref(epi), _stream())
-    if rc == _C.E_UNSUPPORTED and (skip_x is not None or in_norm is not None or (tf32 and residual_upsample)):
-        raise _C.UnsupportedFusion(_C.lib().vdm_last_error_string().decode("utf-8", "replace"))
-    _C.check(rc, "vdm_conv3d_tf32" if tf32 else "vdm_conv3d")
-    _launched(1)
-    if prof is not None:
-        e1.record()
-        # algorithmic FLOPs: real (un-padded) output channels, the channels the caller says it reads
-        prof.append((e0, e1, 2.0 * n_taps * c_in * c_out * b * d * h * w_,
-                     f"{_PROFILE_TAG}{'tf32 ' if tf32 else ''}{c_in}->{c_out} taps={n_taps} grid={d}x{h}x{w_} B={b}"))
+    fused = skip_x is not None or in_norm is not None or bool(tf32 and residual_upsample)
+    _conv_profiled(lambda: _call("vdm_conv3d_tf32" if tf32 else "vdm_conv3d", ctypes.byref(desc), x.data_ptr(),
+                                 w_packed.data_ptr(), out.data_ptr(), ctypes.byref(epi), _stream(), fused=fused),
+                   _PROFILE_TAG + ("tf32 " if tf32 else ""), n_taps, c_in, c_out, b, d, h, w_)
     return out
 
 
@@ -430,16 +428,13 @@ def polyphase_group(w: torch.Tensor, group: int, n_par: int):
 # ---- elementwise ---------------------------------------------------------------------------------
 def channel_stats(x: torch.Tensor, channels: int, x_plane0: int = 0, stats: Optional[torch.Tensor] = None,
                   stats_c0: int = 0) -> torch.Tensor:
-    _planar_ok(x, "channel_stats x")
+    _planar_lanes(x, "channel_stats x", 8)
     b = x.shape[0]
     voxels = x.shape[2] * x.shape[3] * x.shape[4]
     if stats is None:
         stats = torch.zeros((b, channels, 2), dtype=torch.float64, device=x.device)
     v = _view(x, x_plane0)
-    rc = _C.lib().vdm_channel_stats(ctypes.byref(v), b, voxels, channels, stats.data_ptr(), stats.shape[1], stats_c0,
-                                    _stream())
-    _C.check(rc, "vdm_channel_stats")
-    _launched(1)
+    _call("vdm_channel_stats", ctypes.byref(v), b, voxels, channels, stats.data_ptr(), stats.shape[1], stats_c0, _stream())
     return stats
 
 
@@ -461,16 +456,11 @@ def gn_silu(x: torch.Tensor, channels: int, groups: int, stats: torch.Tensor, ga
     vx, vy = _view(x, x_plane0), _view(out, out_plane0)
     if lanes == 4:
         _need(dropout_p == 0.0, "gn_silu: the fp32 (TF32 inference) form has no dropout")
-        rc = _C.lib().vdm_gn_silu_f32(ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
-                                      gamma.data_ptr(), beta.data_ptr(), eps, _stream())
-        _C.check(rc, "vdm_gn_silu_f32")
-        _launched(1)
-        return out
-    rc = _C.lib().vdm_gn_silu_step(ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
-                                   gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag,
-                                   _stream())
-    _C.check(rc, "vdm_gn_silu")
-    _launched(1)
+        _call("vdm_gn_silu_f32", ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
+              gamma.data_ptr(), beta.data_ptr(), eps, _stream())
+    else:
+        _call("vdm_gn_silu_step", ctypes.byref(vx), ctypes.byref(vy), b, voxels, channels, groups, stats.data_ptr(),
+              gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag, _stream())
     return out
 
 
@@ -488,10 +478,8 @@ def gn_coef(stats: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, groups
         out = torch.empty((b, c, 2), dtype=torch.float32, device=stats.device)
     _need(out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (b, c, 2),
           "gn_coef: out must be contiguous CUDA fp32 [B, C, 2]")
-    rc = _C.lib().vdm_gn_coef(stats.data_ptr(), b, c, groups, voxels, gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(),
-                              _stream())
-    _C.check(rc, "vdm_gn_coef")
-    _launched(1)
+    _call("vdm_gn_coef", stats.data_ptr(), b, c, groups, voxels, gamma.data_ptr(), beta.data_ptr(), eps, out.data_ptr(),
+          _stream())
     return out
 
 
@@ -500,8 +488,8 @@ def gn_silu_view(x: torch.Tensor, channels: int, c_off: int, channels_total: int
                  out_plane0: int = 0, upsample=False) -> torch.Tensor:
     """silu(groupnorm(.)) of channels [c_off, c_off + channels) of a ``channels_total``-channel norm, written to a plane
     window of ``out``; with ``upsample`` x is at half the resolution of ``out`` (``vdm_gn_silu_view``)."""
-    _planar_ok(x, "gn_silu_view x")
-    _planar_ok(out, "gn_silu_view out")
+    _planar_lanes(x, "gn_silu_view x", 8)
+    _planar_lanes(out, "gn_silu_view out", 8)
     b, _, d, h, w, _ = out.shape
     if upsample == "coarse":         # x and out on the half grid of the (2d, 2h, 2w) concat the statistics refer to
         _need(tuple(x.shape[2:5]) == (d, h, w) and x.shape[0] == b, "gn_silu_view: x grid does not match out")
@@ -515,11 +503,9 @@ def gn_silu_view(x: torch.Tensor, channels: int, c_off: int, channels_total: int
           beta.numel() == channels_total and gamma.is_cuda and beta.is_cuda,
           "gn_silu_view: gamma/beta must be CUDA fp32 [channels_total]")
     vx, vy = _view(x, x_plane0), _view(out, out_plane0)
-    rc = _C.lib().vdm_gn_silu_view(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, c_off, channels_total, groups,
-                                   stats.data_ptr(), gamma.data_ptr(), beta.data_ptr(), eps,
-                                   2 if upsample == "coarse" else (1 if upsample else 0), _stream())
-    _C.check(rc, "vdm_gn_silu_view")
-    _launched(1)
+    _call("vdm_gn_silu_view", ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, c_off, channels_total, groups,
+          stats.data_ptr(), gamma.data_ptr(), beta.data_ptr(), eps, 2 if upsample == "coarse" else (1 if upsample else 0),
+          _stream())
     return out
 
 
@@ -531,11 +517,8 @@ def avgpool2(x: torch.Tensor, channels: int, *, x_plane0: int = 0, out: Optional
         out = torch.empty((b, channels // lanes, d // 2, h // 2, w // 2, lanes), dtype=x.dtype, device=x.device)
     _same_lanes(lanes, out, "avgpool2 out")
     vx, vy = _view(x, x_plane0), _view(out, out_plane0)
-    fn = _C.lib().vdm_avgpool2_f32 if lanes == 4 else _C.lib().vdm_avgpool2
-    rc = fn(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats), 0 if stats is None else stats.shape[1],
-            stats_c0, _stream())
-    _C.check(rc, "vdm_avgpool2_f32" if lanes == 4 else "vdm_avgpool2")
-    _launched(1)
+    _call(_by_lanes("vdm_avgpool2", lanes), ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats),
+          0 if stats is None else stats.shape[1], stats_c0, _stream())
     return out
 
 
@@ -546,11 +529,8 @@ def upsample2(coarse: torch.Tensor, channels: int, out: torch.Tensor, *, coarse_
     b, _, d, h, w, _ = out.shape
     _need(tuple(coarse.shape[2:5]) == (d // 2, h // 2, w // 2), "upsample2: coarse grid must be half the fine grid")
     vx, vy = _view(coarse, coarse_plane0), _view(out, out_plane0)
-    fn = _C.lib().vdm_upsample2_f32 if lanes == 4 else _C.lib().vdm_upsample2
-    rc = fn(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats), 0 if stats is None else stats.shape[1],
-            stats_c0, _stream())
-    _C.check(rc, "vdm_upsample2_f32" if lanes == 4 else "vdm_upsample2")
-    _launched(1)
+    _call(_by_lanes("vdm_upsample2", lanes), ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels, _ptr(stats),
+          0 if stats is None else stats.shape[1], stats_c0, _stream())
     return out
 
 
@@ -566,9 +546,7 @@ def pad_circular(x: torch.Tensor, channels: int, *, x_plane0: int = 0, out: Opti
     _need(channels % lanes == 0, f"pad_circular: channels={channels} is not a whole number of planes")
     vx, vy = _view(x, x_plane0), _view(out, 0)
     # the C entry point counts 8 channels per 16-byte plane
-    rc = _C.lib().vdm_pad_circular(ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels * 8 // lanes, _stream())
-    _C.check(rc, "vdm_pad_circular")
-    _launched(1)
+    _call("vdm_pad_circular", ctypes.byref(vx), ctypes.byref(vy), b, d, h, w, channels * 8 // lanes, _stream())
     return out
 
 
@@ -592,10 +570,8 @@ def pack_input(z: torch.Tensor, cond: Optional[torch.Tensor], c_pad: int = 16,
         out = torch.empty((b, c_pad // lanes, d, h, w, lanes), dtype=dtype, device=z.device)
     lanes = _planar_lanes(out, "pack_input out")
     vo = _view(out, 0)
-    fn = _C.lib().vdm_pack_input_f32 if lanes == 4 else _C.lib().vdm_pack_input
-    rc = fn(z.data_ptr(), _ptr(cond), ctypes.byref(vo), b, d * h * w, n_cond, c_pad, _stream())
-    _C.check(rc, "vdm_pack_input_f32" if lanes == 4 else "vdm_pack_input")
-    _launched(1)
+    _call(_by_lanes("vdm_pack_input", lanes), z.data_ptr(), _ptr(cond), ctypes.byref(vo), b, d * h * w, n_cond, c_pad,
+          _stream())
     return out
 
 
@@ -607,8 +583,8 @@ def conv3d_wgrad(a: torch.Tensor, g: torch.Tensor, c_in: int, c_out: int, kernel
 
     a, g: planar buffers on the same grid; the g window must hold c_out rounded up to 16 channels.
     ``out`` is accumulated into (allocated and zeroed when None)."""
-    _planar_ok(a, "conv3d_wgrad a")
-    _planar_ok(g, "conv3d_wgrad g")
+    _planar_lanes(a, "conv3d_wgrad a", 8)
+    _planar_lanes(g, "conv3d_wgrad g", 8)
     b, ap, d, h, w_, _ = a.shape
     if a_padded:                       # a carries a one-voxel periodic halo (circular convs)
         d, h, w_ = d - 2, h - 2, w_ - 2
@@ -634,17 +610,8 @@ def conv3d_wgrad(a: torch.Tensor, g: torch.Tensor, c_in: int, c_out: int, kernel
     desc.g_planes, desc.g_plane0 = g.shape[1], g_plane0
     desc.a_padded = 1 if a_padded else 0
     desc.g_padded = 1 if g_padded else 0
-    prof = _CONV_PROFILE
-    if prof is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-    rc = _C.lib().vdm_conv3d_wgrad(ctypes.byref(desc), a.data_ptr(), g.data_ptr(), out.data_ptr(), _stream())
-    _C.check(rc, "vdm_conv3d_wgrad")
-    _launched(1)
-    if prof is not None:
-        e1.record()
-        prof.append((e0, e1, 2.0 * kernel ** 3 * c_in * c_out * b * d * h * w_,
-                     f"wgrad {c_in}->{c_out} taps={kernel ** 3} grid={d}x{h}x{w_} B={b}"))
+    _conv_profiled(lambda: _call("vdm_conv3d_wgrad", ctypes.byref(desc), a.data_ptr(), g.data_ptr(), out.data_ptr(), _stream()),
+                   "wgrad ", kernel ** 3, c_in, c_out, b, d, h, w_)
     return out
 
 
@@ -655,7 +622,7 @@ def wgrad_to_torch(dw: torch.Tensor, kernel: int) -> torch.Tensor:
 
 
 def _gn_common(x, channels, stats, gamma, beta, who):
-    _planar_ok(x, f"{who} x")
+    _planar_lanes(x, f"{who} x", 8)
     b = x.shape[0]
     _need(stats.dtype == torch.float64 and tuple(stats.shape) == (b, channels, 2) and stats.is_contiguous(),
           f"{who}: stats must be double [B, channels, 2]")
@@ -674,61 +641,53 @@ def gn_silu_bwd(x: torch.Tensor, dy: torch.Tensor, channels: int, groups: int, s
     (sum du, sum du*xhat), i.e. dbeta = sums[..., 0].sum(0), dgamma = sums[..., 1].sum(0).
     dx = GroupNorm/SiLU/dropout backward of dy [+ add]; ``out_stats`` accumulates (sum, sumsq) of dx."""
     b, voxels = _gn_common(x, channels, stats, gamma, beta, "gn_silu_bwd")
-    _planar_ok(dy, "gn_silu_bwd dy")
+    _planar_lanes(dy, "gn_silu_bwd dy", 8)
     if out is None:
         out = torch.empty((b, channels // 8) + tuple(x.shape[2:]), dtype=torch.bfloat16, device=x.device)
-    _planar_ok(out, "gn_silu_bwd out")
+    _planar_lanes(out, "gn_silu_bwd out", 8)
     if sums is None:
         sums = torch.zeros((b, channels, 2), dtype=torch.float64, device=x.device)
     _need(sums.dtype == torch.float64 and sums.is_contiguous() and sums.dim() == 3 and sums.shape[0] == b and
           sums.shape[2] == 2 and sums_c0 + channels <= sums.shape[1], "gn_silu_bwd: sums must be a zeroed double [B, >= channels, 2]")
     vx, vg, vo = _view(x, x_plane0), _view(dy, dy_plane0), _view(out, out_plane0)
-    lib = _C.lib()
-    rc = lib.vdm_gn_silu_bwd_reduce(ctypes.byref(vx), ctypes.byref(vg), b, voxels, channels, groups, stats.data_ptr(),
-                                    gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag,
-                                    sums.data_ptr(), sums.shape[1], sums_c0, _stream())
-    _C.check(rc, "vdm_gn_silu_bwd_reduce")
+    _call("vdm_gn_silu_bwd_reduce", ctypes.byref(vx), ctypes.byref(vg), b, voxels, channels, groups, stats.data_ptr(),
+          gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag, sums.data_ptr(), sums.shape[1],
+          sums_c0, _stream())
     va = None
     if add is not None:
-        _planar_ok(add, "gn_silu_bwd add")
+        _planar_lanes(add, "gn_silu_bwd add", 8)
         va = ctypes.byref(_view(add, add_plane0))
-    rc = lib.vdm_gn_silu_bwd_apply(ctypes.byref(vx), ctypes.byref(vg), va, ctypes.byref(vo), b, voxels, channels, groups,
-                                   stats.data_ptr(), gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step),
-                                   layer_tag, sums.data_ptr(), sums.shape[1], sums_c0, _ptr(out_stats),
-                                   0 if out_stats is None else out_stats.shape[1], out_stats_c0, _stream())
-    _C.check(rc, "vdm_gn_silu_bwd_apply")
-    _launched(2)
+    _call("vdm_gn_silu_bwd_apply", ctypes.byref(vx), ctypes.byref(vg), va, ctypes.byref(vo), b, voxels, channels, groups,
+          stats.data_ptr(), gamma.data_ptr(), beta.data_ptr(), eps, dropout_p, seed, _ptr(seed_step), layer_tag,
+          sums.data_ptr(), sums.shape[1], sums_c0, _ptr(out_stats), 0 if out_stats is None else out_stats.shape[1],
+          out_stats_c0, _stream())
     return out, sums
 
 
 def avgpool2_bwd(dy: torch.Tensor, channels: int, dx: torch.Tensor, *, dy_plane0: int = 0, dx_plane0: int = 0,
                  accumulate: bool = False, stats: Optional[torch.Tensor] = None, stats_c0: int = 0) -> torch.Tensor:
     """dx[window] = (dx[window] if accumulate else 0) + upsample(dy)/8; dx is on the fine grid."""
-    _planar_ok(dy, "avgpool2_bwd dy")
-    _planar_ok(dx, "avgpool2_bwd dx")
+    _planar_lanes(dy, "avgpool2_bwd dy", 8)
+    _planar_lanes(dx, "avgpool2_bwd dx", 8)
     b, _, d, h, w, _ = dx.shape
     _need(tuple(dy.shape[2:5]) == (d // 2, h // 2, w // 2), "avgpool2_bwd: dy grid must be half the dx grid")
     vg, vx = _view(dy, dy_plane0), _view(dx, dx_plane0)
-    rc = _C.lib().vdm_avgpool2_bwd(ctypes.byref(vg), ctypes.byref(vx), b, d, h, w, channels, 1 if accumulate else 0,
-                                   _ptr(stats), 0 if stats is None else stats.shape[1], stats_c0, _stream())
-    _C.check(rc, "vdm_avgpool2_bwd")
-    _launched(1)
+    _call("vdm_avgpool2_bwd", ctypes.byref(vg), ctypes.byref(vx), b, d, h, w, channels, 1 if accumulate else 0, _ptr(stats),
+          0 if stats is None else stats.shape[1], stats_c0, _stream())
     return dx
 
 
 def upsample2_bwd(dy: torch.Tensor, channels: int, *, dy_plane0: int = 0, out: Optional[torch.Tensor] = None,
                   out_plane0: int = 0, stats: Optional[torch.Tensor] = None, stats_c0: int = 0) -> torch.Tensor:
     """dcoarse = sum over each 2x2x2 block of the fine gradient window dy."""
-    _planar_ok(dy, "upsample2_bwd dy")
+    _planar_lanes(dy, "upsample2_bwd dy", 8)
     b, _, d, h, w, _ = dy.shape
     if out is None:
         out = torch.empty((b, channels // 8, d // 2, h // 2, w // 2, 8), dtype=torch.bfloat16, device=dy.device)
-    _planar_ok(out, "upsample2_bwd out")
+    _planar_lanes(out, "upsample2_bwd out", 8)
     vg, vo = _view(dy, dy_plane0), _view(out, out_plane0)
-    rc = _C.lib().vdm_upsample2_bwd(ctypes.byref(vg), ctypes.byref(vo), b, d, h, w, channels, _ptr(stats),
-                                    0 if stats is None else stats.shape[1], stats_c0, _stream())
-    _C.check(rc, "vdm_upsample2_bwd")
-    _launched(1)
+    _call("vdm_upsample2_bwd", ctypes.byref(vg), ctypes.byref(vo), b, d, h, w, channels, _ptr(stats),
+          0 if stats is None else stats.shape[1], stats_c0, _stream())
     return out
 
 
@@ -744,10 +703,8 @@ def augment_crop(raw: torch.Tensor, crop, anchor, flip, perm, *, alpha: float = 
     _need(out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape[-3:]) == n and out.numel() == n[0] * n[1] * n[2],
           "augment_crop: out must be contiguous CUDA fp32 with the permuted crop shape")
     arr = lambda v: (ctypes.c_int32 * 3)(*v)
-    rc = _C.lib().vdm_augment_crop(raw.data_ptr(), out.data_ptr(), arr(raw.shape), arr(crop), arr(anchor), arr(flip), arr(perm),
-                                   alpha, mean, std, 1 if do_log else 0, _stream())
-    _C.check(rc, "vdm_augment_crop")
-    _launched(1)
+    _call("vdm_augment_crop", raw.data_ptr(), out.data_ptr(), arr(raw.shape), arr(crop), arr(anchor), arr(flip), arr(perm),
+          alpha, mean, std, 1 if do_log else 0, _stream())
     return out
 
 
@@ -758,9 +715,7 @@ def log_histogram(fields: torch.Tensor, lo: float, hi: float, nbins: int, add: f
           "log_histogram: fields must be contiguous CUDA fp32 (F, ...)")
     f = fields.shape[0]
     counts = torch.zeros((f, nbins), dtype=torch.int64, device=fields.device)
-    rc = _C.lib().vdm_log_histogram(fields.data_ptr(), f, fields.numel() // f, add, lo, hi, nbins, counts.data_ptr(), _stream())
-    _C.check(rc, "vdm_log_histogram")
-    _launched(1)
+    _call("vdm_log_histogram", fields.data_ptr(), f, fields.numel() // f, add, lo, hi, nbins, counts.data_ptr(), _stream())
     return counts
 
 
@@ -769,8 +724,7 @@ def sumsq(x: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     _need(x.is_cuda and x.dtype == torch.float32 and x.is_contiguous(), "sumsq: x must be contiguous CUDA fp32")
     if out is None:
         out = torch.zeros(1, dtype=torch.float64, device=x.device)
-    _C.check(_C.lib().vdm_sumsq(x.data_ptr(), x.numel(), out.data_ptr(), _stream()), "vdm_sumsq")
-    _launched(1)
+    _call("vdm_sumsq", x.data_ptr(), x.numel(), out.data_ptr(), _stream())
     return out
 
 
@@ -783,11 +737,8 @@ def adamw_step(param: torch.Tensor, grad: torch.Tensor, exp_avg: torch.Tensor, e
     for t in (param, grad, exp_avg, exp_avg_sq):
         _need(t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and t.numel() == param.numel(),
               "adamw_step: buckets must be contiguous CUDA fp32 of equal length")
-    rc = _C.lib().vdm_adamw_step_dev(param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(),
-                                     param.numel(), lr, beta1, beta2, eps, weight_decay, step, _ptr(step_ptr),
-                                     _ptr(grad_sumsq), max_norm, grad_scale, _stream())
-    _C.check(rc, "vdm_adamw_step")
-    _launched(1)
+    _call("vdm_adamw_step_dev", param.data_ptr(), grad.data_ptr(), exp_avg.data_ptr(), exp_avg_sq.data_ptr(), param.numel(),
+          lr, beta1, beta2, eps, weight_decay, step, _ptr(step_ptr), _ptr(grad_sumsq), max_norm, grad_scale, _stream())
 
 
 # ---- sampler ---------------------------------------------------------------------------------------
@@ -813,11 +764,8 @@ def sampler_step(z: torch.Tensor, eps_hat: torch.Tensor, coef: torch.Tensor, *, 
     if noise is not None:
         _need(noise.dtype == torch.float32 and noise.is_contiguous() and noise.numel() == z.numel(),
               "sampler_step: injected noise must be fp32 with z's shape")
-    rc = _C.lib().vdm_sampler_step(z.data_ptr(), eps_hat.data_ptr(), out.data_ptr(), b, voxels, coef.data_ptr(),
-                                   _ptr(step_ptr), seed, _ptr(realisation_id), draw_base, _ptr(noise), _ptr(cond),
-                                   n_cond, _ptr(packed_out), packed_planes, _stream())
-    _C.check(rc, "vdm_sampler_step")
-    _launched(1)
+    _call("vdm_sampler_step", z.data_ptr(), eps_hat.data_ptr(), out.data_ptr(), b, voxels, coef.data_ptr(), _ptr(step_ptr),
+          seed, _ptr(realisation_id), draw_base, _ptr(noise), _ptr(cond), n_cond, _ptr(packed_out), packed_planes, _stream())
     return out
 
 
@@ -825,15 +773,12 @@ def philox_normal(shape, seed: int, draw: int, realisation_id: Optional[torch.Te
                   device="cuda") -> torch.Tensor:
     out = torch.empty(shape, dtype=torch.float32, device=device)
     b = shape[0]
-    rc = _C.lib().vdm_philox_normal(out.data_ptr(), b, out.numel() // b, seed, _ptr(realisation_id), draw, _stream())
-    _C.check(rc, "vdm_philox_normal")
-    _launched(1)
+    _call("vdm_philox_normal", out.data_ptr(), b, out.numel() // b, seed, _ptr(realisation_id), draw, _stream())
     return out
 
 
 def increment(counter: torch.Tensor) -> None:
-    _C.check(_C.lib().vdm_increment(counter.data_ptr(), _stream()), "vdm_increment")
-    _launched(1)
+    _call("vdm_increment", counter.data_ptr(), _stream())
 
 
 # ---- P(k) --------------------------------------------------------------------------------------------
@@ -856,17 +801,14 @@ def pk_fields(fields: torch.Tensor, fields2: Optional[torch.Tensor] = None):
     if fields2 is not None:
         _need(fields2.shape == fields.shape and fields2.dtype == torch.float32 and fields2.is_contiguous(),
               "pk: fields2 must match fields")
-    lib = _C.lib()
-    nbytes = lib.vdm_pk_work_bytes(f, b, c, n0, n1, n2, 0 if fields2 is None else 1)
+    nbytes = _C.lib().vdm_pk_work_bytes(f, b, c, n0, n1, n2, 0 if fields2 is None else 1)
     work = torch.empty(nbytes, dtype=torch.uint8, device=fields.device)
     kmax = (min(n1, n2) if n0 == 1 else min(n0, n1, n2)) // 2
     k = torch.empty((f, kmax), dtype=torch.float64, device=fields.device)
     p = torch.empty_like(k)
     n = torch.empty((f, kmax), dtype=torch.int64, device=fields.device)
-    rc = lib.vdm_pk(fields.data_ptr(), _ptr(fields2), f, b, c, n0, n1, n2, work.data_ptr(), nbytes, k.data_ptr(),
-                    p.data_ptr(), n.data_ptr(), _stream())
-    _C.check(rc, "vdm_pk")
-    _launched(3)
+    _call("vdm_pk", fields.data_ptr(), _ptr(fields2), f, b, c, n0, n1, n2, work.data_ptr(), nbytes, k.data_ptr(), p.data_ptr(),
+          n.data_ptr(), _stream(), launches=3)
     return k, p, n
 
 
@@ -875,15 +817,12 @@ def pk_cross3(fields1: torch.Tensor, fields2: torch.Tensor):
     f, b, c, n0, n1, n2 = _pk_shape(fields1)
     _need(fields2.shape == fields1.shape and fields2.dtype == torch.float32 and fields2.is_contiguous() and
           fields2.is_cuda, "pk_cross3: fields2 must match fields1")
-    lib = _C.lib()
-    nbytes = lib.vdm_pk_work_bytes(f, b, c, n0, n1, n2, 1)
+    nbytes = _C.lib().vdm_pk_work_bytes(f, b, c, n0, n1, n2, 1)
     work = torch.empty(nbytes, dtype=torch.uint8, device=fields1.device)
     kmax = (min(n1, n2) if n0 == 1 else min(n0, n1, n2)) // 2
     k = torch.empty((f, kmax), dtype=torch.float64, device=fields1.device)
     p11, p22, p12 = torch.empty_like(k), torch.empty_like(k), torch.empty_like(k)
     n = torch.empty((f, kmax), dtype=torch.int64, device=fields1.device)
-    rc = lib.vdm_pk_cross3(fields1.data_ptr(), fields2.data_ptr(), f, b, c, n0, n1, n2, work.data_ptr(), nbytes,
-                           k.data_ptr(), p11.data_ptr(), p22.data_ptr(), p12.data_ptr(), n.data_ptr(), _stream())
-    _C.check(rc, "vdm_pk_cross3")
-    _launched(3)
+    _call("vdm_pk_cross3", fields1.data_ptr(), fields2.data_ptr(), f, b, c, n0, n1, n2, work.data_ptr(), nbytes, k.data_ptr(),
+          p11.data_ptr(), p22.data_ptr(), p12.data_ptr(), n.data_ptr(), _stream(), launches=3)
     return k, p11, p22, p12, n
