@@ -388,6 +388,18 @@ __device__ __forceinline__ uint4 gn_silu8(const uint4 x, const float (&ca)[8], c
   return pack8(f).u;
 }
 
+// (a, b) of 8 channels, stored interleaved [channel][a | b], into ca[8], cb[8]: from shared memory, or (LDG) from global
+// memory through the read-only path.
+template <bool LDG>
+__device__ __forceinline__ void load_coef8(const float* src, float (&ca)[8], float (&cb)[8]) {
+  const float4* cs = reinterpret_cast<const float4*>(src);
+#pragma unroll
+  for (int j4 = 0; j4 < 4; ++j4) {
+    const float4 c4 = LDG ? __ldg(cs + j4) : cs[j4];
+    ca[2 * j4] = c4.x; cb[2 * j4] = c4.y; ca[2 * j4 + 1] = c4.z; cb[2 * j4 + 1] = c4.w;
+  }
+}
+
 template <int MT, int KJ>
 __device__ __forceinline__ void transform_tiles(const ConvKernelParams& p, ConvShared* sh, uint8_t* a_smem, float* coef) {
   constexpr int planes = 2 * KJ;
@@ -435,14 +447,7 @@ __device__ __forceinline__ void transform_tiles(const ConvKernelParams& p, ConvS
 #pragma unroll 1
         for (int pl = pl0; pl < planes; pl += pl_step) {
           float ca[8], cb[8];
-          {
-            const float4* cs = reinterpret_cast<const float4*>(coef + (size_t)((kc * planes + pl) * 8) * 2);
-#pragma unroll
-            for (int j4 = 0; j4 < 4; ++j4) {
-              const float4 c4 = cs[j4];
-              ca[2 * j4] = c4.x; cb[2 * j4] = c4.y; ca[2 * j4 + 1] = c4.z; cb[2 * j4 + 1] = c4.w;
-            }
-          }
+          load_coef8<false>(coef + (size_t)((kc * planes + pl) * 8) * 2, ca, cb);
           uint4* base = reinterpret_cast<uint4*>(stage + (size_t)pl * p.plane_bytes);
           // Software pipeline, kXfGroup units per group, the NEXT group's loads in flight while this one is computed:
           // while the tensor core streams its operands out of the same shared memory (the N = 96 MMAs of the narrow layers
@@ -501,6 +506,133 @@ constexpr int kEpiRes = 1, kEpiStats = 2, kEpiFp32 = 4;
 // residual is read in the same layout, and the statistics are those of the stored, un-rounded fp32 values.
 constexpr int kEpiF32Planar = 8;
 
+// Bias + conditioning rows of the launch, [B][c_out] (the sampler step's rows when they vary per step), or null.
+__device__ __forceinline__ const float* cadd_rows(const ConvKernelParams& p) {
+  const long long cadd_step = (p.chan_add && p.step_ptr) ? (long long)(*p.step_ptr) : 0ll;
+  return p.chan_add ? p.chan_add + cadd_step * p.chan_add_step_stride : nullptr;
+}
+
+__device__ __forceinline__ void load_row16(const float* src, float (&v)[16]) {
+  const float4* cs = reinterpret_cast<const float4*>(src);
+#pragma unroll
+  for (int j4 = 0; j4 < 4; ++j4) {
+    const float4 cv = cs[j4];
+    v[4 * j4] = cv.x; v[4 * j4 + 1] = cv.y; v[4 * j4 + 2] = cv.z; v[4 * j4 + 3] = cv.w;
+  }
+}
+
+// The pieces below are macros, not functions: nvcc optimises a __forceinline__ function on its own before it inlines it, and
+// written as functions they changed the code of most conv kernels (address arithmetic, loop bounds and branches moved).
+// Expanded in place, every expression stays where the caller's code had it and both schedules compile as before.
+
+// Bias + conditioning rows of every sample (cadd_g: cadd_rows) -> shared-memory table dst[rows][cols], zeros past c_out and
+// without rows, so that the unit code has no "is there a bias" branch; filled by the kThreads epilogue threads (et = 0 ..
+// kThreads - 1), which then meet at named barrier 1.
+#define VDM_CADD_TABLE_FILL(dst, cadd_g, rows, cols, c_out, et, kThreads)                                                    \
+  {                                                                                                                         \
+    for (int i_ = (et); i_ < (rows) * (cols); i_ += (kThreads)) {                                                          \
+      const int bb_ = i_ / (cols), c_ = i_ - bb_ * (cols);                                                                  \
+      (dst)[i_] = ((cadd_g) && c_ < (c_out)) ? __ldg((cadd_g) + (long long)bb_ * (c_out) + c_) : 0.f;                      \
+    }                                                                                                                       \
+    asm volatile("bar.sync 1, %0;" ::"n"(kThreads) : "memory");                                                           \
+  }
+
+// fp32 NCDHW output (conv_out): the first c_left channels of the 16-channel unit f, V (one channel) apart from yp on.
+#define VDM_STORE_FP32_NCDHW(yp, f, c_left, V)                                                                              \
+  {                                                                                                                         \
+    float* yp_ = (yp);                                                                                                      \
+    _Pragma("unroll") for (int j_ = 0; j_ < 16; ++j_) if (j_ < (c_left)) yp_[(long long)j_ * (V)] = (f)[j_];                \
+  }
+
+// Half h (channels 8h .. 8h + 7) of the 16-channel unit f of planar output: + residual, store, per-lane statistics
+// s1[8h + j] += y, s2[8h + j] += y^2 of the STORED values (for bf16 output: after rounding).  bf16 planes: residual r0, one
+// store at y_out[off].  fp32 planes: residual r0, r1, stores at y_out[off0], y_out[off1].  RES, STATS: compile-time flags.
+#define VDM_HALF_STATS(g, h, s1, s2)                                                                                        \
+  {                                                                                                                         \
+    _Pragma("unroll") for (int j_ = 0; j_ < 8; j_ += 2) {                                                                   \
+      add2((s1)[(h) * 8 + j_], (s1)[(h) * 8 + j_ + 1], (g)[j_], (g)[j_ + 1]);                                               \
+      fma2_sq((s2)[(h) * 8 + j_], (s2)[(h) * 8 + j_ + 1], (g)[j_], (g)[j_ + 1]);                                            \
+    }                                                                                                                       \
+  }
+#define VDM_STORE_HALF_BF16(RES, STATS, f, h, r0, y_out, off, s1, s2)                                                       \
+  {                                                                                                                         \
+    float g_[8];                                                                                                            \
+    _Pragma("unroll") for (int j_ = 0; j_ < 8; ++j_) g_[j_] = (f)[(h) * 8 + j_];                                            \
+    if (RES) {                                                                                                              \
+      float rr_[8];                                                                                                         \
+      bf16x8 rv_;                                                                                                           \
+      rv_.u = (r0);                                                                                                         \
+      unpack8(rv_, rr_);                                                                                                    \
+      _Pragma("unroll") for (int j_ = 0; j_ < 8; j_ += 2) add2(g_[j_], g_[j_ + 1], rr_[j_], rr_[j_ + 1]);                   \
+    }                                                                                                                       \
+    const bf16x8 packed_ = pack8(g_);                                                                                       \
+    (y_out)[off] = packed_;                                                                                                 \
+    if (STATS) {                                                                                                            \
+      unpack8(packed_, g_);                                                                                                 \
+      VDM_HALF_STATS(g_, h, s1, s2);                                                                                        \
+    }                                                                                                                       \
+  }
+#define VDM_STORE_HALF_F32P(RES, STATS, f, h, r0, r1, y_out, off0, off1, s1, s2)                                            \
+  {                                                                                                                         \
+    float g_[8];                                                                                                            \
+    _Pragma("unroll") for (int j_ = 0; j_ < 8; ++j_) g_[j_] = (f)[(h) * 8 + j_];                                            \
+    if (RES) {                                                                                                              \
+      const uint4 ra_ = (r0), rb_ = (r1);                                                                                   \
+      add2(g_[0], g_[1], __uint_as_float(ra_.x), __uint_as_float(ra_.y));                                                   \
+      add2(g_[2], g_[3], __uint_as_float(ra_.z), __uint_as_float(ra_.w));                                                   \
+      add2(g_[4], g_[5], __uint_as_float(rb_.x), __uint_as_float(rb_.y));                                                   \
+      add2(g_[6], g_[7], __uint_as_float(rb_.z), __uint_as_float(rb_.w));                                                   \
+    }                                                                                                                       \
+    (y_out)[off0] = make_float4(g_[0], g_[1], g_[2], g_[3]);                                                                \
+    (y_out)[off1] = make_float4(g_[4], g_[5], g_[6], g_[7]);                                                                \
+    if (STATS) VDM_HALF_STATS(g_, h, s1, s2);                                                                               \
+  }
+
+// Per-lane statistics s1, s2 of a 16-channel chunk (channels c0 .. c0 + 15 of the CTA) -> this warp's slots: one transpose
+// reduction, then part[ew][c] = sum, part[kSlotWarps + ew][c] = sum of squares (rows of `cols` channels).
+#define VDM_STATS_TO_SLOTS(s1, s2, part, ew, cols, c0, kSlotWarps, lane)                                                     \
+  {                                                                                                                         \
+    warp_column_sums16(s1);                                                                                                 \
+    warp_column_sums16(s2);                                                                                                 \
+    if (((lane) & 1) == 0) {                                                                                                \
+      const int c_ = (c0) + ((lane) >> 1);                                                                                  \
+      (part)[(ew) * (cols) + c_] = (s1)[0];                                                                                 \
+      (part)[((kSlotWarps) + (ew)) * (cols) + c_] = (s2)[0];                                                                \
+    }                                                                                                                       \
+  }
+
+// Channel c of the CTA: the slots of its kWarps warps, summed in a fixed order (statistics do not depend on timing), into the
+// fp64 running sums acc[c], acc[cols + c]; on `flush` (the CTA moves on to another sample or channel slice, or ends) those go
+// to the (sum, sumsq) of (sample b, channel cbase + c) with fp64 atomics -- never for padded channels -- and restart.
+// kZeroSlots: the slots are cleared as they are read, for a caller whose warps do not write every slot of every round.
+#define VDM_FOLD_STATS(p, part, acc, cols, c, kWarps, kSlotWarps, kZeroSlots, flush, b, cbase)                              \
+  {                                                                                                                         \
+    const int c_ = (c);                                                                                                     \
+    float t1_ = 0.f, t2_ = 0.f;                                                                                             \
+    _Pragma("unroll") for (int wv_ = 0; wv_ < (kWarps); ++wv_) {                                                            \
+      t1_ += (part)[wv_ * (cols) + c_];                                                                                     \
+      t2_ += (part)[((kSlotWarps) + wv_) * (cols) + c_];                                                                    \
+      if (kZeroSlots) {                                                                                                     \
+        (part)[wv_ * (cols) + c_] = 0.f;                                                                                    \
+        (part)[((kSlotWarps) + wv_) * (cols) + c_] = 0.f;                                                                   \
+      }                                                                                                                     \
+    }                                                                                                                       \
+    const double a1_ = (acc)[c_] + (double)t1_;                                                                             \
+    const double a2_ = (acc)[(cols) + c_] + (double)t2_;                                                                    \
+    if (flush) {                                                                                                            \
+      if ((cbase) + c_ < (p).c_out) {                                                                                       \
+        double* dst_ = (p).stats + ((long long)(b) * (p).stats_channels + (p).stats_c0 + (cbase) + c_) * 2;                 \
+        atomicAdd(dst_, a1_);                                                                                               \
+        atomicAdd(dst_ + 1, a2_);                                                                                           \
+      }                                                                                                                     \
+      (acc)[c_] = 0.0;                                                                                                      \
+      (acc)[(cols) + c_] = 0.0;                                                                                             \
+    } else {                                                                                                                \
+      (acc)[c_] = a1_;                                                                                                      \
+      (acc)[(cols) + c_] = a2_;                                                                                             \
+    }                                                                                                                       \
+  }
+
 template <int MT, int MODE>
 __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvShared* sh, uint8_t* smem, float* stat_part,
                                                double* stat_acc, const uint32_t tmem_base) {
@@ -526,15 +658,8 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
   // A launch without rows gets zeros, so that the unit code has no "is there a bias" branch.
   float* cadd_tab = &sh->cadd[0][0];
   const bool cadd_table = p.B * p.n_pad <= 512;
-  const long long cadd_step = (p.chan_add && p.step_ptr) ? (long long)(*p.step_ptr) : 0ll;
-  const float* cadd_g = p.chan_add ? p.chan_add + cadd_step * p.chan_add_step_stride : nullptr;
-  if (cadd_table) {
-    for (int i = et; i < p.B * p.n_pad; i += kEpiThreads) {
-      const int bb = i / p.n_pad, c = i - bb * p.n_pad;
-      cadd_tab[i] = (cadd_g && c < p.c_out) ? __ldg(cadd_g + (long long)bb * p.c_out + c) : 0.f;
-    }
-    asm volatile("bar.sync 1, 256;" ::: "memory");
-  }
+  const float* cadd_g = cadd_rows(p);
+  if (cadd_table) VDM_CADD_TABLE_FILL(cadd_tab, cadd_g, p.B, p.n_pad, p.c_out, et, kEpiThreads);
   // Residual prefetch ring in SHARED memory.  The residual does not depend on the accumulator, and a dependent
   // 16-byte global load per (unit, half) cost ~700 cycles each (r01f: 0.44 -> 0.76 ms on the 32->32 level-0 conv).
   // This warp consumes its units in a fixed order; p.res_depth of them are always in flight as cp.async copies
@@ -644,22 +769,15 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
       const int c_left = p.c_out - c0;
       const int nhf = c_left >= 16 ? 2 : (c_left >= 8 ? 1 : 0);
       float cb[16];                              // bias + conditioning row of this chunk, for all slices of the tile
-      {
-        const float4* cs = reinterpret_cast<const float4*>(cadd_row + ch * 16);
-#pragma unroll
-        for (int j4 = 0; j4 < 4; ++j4) {
-          const float4 cv = cs[j4];
-          cb[4 * j4] = cv.x; cb[4 * j4 + 1] = cv.y; cb[4 * j4 + 2] = cv.z; cb[4 * j4 + 3] = cv.w;
-        }
-      }
+      load_row16(cadd_row + ch * 16, cb);
       float s1[16], s2[16];                      // per-lane statistics of this chunk over the warp's slices
       if (STATS) {
 #pragma unroll
         for (int j = 0; j < 16; ++j) s1[j] = s2[j] = 0.f;
       }
-      bf16x8* y_ch = reinterpret_cast<bf16x8*>(p.y) + ((long long)t.b * p.y_planes + p.y_plane0 + (c0 >> 3)) * V + vox0;
+      typename Unit<F32P>::T* y_ch = reinterpret_cast<typename Unit<F32P>::T*>(p.y) +
+                                     ((long long)t.b * p.y_planes + p.y_plane0 + (c0 >> kPlaneShift)) * V + vox0;
       float* y32_ch = static_cast<float*>(p.y) + ((long long)t.b * p.c_out + c0) * V + vox0;
-      float4* y4_ch = static_cast<float4*>(p.y) + ((long long)t.b * p.y_planes + p.y_plane0 + (c0 >> 2)) * V + vox0;
       auto process = [&](uint32_t (&raw)[16], int s) __attribute__((always_inline)) {
         const bool valid = hw_ok && (t.d0 + s < p.D);
         uint4 rcur0 = make_uint4(0, 0, 0, 0), rcur1 = make_uint4(0, 0, 0, 0);
@@ -680,66 +798,19 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
           add2(f[j], f[j + 1], cb[j], cb[j + 1]);
         }
         if (FP32) {
-          if (valid) {
-            float* yp = y32_ch + (long long)s * HW;
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (j < c_left) yp[(long long)j * V] = f[j];
-          }
+          if (valid) VDM_STORE_FP32_NCDHW(y32_ch + (long long)s * HW, f, c_left, V);
           return;
         }
         if (nhf == 0 || !valid) return;          // padded output channels (warp-uniform) / voxels beyond the grid
-        if (F32P) {
-          float4* yp = y4_ch + (long long)s * HW;
-#pragma unroll
-          for (int hf = 0; hf < 2; ++hf) {
-            if (hf == 1 && nhf < 2) break;
-            float g[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) g[j] = f[hf * 8 + j];
-            if (RES) {
-              const uint4 ra = hf == 0 ? rcur0 : rcur2, rb = hf == 0 ? rcur1 : rcur3;
-              add2(g[0], g[1], __uint_as_float(ra.x), __uint_as_float(ra.y));
-              add2(g[2], g[3], __uint_as_float(ra.z), __uint_as_float(ra.w));
-              add2(g[4], g[5], __uint_as_float(rb.x), __uint_as_float(rb.y));
-              add2(g[6], g[7], __uint_as_float(rb.z), __uint_as_float(rb.w));
-            }
-            yp[(long long)(2 * hf) * V] = make_float4(g[0], g[1], g[2], g[3]);
-            yp[(long long)(2 * hf + 1) * V] = make_float4(g[4], g[5], g[6], g[7]);
-            if (STATS) {
-#pragma unroll
-              for (int j = 0; j < 8; j += 2) {
-                add2(s1[hf * 8 + j], s1[hf * 8 + j + 1], g[j], g[j + 1]);
-                fma2_sq(s2[hf * 8 + j], s2[hf * 8 + j + 1], g[j], g[j + 1]);
-              }
-            }
-          }
-          return;
-        }
-        bf16x8* yp = y_ch + (long long)s * HW;
+        typename Unit<F32P>::T* yp = y_ch + (long long)s * HW;
 #pragma unroll
         for (int hf = 0; hf < 2; ++hf) {
           if (hf == 1 && nhf < 2) break;
-          float g[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) g[j] = f[hf * 8 + j];
-          if (RES) {
-            float rr[8];
-            bf16x8 rv;
-            rv.u = hf == 0 ? rcur0 : rcur1;
-            unpack8(rv, rr);
-#pragma unroll
-            for (int j = 0; j < 8; j += 2) add2(g[j], g[j + 1], rr[j], rr[j + 1]);
-          }
-          const bf16x8 packed = pack8(g);
-          yp[hf == 0 ? 0 : V] = packed;
-          if (STATS) {
-            unpack8(packed, g);                  // statistics describe the stored (rounded) tensor
-#pragma unroll
-            for (int j = 0; j < 8; j += 2) {
-              add2(s1[hf * 8 + j], s1[hf * 8 + j + 1], g[j], g[j + 1]);
-              fma2_sq(s2[hf * 8 + j], s2[hf * 8 + j + 1], g[j], g[j + 1]);
-            }
+          if constexpr (F32P) {
+            VDM_STORE_HALF_F32P(RES, STATS, f, hf, hf == 0 ? rcur0 : rcur2, hf == 0 ? rcur1 : rcur3, yp, (long long)(2 * hf) * V,
+                                (long long)(2 * hf + 1) * V, s1, s2);
+          } else {
+            VDM_STORE_HALF_BF16(RES, STATS, f, hf, hf == 0 ? rcur0 : rcur1, yp, hf == 0 ? 0 : V, s1, s2);
           }
         }
       };
@@ -769,17 +840,8 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
         else process(raw_b, s);
         s = sn;
       }
-      if (STATS && nhf > 0) {
-        // one transpose-reduction per chunk and tile (r01j: per (slice, chunk) it cost 0.22 -> 0.30 ms on 32->32)
-        warp_column_sums16(s1);
-        warp_column_sums16(s2);
-        if ((lane & 1) == 0) {
-          // one slot per (warp, channel), summed in a fixed order below: statistics do not depend on timing
-          const int c = ch * 16 + (lane >> 1);
-          sp[ew * n_cta + c] = s1[0];
-          sp[(8 + ew) * n_cta + c] = s2[0];
-        }
-      }
+      // one transpose-reduction per chunk and tile (r01j: per (slice, chunk) it cost 0.22 -> 0.30 ms on 32->32)
+      if (STATS && nhf > 0) VDM_STATS_TO_SLOTS(s1, s2, sp, ew, n_cta, ch * 16, 8, lane);
     }
     if (!released) {
       ptx::tc_fence_before();
@@ -799,29 +861,8 @@ __device__ __forceinline__ void epilogue_tiles(const ConvKernelParams& p, ConvSh
           const TileCoord tn = decode_tile(p, next_tile);
           flush = (tn.b != t.b) || (tn.ns != t.ns);
         }
-        const int c = et;
-        float t1 = 0.f, t2 = 0.f;
-#pragma unroll
-        for (int wv = 0; wv < 8; ++wv) {
-          t1 += sp[wv * n_cta + c];
-          t2 += sp[(8 + wv) * n_cta + c];
-          sp[wv * n_cta + c] = 0.f;
-          sp[(8 + wv) * n_cta + c] = 0.f;
-        }
-        const double a1 = stat_acc[c] + (double)t1;
-        const double a2 = stat_acc[n_cta + c] + (double)t2;
-        if (flush) {
-          if (cbase + c < p.c_out) {
-            double* dst = p.stats + ((long long)t.b * p.stats_channels + p.stats_c0 + cbase + c) * 2;
-            atomicAdd(dst, a1);
-            atomicAdd(dst + 1, a2);
-          }
-          stat_acc[c] = 0.0;
-          stat_acc[n_cta + c] = 0.0;
-        } else {
-          stat_acc[c] = a1;
-          stat_acc[n_cta + c] = a2;
-        }
+        // a warp writes the slots of its own chunks only (split by chunk, padded chunks skipped): clear them as they are read
+        VDM_FOLD_STATS(p, sp, stat_acc, n_cta, et, 8, 8, true, flush, t.b, cbase);
       }
     }
   }
@@ -906,6 +947,13 @@ __device__ __forceinline__ void issue_generic_tiles(const ConvKernelParams& p, C
   }
 }
 
+// The dynamic shared-memory window of a conv kernel, rounded up to 1024 bytes by POINTER ARITHMETIC on the __shared__ array:
+// a round trip through uintptr_t made nvcc lose the address space, and every access through the shared structures and the
+// residual ring compiled to generic LD / ST (R2b ncu: LD.E.128 for the bias rows and the ring slots in the epilogue's inner loop).
+__device__ __forceinline__ uint8_t* smem_window_1024(uint8_t* smem_raw) {
+  return smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
+}
+
 // MT = d-slices (accumulators) per tile, KJ = K=16 MMAs per channel chunk (KC = 16*KJ), NF = 0 for the generic
 // path or Cout_pad for the kd-folded path: compile-time so that the MMA issue loops are straight lines of
 // tcgen05.mma with immediate offsets (r01a: a generic loop cost ~240 issue cycles per MMA).
@@ -920,10 +968,7 @@ conv3d_planar_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_co
   static_assert(!TF32 || NF == 0, "the TF32 instances run the generic schedule only");
   constexpr ptx::MmaKind kKind = TF32 ? ptx::MmaKind::kTF32 : ptx::MmaKind::kF16;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  // Round the window up to 1024 bytes by POINTER ARITHMETIC on the __shared__ array: a round trip through uintptr_t
-  // made nvcc lose the address space, and every access through `sh` / the residual ring compiled to generic LD / ST
-  // (R2b ncu: LD.E.128 for the bias rows and the ring slots in the epilogue's inner loop).
-  uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_window_1024(smem_raw);
   uint8_t* a_smem = smem;
   uint8_t* b_smem = smem + (size_t)p.nsa * p.a_stage_bytes;
   ConvShared* sh = reinterpret_cast<ConvShared*>(b_smem + (size_t)p.nsb * p.b_stage_bytes + p.skip_w_bytes);

@@ -114,16 +114,9 @@ __device__ __forceinline__ void march_epilogue(const ConvKernelParams& p, MarchS
   const int r = q * 32 + lane;
   const int lh = r >> 3, lw = r & 7;
   const long long HW = (long long)p.H * p.W, V = (long long)p.D * HW;
-  const long long cadd_step = (p.chan_add && p.step_ptr) ? (long long)(*p.step_ptr) : 0ll;
-  const float* cadd_g = p.chan_add ? p.chan_add + cadd_step * p.chan_add_step_stride : nullptr;
+  const float* cadd_g = cadd_rows(p);
   const bool cadd_table = p.B * NF <= kMarchCaddMax;
-  if (cadd_table) {
-    for (int i = et; i < p.B * NF; i += kThreadsE) {
-      const int bb = i / NF, c = i - bb * NF;
-      cadd_s[i] = (cadd_g && c < p.c_out) ? __ldg(cadd_g + (long long)bb * p.c_out + c) : 0.f;
-    }
-    asm volatile("bar.sync 1, %0;" ::"n"(kThreadsE) : "memory");
-  }
+  if (cadd_table) VDM_CADD_TABLE_FILL(cadd_s, cadd_g, p.B, NF, p.c_out, et, kThreadsE);
   // valid 8-channel planes (bf16 output: c_out % 8 == 0)
   const int n_valid_planes = (p.c_out >> 3) < n_planes ? (p.c_out >> 3) : n_planes;
   // residual ring: slot i, plane pl of this thread: r_ring[(i * n_planes + pl) * kMEpiThreads]
@@ -205,12 +198,7 @@ __device__ __forceinline__ void march_epilogue(const ConvKernelParams& p, MarchS
       for (int c = 0; c < n_chunks; ++c) {
         float f[16];
         if (cadd_table) {
-          const float4* cs = reinterpret_cast<const float4*>(cadd_row + c * 16);
-#pragma unroll
-          for (int j4 = 0; j4 < 4; ++j4) {
-            const float4 cv = cs[j4];
-            f[4 * j4] = cv.x; f[4 * j4 + 1] = cv.y; f[4 * j4 + 2] = cv.z; f[4 * j4 + 3] = cv.w;
-          }
+          load_row16(cadd_row + c * 16, f);
         } else {
 #pragma unroll
           for (int j = 0; j < 16; ++j)
@@ -219,39 +207,14 @@ __device__ __forceinline__ void march_epilogue(const ConvKernelParams& p, MarchS
 #pragma unroll
         for (int j = 0; j < 16; j += 2) add2(f[j], f[j + 1], __uint_as_float(raw[c][j]), __uint_as_float(raw[c][j + 1]));
         if (FP32) {
-          if (hw_ok) {
-            float* yp = y32_b + (long long)(c * 16) * V + (long long)s * HW;
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (c * 16 + j < p.c_out) yp[(long long)j * V] = f[j];
-          }
+          if (hw_ok) VDM_STORE_FP32_NCDHW(y32_b + (long long)(c * 16) * V + (long long)s * HW, f, p.c_out - c * 16, V);
           continue;
         }
 #pragma unroll
         for (int hf = 0; hf < 2; ++hf) {
           const int pl = c * 2 + hf;
           if (pl >= n_valid_planes || !hw_ok) continue;
-          float gv[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) gv[j] = f[hf * 8 + j];
-          if (RES) {
-            float rr[8];
-            bf16x8 rv;
-            rv.u = slot[pl * kMEpiThreads];
-            unpack8(rv, rr);
-#pragma unroll
-            for (int j = 0; j < 8; j += 2) add2(gv[j], gv[j + 1], rr[j], rr[j + 1]);
-          }
-          const bf16x8 packed = pack8(gv);
-          y_b[(long long)pl * V + (long long)s * HW] = packed;
-          if (STATS) {
-            unpack8(packed, gv);                  // statistics describe the stored (rounded) tensor
-#pragma unroll
-            for (int j = 0; j < 8; j += 2) {
-              add2(s1[c][hf * 8 + j], s1[c][hf * 8 + j + 1], gv[j], gv[j + 1]);
-              fma2_sq(s2[c][hf * 8 + j], s2[c][hf * 8 + j + 1], gv[j], gv[j + 1]);
-            }
-          }
+          VDM_STORE_HALF_BF16(RES, STATS, f, hf, slot[pl * kMEpiThreads], y_b, (long long)pl * V + (long long)s * HW, s1[c], s2[c]);
         }
       }
       if (RES) {
@@ -262,41 +225,13 @@ __device__ __forceinline__ void march_epilogue(const ConvKernelParams& p, MarchS
     ob += (uint32_t)m.len;
     if (STATS) {
 #pragma unroll
-      for (int c = 0; c < n_chunks; ++c) {
-        warp_column_sums16(s1[c]);
-        warp_column_sums16(s2[c]);
-        if ((lane & 1) == 0) {
-          const int ch = c * 16 + (lane >> 1);
-          stat_part[ew * NF + ch] = s1[c][0];
-          stat_part[(kMEpiWarps + ew) * NF + ch] = s2[c][0];
-        }
-      }
+      for (int c = 0; c < n_chunks; ++c) VDM_STATS_TO_SLOTS(s1[c], s2[c], stat_part, ew, NF, c * 16, kMEpiWarps, lane);
       asm volatile("bar.sync 2, %0;" ::"n"(kThreadsE) : "memory");
       if (et < NF) {
         const int next_u = u + (int)gridDim.x;
         bool flush = next_u >= p.m_units;
         if (!flush) flush = decode_unit(p, next_u).b != m.b;
-        const int c = et;
-        float t1 = 0.f, t2 = 0.f;
-#pragma unroll
-        for (int wv = 0; wv < 4 * EW; ++wv) {
-          t1 += stat_part[wv * NF + c];
-          t2 += stat_part[(kMEpiWarps + wv) * NF + c];
-        }
-        const double a1 = stat_acc[c] + (double)t1;
-        const double a2 = stat_acc[NF + c] + (double)t2;
-        if (flush) {
-          if (c < p.c_out) {
-            double* dst = p.stats + ((long long)m.b * p.stats_channels + p.stats_c0 + c) * 2;
-            atomicAdd(dst, a1);
-            atomicAdd(dst + 1, a2);
-          }
-          stat_acc[c] = 0.0;
-          stat_acc[NF + c] = 0.0;
-        } else {
-          stat_acc[c] = a1;
-          stat_acc[NF + c] = a2;
-        }
+        VDM_FOLD_STATS(p, stat_part, stat_acc, NF, et, 4 * EW, kMEpiWarps, false, flush, m.b, 0);
       }
       asm volatile("bar.sync 2, %0;" ::"n"(kThreadsE) : "memory");     // the slots are read before the next unit overwrites them
     }
@@ -310,8 +245,12 @@ __device__ __forceinline__ void march_epilogue(const ConvKernelParams& p, MarchS
 // tensor WHOLE (so its wait -> LDS -> arithmetic -> STS chain may last four slices: in the tile kernel four warps shared every
 // stage and the chain, not the bandwidth, made the transform slower than the MMAs, R2h); a lane owns one 8-channel plane,
 // its 16 coefficients stay in registers while the sample does not change.  Skip-tensor stages are not transformed.
-// NXW = number of transform warps (the last NXW warps of the CTA): 4, or 8 for conv_out (see the role dispatch in the kernel:
-// a warp may not skip a whole phase of a barrier it waits on, which rules NXW = 8 out when skip-tensor stages are interleaved).
+// Hand-off with skip-tensor stages interleaved (that of the tile kernel's transform_tiles): EVERY warp waits for EVERY stage
+// in order, main and skip alike, and arrives on a_ready[s] (count NXW) when it is done with it -- the owner after its
+// transform and fence, the others right away.  No stage can be consumed, and so refilled, before all NXW warps have arrived,
+// so no warp can fall two phases behind a barrier it waits on by parity.  Without skip stages all phases of a stage belong to
+// its owner (stages j, j + NXW, ...), and the owner alone waits and arrives (count 1): there the all-warp form cost conv_out
+// 5 % and the fused 32->32 convs 3 %.  NXW = number of transform warps (the last NXW warps of the CTA): 4, or 8 for conv_out.
 template <int KJ, bool SKIP, int NXW>
 __device__ __forceinline__ void march_transform(const ConvKernelParams& p, MarchShared* sh, uint8_t* a_smem) {
   constexpr int planes = 2 * KJ, S = kMarchStages;
@@ -327,17 +266,12 @@ __device__ __forceinline__ void march_transform(const ConvKernelParams& p, March
   const int skip_chunks = SKIP ? p.skip_chunks : 0;
   float ca[8], cb[8];
   int cur_b = -1;
-  uint32_t it = 0, n_main = 0, n_skip = 0;                 // stage counter (all stages), main / skip-tensor stages so far
+  uint32_t it = 0, n_main = 0;                             // stage counter (all stages), main-tensor stages so far
   for (int u = blockIdx.x; u < p.m_units; u += gridDim.x) {
     const MarchUnit m = decode_unit(p, u);
     if (m.b != cur_b) {
       cur_b = m.b;
-      const float4* cs = reinterpret_cast<const float4*>(p.in_norm + ((long long)m.b * p.c_in + pl * 8) * 2);
-#pragma unroll
-      for (int j4 = 0; j4 < 4; ++j4) {
-        const float4 c4 = __ldg(cs + j4);
-        ca[2 * j4] = c4.x; cb[2 * j4] = c4.y; ca[2 * j4 + 1] = c4.z; cb[2 * j4 + 1] = c4.w;
-      }
+      load_coef8<true>(p.in_norm + ((long long)m.b * p.c_in + pl * 8) * 2, ca, cb);
     }
     // voxels of this lane that lie outside the grid in h / w (zero padding applies AFTER the non-linearity): bit k = voxel
     // l0 + k * lpp of the (kTileH + 2) x (kTileW + 2) halo slice, the same for every slice of the unit
@@ -350,11 +284,13 @@ __device__ __forceinline__ void march_transform(const ConvKernelParams& p, March
       }
     }
     for (int i = 0; i < m.len + 2; ++i, ++n_main) {
-      if ((int)(n_main % (uint32_t)NXW) == j) {
+      const bool own = (int)(n_main % (uint32_t)NXW) == j;
+      if (SKIP || own) {
         const uint32_t s = it % (uint32_t)S;
         ptx::mbar_wait(&sh->a_full[s], (it / (uint32_t)S) & 1);
         const int dz = m.d0 - 1 + i;
-        if (dz >= 0 && dz < p.D) {                         // (a slice beyond the grid is all zero padding: nothing to do)
+        // the owner transforms the slice (one beyond the grid is all zero padding: nothing to do)
+        if (own && dz >= 0 && dz < p.D) {
           uint4* base = reinterpret_cast<uint4*>(a_smem + (size_t)s * kStageBytes + (size_t)pl * kSliceBytes);
           // BRANCH-FREE body: G independent 16-byte chains per lane that ptxas can interleave (R5g: with a guard and an edge
           // branch around every voxel the chains ran one after another at ~4.5 cycles per instruction and the four transform
@@ -379,17 +315,13 @@ __device__ __forceinline__ void march_transform(const ConvKernelParams& p, March
         if (lane == 0) ptx::mbar_arrive(&sh->a_ready[s]);
       }
       ++it;
-      // the skip-tensor stages of this output slice are not transformed, but a_ready has to complete one phase per use of a
-      // stage like a_full does (the issuer waits on a_ready for every stage): forward the arrival.
-      // (With skip stages interleaved, consecutive phases of a stage's a_full belong to different warps; the parity waits here
-      // rely on loads issued >= 3 stages apart landing in order -- see DESIGN.md 3.10a, "known weakness", for the sound form.)
+      // the skip-tensor stages of this output slice are not transformed: every warp waits for them and arrives all the same
       if (i < m.len) {
-        for (int c = 0; c < skip_chunks; ++c, ++it, ++n_skip) {
-          if ((int)(n_skip % (uint32_t)NXW) == j) {
-            const uint32_t s = it % (uint32_t)S;
-            ptx::mbar_wait(&sh->a_full[s], (it / (uint32_t)S) & 1);
-            if (lane == 0) ptx::mbar_arrive(&sh->a_ready[s]);
-          }
+        for (int c = 0; c < skip_chunks; ++c, ++it) {
+          const uint32_t s = it % (uint32_t)S;
+          ptx::mbar_wait(&sh->a_full[s], (it / (uint32_t)S) & 1);
+          __syncwarp();
+          if (lane == 0) ptx::mbar_arrive(&sh->a_ready[s]);
         }
       }
     }
@@ -401,7 +333,7 @@ __global__ void __launch_bounds__(kConvThreads, 1)
 conv3d_march_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_x2,
                     const __grid_constant__ ConvKernelParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_window_1024(smem_raw);
   constexpr int planes = 2 * KJ;
   constexpr int kSliceBytes = (kTileH + 2) * (kTileW + 2) * 16;        // one plane of one input slice
   constexpr int kStageBytes = planes * kSliceBytes;
@@ -414,6 +346,15 @@ conv3d_march_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
   double* stat_acc = reinterpret_cast<double*>(stat_part + 2 * kMEpiWarps * NF);   // [sum | sumsq][channel]: this sample so far
   float* cadd_s = reinterpret_cast<float*>(stat_acc + 2 * NF);         // [B][NF] bias + conditioning rows
 
+  // conv_out (16 output columns, one fp32 channel stored): the epilogue is a few instructions per voxel and the layer is
+  // bound by the input transform (R5i: 26 % tensor-pipe activity, transform warps busy ~90 %), so eight warps transform
+  // and four drain.  Only without the fused skip conv, whose 32-column epilogues (bias + residual + statistics) need their
+  // eight warps.
+  constexpr bool kWideXf = XF && !SKIP && NF == 16;
+  // Arrivals per phase of a_ready (unused without XF): with skip stages interleaved every transform warp arrives, else the
+  // owner alone (march_transform).  The count is that of the four-warp form, the only one that runs with skip stages.
+  static_assert(!(kWideXf && SKIP), "a_ready expects four arrivals per phase when skip stages are interleaved");
+  constexpr int kReadyCount = XF && SKIP ? 4 : 1;
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   if (threadIdx.x == 0) {
@@ -421,7 +362,7 @@ conv3d_march_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
     for (int s = 0; s < S; ++s) {
       ptx::mbar_init(&sh->a_full[s], 1);
       ptx::mbar_init(&sh->a_empty[s], 1);
-      ptx::mbar_init(&sh->a_ready[s], 1);
+      ptx::mbar_init(&sh->a_ready[s], kReadyCount);
     }
     ptx::mbar_init(&sh->b_full, 1);
     for (int g = 0; g < R; ++g) {
@@ -615,11 +556,6 @@ conv3d_march_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
     // ===================== epilogue (12 warps, three per TMEM lane quarter; with the fused input transform eight, and
     // warps 12..15 transform; conv_out four, and warps 8..15 transform): see march_epilogue / march_transform =====================
     ptx::setmaxnreg_inc<kRegsMEpi>();
-    // conv_out (16 output columns, one fp32 channel stored): the epilogue is a few instructions per voxel and the layer is
-    // bound by the input transform (R5i: 26 % tensor-pipe activity, transform warps busy ~90 %), so eight warps transform
-    // and four drain.  Only without the fused skip conv: there a warp that takes every EIGHTH main stage would skip a whole
-    // phase of a stage's a_full barrier, and a parity wait cannot tell phase n from phase n + 2.
-    constexpr bool kWideXf = XF && !SKIP && NF == 16;
     if (kWideXf && p.out_fp32) {
       if (warp >= 8) march_transform<KJ, SKIP, 8>(p, sh, a_smem);
       else march_epilogue<NF, kEpiFp32, 1>(p, sh, smem, stat_part, stat_acc, cadd_s, tmem_base);
